@@ -2,6 +2,7 @@
 """bench.py -- benchmark of the innr batch similarity-search hot path on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME|all] [--impl reference] [--sharding nccl|inproc]
+                  [--dump-outputs DIR]
   (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 A "step" is one pass of the hot path over one batch of synthetic input. Prints ONE JSON line on rank 0.
@@ -306,6 +307,10 @@ class Workload:
         sk = getattr(self, "sk", None)
         if sk is not None:
             sk.drain()
+
+    def outputs(self, result):
+        """Host copies of what a caller of step_dev receives from one step (the top-k workloads' result pair)."""
+        return {"indices": result[0].cpu().numpy(), "scores": result[1].cpu().numpy()}
 
     def close(self):
         """Drop the device shard (and the CPU sample) before the next workload is built."""
@@ -612,6 +617,9 @@ class MaxSim(Workload):
                C.c_void_p(self.out.data_ptr()), s)
         return self.out
 
+    def outputs(self, result):
+        return {"scores": result.cpu().numpy()}
+
     def step_e2e(self, i):
         import innr_b200 as ib
         return ib.maxsim_corpus(self.q_host[i % 4], self.shard, cosine=True, out=self.out_host)
@@ -745,12 +753,14 @@ def measure(w, args, env):
     ev[0].record()
     for i in range(steps):
         kev[i][0].record()
-        w.step_dev(i)
+        last = w.step_dev(i)
         kev[i][1].record()
     w.drain()  # N > 1: the exchanges run on a side stream under the next scan; the region ends when the last one has
     ev[1].record()
     barrier()
     sampler.mark_end()
+    # copied before anything else runs: the result buffers are reused by the measurements below
+    w.last_outputs = w.outputs(last) if args.dump_outputs and rank == 0 else None
     total_ms = max_over_ranks(ev[0].elapsed_time(ev[1]))
     launches = ib.launch_count() - l0
     step_ms = [a.elapsed_time(b) for a, b in kev]
@@ -870,6 +880,26 @@ def measure(w, args, env):
             if exchange_check:
                 entry["exchange_check"] = exchange_check
     return entry
+
+
+DUMP_SAMPLE = 1 << 20  # elements; a longer output is written as a seeded sample of this many
+
+
+def dump_outputs(out_dir, workload, arrays):
+    """Writes the arrays of one workload's last timed step as <out_dir>/<workload>_<name>.npy: float32 scores as they
+    are, indices and integer distances as float64 (exact). An output of more than DUMP_SAMPLE elements is written as the
+    values at a fixed, seeded set of flat positions, stored beside it as <workload>_<name>_positions.npy, so that the
+    dumps of two builds compare element for element and the whole dump stays under 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        base = os.path.join(out_dir, f"{workload}_{name}")
+        if a.size > DUMP_SAMPLE:
+            pos = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            np.save(base + "_positions.npy", pos.astype(np.float64))
+            a = a.reshape(-1)[pos]
+        np.save(base + ".npy", a)
 
 
 def run_inproc(args):
@@ -1032,7 +1062,14 @@ def main():
     ap.add_argument("--ref-budget-s", type=float, default=420.0,
                     help="reference arm: wall-clock bound of the whole run; if W + K full-size steps would exceed it, the "
                          "steps after the first use the prefix of the rows that fits (flagged extrapolated)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what each workload's last device-resident timed step returned as DIR/<workload>_<name>.npy "
+                         "(rank 0's results at N > 1); the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.sharding == "inproc"):
+        ap.error("--dump-outputs covers the device-resident steps of the b200 arm (not --impl reference or --sharding inproc)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -1086,6 +1123,8 @@ def main():
         w = make_workload(args, name, rank, world)
         try:
             entry = measure(w, args, env)
+            if w.last_outputs is not None:
+                dump_outputs(args.dump_outputs, name, w.last_outputs)
             if rank == 0 and world == 1 and not args.no_cpu_baseline:
                 w.close()  # device memory first: the CPU leg needs the host RAM, not the GPU
                 entry["cpu_baseline"] = cpu_baseline_entry(w, WORKLOADS[name][3], cpu_cache)

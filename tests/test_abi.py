@@ -156,35 +156,70 @@ def test_rust_shim_is_complete_source():
     assert not re.search(r"^innr\s*=", cargo, flags=re.M), "innr-cuda must not depend on innr (innr's cuda feature depends on it)"
 
 
-def test_integration_patch_applies_to_the_reference():
-    """integration/innr-cuda.patch (Backend::Cuda, the `cuda` feature, feature-gated branches, src/cuda.rs) must apply
-    cleanly to the reference tree and be structurally whole. The reference exists only in the build container."""
-    import shutil
-    import subprocess
-    import tempfile
-    patch = os.path.join(ROOT, "integration", "innr-cuda.patch")
-    ptxt = open(patch).read()
+PATCH = os.path.join(ROOT, "integration", "innr-cuda.patch")
+CUDA_RS_DEFINED_ELSEWHERE = {"VerticalBatch", "BatchKnnResult", "PackedBinary", "QuantizedU8", "QuantizationParams", "Error",
+                             "Metric", "F32Corpus", "BinaryCorpus", "U8Corpus", "TokenCorpus", "L2", "Dot", "Cosine"}
+CUDA_FEATURE_GATE = '#[cfg(feature = "cuda")]'
+
+
+def _patch_sections(ptxt):
+    """{path in the patched tree: (lines added, lines removed)} of a unified diff."""
+    out, cur = {}, None
+    for line in ptxt.splitlines():
+        if line.startswith("+++ b/"):
+            cur = out.setdefault(line[len("+++ b/"):].split("\t")[0], ([], []))
+        elif line.startswith(("--- ", "diff ")):
+            continue
+        elif cur is not None and line[:1] in ("+", "-"):
+            cur[line[0] == "-"].append(line[1:])
+    return out
+
+
+def _check_cuda_rs(path):
+    """src/cuda.rs of the patched reference: whole, every adapter of the feature present, and every call into innr-cuda
+    defined by innr-cuda/src/lib.rs."""
+    text, fns = _check_rust_source(path, extra_defined=CUDA_RS_DEFINED_ELSEWHERE)
+    for need in ("from_batch", "knn_l2", "knn_dot", "knn_cosine", "l2_squared_into", "dot_into", "norms_into", "cosine_into",
+                 "from_codes", "hamming_top_k", "from_quantized", "batch_knn_u8", "from_docs", "maxsim", "maxsim_cosine",
+                 "get_or_upload", "device_available"):
+        assert need in fns, f"src/cuda.rs lacks `{need}`"
+    lib_methods = _check_rust_source(os.path.join(ROOT, "innr-cuda", "src", "lib.rs"),
+                                     extra_defined={"innr_cuda_corpus", "innr_cuda_exchange", "innr_cuda_ticket"})[1]
+    for m in set(re.findall(r"self\.inner\.([a-z_0-9]+)\(", text)):   # every call into innr-cuda exists there
+        assert m in lib_methods, f"src/cuda.rs calls innr_cuda::*::{m}, which innr-cuda/src/lib.rs does not define"
+
+
+def test_integration_patch_is_whole(tmp_path):
+    """integration/innr-cuda.patch (Backend::Cuda, the `cuda` feature, feature-gated branches, src/cuda.rs) is
+    structurally whole, read from the patch alone: src/cuda.rs is a new file, so its whole text is in the patch, and the
+    feature-gated branches it adds to src/batch.rs are counted on the added lines."""
+    ptxt = open(PATCH).read()
     for needle in ('+    Cuda,', '+            Backend::Cuda => "cuda",', '+cuda = ["dep:innr-cuda"]', '+pub mod cuda;',
                    '+    if let Some(dev) = batch.device() {', '+++ b/src/cuda.rs'):
         assert needle in ptxt, needle
-    ref = "/root/reference"
+    sections = _patch_sections(ptxt)
+    added, removed = sections["src/cuda.rs"]
+    assert added and not removed
+    (tmp_path / "cuda.rs").write_text("\n".join(added) + "\n")
+    _check_cuda_rs(str(tmp_path / "cuda.rs"))
+    assert "\n".join(sections["src/batch.rs"][0]).count(CUDA_FEATURE_GATE) >= 13
+
+
+def test_integration_patch_applies_to_the_reference():
+    """integration/innr-cuda.patch applies cleanly to the reference tree, and the patched tree passes the checks of
+    test_integration_patch_is_whole. The reference (innr 0.6.3, a Rust crate) is not part of this repository: point
+    INNR_REFERENCE_DIR at a checkout of it to run this test."""
+    import shutil
+    import subprocess
+    import tempfile
+    ref = os.environ.get("INNR_REFERENCE_DIR", "")
     if not os.path.isdir(ref):
-        pytest.skip("the reference tree is not present on this box")
+        pytest.skip("INNR_REFERENCE_DIR does not name a checkout of innr 0.6.3")
     with tempfile.TemporaryDirectory() as tmp:
         shutil.copy(os.path.join(ref, "Cargo.toml"), tmp)
         shutil.copytree(os.path.join(ref, "src"), os.path.join(tmp, "src"))
-        r = subprocess.run(["patch", "-p1", "--batch", "-i", patch], cwd=tmp, capture_output=True, text=True)
+        r = subprocess.run(["patch", "-p1", "--batch", "-i", PATCH], cwd=tmp, capture_output=True, text=True)
         assert r.returncode == 0, r.stdout + r.stderr
-        text, fns = _check_rust_source(os.path.join(tmp, "src", "cuda.rs"),
-                                       extra_defined={"VerticalBatch", "BatchKnnResult", "PackedBinary", "QuantizedU8", "QuantizationParams",
-                                                      "Error", "Metric", "F32Corpus", "BinaryCorpus", "U8Corpus", "TokenCorpus", "L2", "Dot", "Cosine"})
-        for need in ("from_batch", "knn_l2", "knn_dot", "knn_cosine", "l2_squared_into", "dot_into", "norms_into", "cosine_into",
-                     "from_codes", "hamming_top_k", "from_quantized", "batch_knn_u8", "from_docs", "maxsim", "maxsim_cosine",
-                     "get_or_upload", "device_available"):
-            assert need in fns, f"src/cuda.rs lacks `{need}`"
-        lib_methods = _check_rust_source(os.path.join(ROOT, "innr-cuda", "src", "lib.rs"),
-                                         extra_defined={"innr_cuda_corpus", "innr_cuda_exchange", "innr_cuda_ticket"})[1]
-        for m in set(re.findall(r"self\.inner\.([a-z_0-9]+)\(", text)):   # every call into innr-cuda exists there
-            assert m in lib_methods, f"src/cuda.rs calls innr_cuda::*::{m}, which innr-cuda/src/lib.rs does not define"
+        _check_cuda_rs(os.path.join(tmp, "src", "cuda.rs"))
         batch = open(os.path.join(tmp, "src", "batch.rs")).read()
-        assert batch.count("#[cfg(feature = \"cuda\")]") >= 13
+        assert batch.count(CUDA_FEATURE_GATE) >= 13
