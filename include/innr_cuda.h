@@ -86,10 +86,20 @@ int innr_cuda_knn_tc_last_stats(float* out_filter_ms, float* out_total_ms, doubl
 int innr_cuda_knn_tc_debug_bounds(const innr_cuda_corpus* c, int metric, const float* queries, size_t n_queries,
                                   size_t query_len, float* out_lower, size_t* out_rows, float* out_eps,
                                   uint32_t* out_qflags);
+/* Test hook for the screened single-query kNN of a split corpus: the interval [lower, upper] the screen gives every row
+ * for this query, exactly as production computes it (n floats each). The tests assert lower <= reference score <= upper
+ * on adversarial rows. INNR_EUNSUPPORTED when the corpus is not split, has a non-finite row or the query cannot be
+ * screened (norm not finite; cosine: below the reference's epsilon). */
+int innr_cuda_knn_screen_debug_bounds(const innr_cuda_corpus* c, int metric, const float* query, size_t query_len,
+                                      float* out_lower, float* out_upper);
 /* number of kernels the library has launched so far (bench.py's gpu_launches counter) */
 int innr_cuda_launch_count(uint64_t* out_count);
 
 /* ---- f32 VerticalBatch (PDX) corpus: src/batch.rs:88-220 ------------------------------------- */
+/* Owned corpora of at least f32_split_min_rows rows (innr_cuda_set_option; default 1,000,000) are stored split: the
+ * same bytes as two 16-bit planes (high halves, then low halves, same pitch), which lets a single-query kNN read only
+ * the high halves before it rescores a few dozen rows exactly. Every entry gives the same bits on either layout;
+ * corpus_info's ld and device_bytes keep their meaning. Wrapped device memory stays as the caller laid it out. */
 /* host_pdx: the buffer VerticalBatch::data() returns (src/batch.rs:212): data[d*n + i]. */
 int innr_cuda_upload_f32_pdx(const float* host_pdx, size_t n, size_t d, uint64_t index_base,
                              innr_cuda_corpus** out);

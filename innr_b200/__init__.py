@@ -12,7 +12,8 @@ from .batch import (BatchKnnResult, DeviceBatch, VerticalBatch, batch_cosine, ba
                     batch_dimension_variance, batch_dot, batch_dot_into, batch_knn, batch_knn_adaptive, batch_knn_cosine,
                     batch_knn_dot,
                     batch_knn_filtered, batch_knn_many, batch_knn_reordered, batch_knn_subset, batch_l2_squared,
-                    batch_l2_squared_into, batch_l2_squared_pruning, batch_norms, batch_norms_into, knn_tc_debug_bounds)
+                    batch_l2_squared_into, batch_l2_squared_pruning, batch_norms, batch_norms_into, knn_tc_debug_bounds,
+                    knn_screen_debug_bounds)
 from .binary import (BinaryCorpus, PackedBinary, binary_dot, binary_dot_all, binary_hamming, binary_jaccard,  # noqa: F401
                      binary_jaccard_all, binary_topk, encode_binary, hamming_all,
                      hamming_topk, hamming_topk_many)

@@ -39,6 +39,7 @@ SIGNATURES = {
     "innr_cuda_set_option": [C.c_char_p, C.c_double],
     "innr_cuda_knn_tc_last_stats": [f32p, f32p, C.POINTER(C.c_double), u64p, C.POINTER(C.c_uint32), C.POINTER(ci)],
     "innr_cuda_knn_tc_debug_bounds": [vp, ci, f32p, sz, sz, f32p, szp, f32p, u32p],
+    "innr_cuda_knn_screen_debug_bounds": [vp, ci, f32p, sz, f32p, f32p],
     "innr_cuda_launch_count": [u64p],
     "innr_cuda_last_kernel_ms": [f32p],
     "innr_cuda_upload_f32_pdx": [f32p, sz, sz, u64, handle_p],

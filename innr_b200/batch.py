@@ -297,6 +297,18 @@ def knn_tc_debug_bounds(metric: str, queries, batch):
     return lower.reshape(-1)[:nq * rows.value].reshape(nq, rows.value), float(eps.value), flags
 
 
+def knn_screen_debug_bounds(metric: str, query, batch):
+    """Test hook (include/innr_cuda.h: innr_cuda_knn_screen_debug_bounds): the screened kNN's interval for every row of a
+    split corpus. Returns (lower[n], upper[n])."""
+    dev = _dev(batch)
+    q = _f32(query).reshape(-1)
+    lower = np.zeros(dev.num_vectors, np.float32)
+    upper = np.zeros(dev.num_vectors, np.float32)
+    m = {"dot": L.METRIC_DOT, "cosine": L.METRIC_COSINE, "l2": L.METRIC_L2}[metric]
+    L.call("innr_cuda_knn_screen_debug_bounds", dev.h, m, _ptr(q, L.f32p), q.size, _ptr(lower, L.f32p), _ptr(upper, L.f32p))
+    return lower, upper
+
+
 def _knn(metric: str, query, batch, k: int) -> BatchKnnResult:
     q = _f32(query).reshape(1, -1)
     idx, sc = batch_knn_many(metric, q, batch, k)

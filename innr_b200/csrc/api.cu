@@ -38,6 +38,12 @@ struct innr_cuda_corpus {
   size_t total_tokens = 0, uniform_tokens = 0;
   CUtensorMap tmap;
   bool tmap_valid = false;
+  // f32 PDX, split layout (pdx.cuh): the low-half plane (the high halves start at `dev`); null for plain corpora
+  uint16_t* lo_plane = nullptr;
+  // f32 PDX, split corpora: the screened kNN's per-row sidecar (built with the corpus): dev_norms (the reference's norm
+  // bits), dev_lo_norm (r_i >= |lo_i|); `screen` = both finite for every row
+  float* dev_lo_norm = nullptr;
+  bool screen = false;
   // f32 PDX: lazily built operands of the tensor-core filter path (knn_tc.cu): exact norms, f16 unit vectors + TMA map
   int tc_state = 0;  // 0 not built, 1 ready, -1 unusable (non-finite norms / no memory): exact scan only
   float* dev_norms = nullptr;
@@ -148,6 +154,7 @@ struct Options {
   bool knn_tc = true;
   size_t knn_tc_min_n = 100000;
   size_t knn_tc_min_queries = 2;  // measured at 10M x 768: filter call 2.6 ms for 2..64 queries, 8-query scan pass 6.3 ms
+  size_t f32_split_min_rows = 1000000;  // owned f32 corpora from this many rows are stored split (DESIGN.md section 2)
   bool maxsim_tc = true;
   bool kernel_timing = false;
 } g_opt;
@@ -222,6 +229,10 @@ int alloc_workspace(Workspace& w, int num_sms) {
   return INNR_OK;
 }
 void free_workspace(Workspace& w) {
+  cudaFree(w.sc_bounds);
+  cudaFree(w.sc_cand);
+  cudaFree(w.sc_keys);
+  cudaFree(w.sc_ctl);
   cudaFree(w.partials);
   cudaFree(w.group_partials);
   cudaFree(w.tickets);
@@ -346,6 +357,7 @@ void destroy_corpus(innr_cuda_corpus* c) {
   if (c->owns && c->dev) cudaFree(c->dev);
   if (c->dev_offsets) cudaFree(c->dev_offsets);
   if (c->dev_norms) cudaFree(c->dev_norms);
+  if (c->dev_lo_norm) cudaFree(c->dev_lo_norm);
   if (c->dev_xh) cudaFree(c->dev_xh);
   if (c->dev_order) cudaFree(c->dev_order);
   delete c;
@@ -373,7 +385,12 @@ int new_corpus(int kind, int device, innr_cuda_corpus** out) {
 }
 
 PdxView pdx_view(const innr_cuda_corpus* c) {
+  if (c->lo_plane) return PdxView{nullptr, c->n, c->d, c->ld, (uint32_t)c->index_base, (const uint16_t*)c->dev, c->lo_plane};
   return PdxView{(const float*)c->dev, c->n, c->d, c->ld, (uint32_t)c->index_base};
+}
+PdxDst pdx_dst(innr_cuda_corpus* c) {
+  if (c->lo_plane) return PdxDst{nullptr, (uint16_t*)c->dev, c->lo_plane, c->ld};
+  return PdxDst{(float*)c->dev, nullptr, nullptr, c->ld};
 }
 BinView bin_view(const innr_cuda_corpus* c) {
   return BinView{(const uint4*)c->dev, c->n, c->ld, c->words, c->chunks, c->dim_bits, (uint32_t)c->index_base};
@@ -467,6 +484,7 @@ int innr_cuda_set_option(const char* name, double value) {
   if (n == "knn_tc") g_opt.knn_tc = value != 0;
   else if (n == "knn_tc_min_n") g_opt.knn_tc_min_n = (size_t)value;
   else if (n == "knn_tc_min_queries") g_opt.knn_tc_min_queries = (size_t)value;
+  else if (n == "f32_split_min_rows") g_opt.f32_split_min_rows = (size_t)value;
   else if (n == "maxsim_tc") g_opt.maxsim_tc = value != 0;
   else if (n == "kernel_timing") g_opt.kernel_timing = value != 0;
   else if (n == "u8_scaled_chains") u8_set_scaled_chains(value != 0);
@@ -518,8 +536,26 @@ static int alloc_pdx(DeviceCtx& ctx, size_t n, size_t d, uint64_t index_base, in
       *out = nullptr;
       return cuda_fail(e, "cudaMalloc(corpus)");
     }
+    if (n >= g_opt.f32_split_min_rows) c->lo_plane = (uint16_t*)c->dev + c->ld * d;
   }
   guard.ok = true;
+  return INNR_OK;
+}
+
+// After a split corpus is written: its sidecar. The norms pass writes whole float4 groups (up to ld entries), the
+// screen reads whole groups of 8: both arrays have ld (+ the tensor-core path's 16 B of scratch) entries.
+static int build_sidecar(innr_cuda_corpus* c, DeviceCtx* ctx) {
+  if (!c->lo_plane) return INNR_OK;
+  CU(cudaMalloc((void**)&c->dev_norms, c->ld * sizeof(float) + 16));
+  CU(cudaMalloc((void**)&c->dev_lo_norm, c->ld * sizeof(float)));
+  const PdxView v = pdx_view(c);
+  CU(launch_pdx_scores(v, PDX_NORMS, nullptr, nullptr, c->dev_norms, ctx->ws, ctx->stream, &g_launches));
+  CU(ctx->h_counts.reserve(64));
+  unsigned* flag = (unsigned*)(c->dev_norms + c->ld);
+  CU(launch_split_sidecar(v, c->dev_norms, c->dev_lo_norm, flag, ctx->stream, &g_launches));
+  CU(cudaMemcpyAsync(ctx->h_counts.p, flag, sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  c->screen = *(unsigned*)ctx->h_counts.p == 0;
   return INNR_OK;
 }
 
@@ -534,12 +570,29 @@ int innr_cuda_upload_f32_pdx(const float* host_pdx, size_t n, size_t d, uint64_t
   if (rc) return rc;
   innr_cuda_corpus* c = *out;
   CorpusGuard guard(out);
-  if (c->bytes) {
+  if (c->bytes && !c->lo_plane) {
     CU(cudaMemsetAsync(c->dev, 0, c->bytes, ctx->stream));
     CU(cudaMemcpy2DAsync(c->dev, c->ld * sizeof(float), host_pdx, n * sizeof(float), n * sizeof(float), d,
                          cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
+  } else if (c->bytes) {
+    // split: dimension rows in chunks through one 256 MB staging buffer, split into the two planes on the device
+    size_t chunk = (size_t)(256u << 20) / (n * sizeof(float));
+    if (chunk < 1) chunk = 1;
+    if (chunk > d) chunk = d;
+    void* stage = nullptr;
+    cudaError_t e = cudaMalloc(&stage, chunk * n * sizeof(float));
+    for (size_t d0 = 0; d0 < d && e == cudaSuccess; d0 += chunk) {
+      const size_t rows = d - d0 < chunk ? d - d0 : chunk;
+      e = cudaMemcpyAsync(stage, host_pdx + d0 * n, rows * n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+      if (e == cudaSuccess) e = launch_pdx_rows_to_dst((const float*)stage, rows, n, pdx_dst(c).at_column(d0 * c->ld), ctx->stream, &g_launches);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (stage) cudaFree(stage);
+    if (e != cudaSuccess) return cuda_fail(e, "upload_f32_pdx");
   }
+  rc = build_sidecar(c, ctx);
+  if (rc) return rc;
   guard.ok = true;
   return INNR_OK;
 }
@@ -569,13 +622,15 @@ int innr_cuda_upload_f32_rows(const float* host_rows, size_t n, size_t d, uint64
       const bool last = i0 + rows == n;
       e = cudaMemcpyAsync(stage, host_rows + i0 * d, rows * d * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
       if (e == cudaSuccess)
-        e = launch_transpose_rows_to_pdx((const float*)stage, rows, d, (float*)c->dev + i0, c->ld,
+        e = launch_transpose_rows_to_pdx((const float*)stage, rows, d, pdx_dst(c).at_column(i0),
                                          last ? c->ld - i0 : rows, ctx->stream, &g_launches);
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (stage) cudaFree(stage);
     if (e != cudaSuccess) return cuda_fail(e, "upload_f32_rows");
   }
+  rc = build_sidecar(c, ctx);
+  if (rc) return rc;
   guard.ok = true;
   return INNR_OK;
 }
@@ -619,6 +674,7 @@ int innr_cuda_prefix_view(const innr_cuda_corpus* c, size_t prefix_dim, innr_cud
   innr_cuda_corpus* v = *out;
   v->owns = false;
   v->dev = c->dev;
+  v->lo_plane = c->lo_plane;  // the parent's planes; its sidecar is for the full d, so the view has none
   v->n = c->n;
   v->d = d;
   v->ld = c->ld;
@@ -639,9 +695,11 @@ int innr_cuda_generate_f32_pdx(int generator, uint64_t salt, uint64_t first_row,
   innr_cuda_corpus* c = *out;
   CorpusGuard guard(out);
   if (c->bytes) {
-    CU(launch_generate_f32_pdx(generator, salt, first_row, n, d, (float*)c->dev, c->ld, ctx->stream, &g_launches));
+    CU(launch_generate_f32_pdx(generator, salt, first_row, n, d, pdx_dst(c), ctx->stream, &g_launches));
     CU(cudaStreamSynchronize(ctx->stream));
   }
+  rc = build_sidecar(c, ctx);
+  if (rc) return rc;
   guard.ok = true;
   return INNR_OK;
 }
@@ -673,6 +731,19 @@ int innr_cuda_extract_vector(const innr_cuda_corpus* c, size_t i, float* out_hos
   int rc = ctx_for(c, &ctx);
   if (rc) return rc;
   if (c->d == 0) return INNR_OK;
+  if (c->lo_plane) {  // the two halves of every element, joined here
+    std::vector<uint16_t> h(c->d), l(c->d);
+    CU(cudaMemcpy2DAsync(h.data(), sizeof(uint16_t), (const uint16_t*)c->dev + i, c->ld * sizeof(uint16_t), sizeof(uint16_t),
+                         c->d, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpy2DAsync(l.data(), sizeof(uint16_t), c->lo_plane + i, c->ld * sizeof(uint16_t), sizeof(uint16_t), c->d,
+                         cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    for (size_t dd = 0; dd < c->d; ++dd) {
+      const uint32_t b = ((uint32_t)h[dd] << 16) | l[dd];
+      std::memcpy(out_host + dd, &b, sizeof(b));
+    }
+    return INNR_OK;
+  }
   CU(cudaMemcpy2DAsync(out_host, sizeof(float), (const float*)c->dev + i, c->ld * sizeof(float), sizeof(float),
                        c->d, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
@@ -734,17 +805,20 @@ static int knn_tc_prepare(innr_cuda_corpus* c, DeviceCtx* ctx, const PdxView& v,
   if (c->tc_state != 0) return INNR_OK;
   c->tc_state = -1;
   const size_t xh_bytes = c->n * knn_tc_dpad(c->d) * 2;
-  if (cudaMalloc(&c->dev_norms, c->n * sizeof(float) + 16) != cudaSuccess ||
+  const bool have_norms = c->dev_norms != nullptr;  // a split corpus' sidecar: the same bits
+  if ((!have_norms && cudaMalloc(&c->dev_norms, c->n * sizeof(float) + 16) != cudaSuccess) ||
       cudaMalloc(&c->dev_xh, xh_bytes) != cudaSuccess) {
     cudaGetLastError();  // out of memory is not an error of the call: exact scan
-    if (c->dev_norms) cudaFree(c->dev_norms);
-    c->dev_norms = nullptr;
+    if (!have_norms && c->dev_norms) cudaFree(c->dev_norms);
+    if (!have_norms) c->dev_norms = nullptr;
     c->dev_xh = nullptr;
     return INNR_OK;
   }
-  CU(ctx->d_scores.reserve(c->ld * sizeof(float)));
-  CU(launch_pdx_scores(v, PDX_NORMS, nullptr, nullptr, (float*)ctx->d_scores.p, ctx->ws, s, &g_launches));
-  CU(cudaMemcpyAsync(c->dev_norms, ctx->d_scores.p, c->n * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  if (!have_norms) {
+    CU(ctx->d_scores.reserve(c->ld * sizeof(float)));
+    CU(launch_pdx_scores(v, PDX_NORMS, nullptr, nullptr, (float*)ctx->d_scores.p, ctx->ws, s, &g_launches));
+    CU(cudaMemcpyAsync(c->dev_norms, ctx->d_scores.p, c->n * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  }
   CU(ctx->h_counts.reserve(64));
   unsigned* nonfinite = (unsigned*)ctx->h_counts.p;
   CU(launch_knn_tc_build(v, c->dev_norms, c->dev_xh, (unsigned*)(c->dev_norms + c->n), &c->tm_xh, nonfinite, s, &g_launches));
@@ -771,7 +845,35 @@ static int big_k_from_scores(DeviceCtx* ctx, const void* dev_scores, int kind, s
 static bool knn_takes_tc_filter(const innr_cuda_corpus* c, const PdxView& v, int mode, size_t nq, size_t k) {
   return g_opt.knn_tc && c->n >= g_opt.knn_tc_min_n && nq >= g_opt.knn_tc_min_queries && knn_tc_supported(v, mode, nq, k);
 }
+// single queries on a split corpus with a finite sidecar take the screened kNN (scan_f32.cu)
+static bool knn_takes_screen(const innr_cuda_corpus* c, size_t nq, size_t k) {
+  return nq == 1 && c->screen && k <= MAX_FUSED_K && k <= c->n && c->d <= SCREEN_MAX_D;
+}
+// its scratch lives in the lane's Workspace (both lanes may run one), sized for `rows` rows (2 x rows for the test hook)
+static int ensure_screen_scratch(Workspace& w, size_t rows) {
+  if (!w.sc_cand) {
+    CU(cudaMalloc((void**)&w.sc_cand, SCREEN_CAP * sizeof(uint32_t)));
+    CU(cudaMalloc((void**)&w.sc_keys, (SCREEN_CAP + MAX_FUSED_K) * sizeof(uint64_t)));
+    CU(cudaMalloc((void**)&w.sc_ctl, 2 * sizeof(unsigned)));
+  }
+  if (w.sc_bounds_cap < rows) {
+    if (w.sc_bounds) cudaFree(w.sc_bounds);  // waits for the device: a launch in flight may still read it
+    w.sc_bounds = nullptr;
+    w.sc_bounds_cap = 0;
+    CU(cudaMalloc((void**)&w.sc_bounds, rows * sizeof(float)));
+    w.sc_bounds_cap = rows;
+  }
+  return INNR_OK;
+}
+static int knn_screened(innr_cuda_corpus* c, Workspace& w, int mode, const float* dev_query, size_t k, uint64_t* dev_keys,
+                        cudaStream_t s) {
+  int rc = ensure_screen_scratch(w, c->ld);
+  if (rc) return rc;
+  CU(launch_pdx_knn_screened(pdx_view(c), mode, c->dev_norms, c->dev_lo_norm, dev_query, k, dev_keys, w, s, &g_launches));
+  return INNR_OK;
+}
 // the plain fused scan (k <= 128, no tensor-core filter) needs a Workspace and nothing else: either lane will do
+// (so does the screened kNN)
 static bool knn_is_scan_only(const innr_cuda_corpus* c, int mode, size_t nq, size_t k) {
   return k <= MAX_FUSED_K && !knn_takes_tc_filter(c, pdx_view(c), mode, nq, k);
 }
@@ -805,10 +907,17 @@ static int knn_keys_dev(innr_cuda_corpus* c, DeviceCtx* ctx, int mode, const flo
       std::lock_guard<std::mutex> lg(g_mu);
       g_tc_stats = st;
     }
-    for (unsigned q : overflow)
-      CU(launch_pdx_knn(v, mode, dev_queries + (size_t)q * c->d, 1, k, dev_keys + (size_t)q * k, ctx->ws, s, &g_launches));
+    for (unsigned q : overflow) {
+      if (knn_takes_screen(c, 1, k)) {
+        int rc = knn_screened(c, ctx->ws, mode, dev_queries + (size_t)q * c->d, k, dev_keys + (size_t)q * k, s);
+        if (rc) return rc;
+      } else {
+        CU(launch_pdx_knn(v, mode, dev_queries + (size_t)q * c->d, 1, k, dev_keys + (size_t)q * k, ctx->ws, s, &g_launches));
+      }
+    }
     return INNR_OK;
   }
+  if (!tc && knn_takes_screen(c, nq, k)) return knn_screened(c, ctx->lane_ws(lane), mode, dev_queries, k, dev_keys, s);
   CU(launch_pdx_knn(v, mode, dev_queries, nq, k, dev_keys, ctx->lane_ws(tc ? 0 : lane), s, &g_launches));
   return INNR_OK;
 }
@@ -842,6 +951,30 @@ extern "C" int innr_cuda_knn_tc_debug_bounds(const innr_cuda_corpus* c, int metr
   CU(cudaMemcpyAsync(ctx->d_query.p, queries, n_queries * c->d * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
   CU(launch_knn_tc_debug_bounds(v, c->tm_xh, c->dev_norms, mode, (const float*)ctx->d_query.p, n_queries, ctx->d_tcws.p, out_lower,
                                 out_rows, out_eps, out_qflags, ctx->ws.num_sms, ctx->stream, &g_launches));
+  return INNR_OK;
+}
+
+extern "C" int innr_cuda_knn_screen_debug_bounds(const innr_cuda_corpus* c, int metric, const float* query,
+                                                 size_t query_len, float* out_lower, float* out_upper) {
+  if (!c || c->kind != 0) return fail(INNR_EINVAL, "need an f32 PDX corpus");
+  int mode;
+  int rc = metric_to_mode(metric, &mode);
+  if (rc) return rc;
+  if (query_len != c->d) return fail(INNR_EINVAL, "query.len() != batch.dimension");
+  if (!query || !out_lower || !out_upper) return fail(INNR_EINVAL, "null argument");
+  if (!c->screen || c->d > SCREEN_MAX_D || c->n == 0) return fail(INNR_EUNSUPPORTED, "corpus cannot take the screened kNN");
+  EntryGuard lk(c->device);
+  DeviceCtx* ctx;
+  rc = ctx_for(c, &ctx);
+  if (rc) return rc;
+  rc = ensure_screen_scratch(ctx->ws, 2 * c->ld);
+  if (rc) return rc;
+  CU(ctx->d_query.reserve((c->d + 4) * sizeof(float)));
+  CU(cudaMemcpyAsync(ctx->d_query.p, query, c->d * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  cudaError_t e = launch_pdx_screen_debug_bounds(pdx_view(c), mode, c->dev_norms, c->dev_lo_norm, (const float*)ctx->d_query.p,
+                                                 out_lower, out_upper, ctx->ws, ctx->stream, &g_launches);
+  if (e == cudaErrorNotSupported) return fail(INNR_EUNSUPPORTED, "the query cannot be screened");
+  CU(e);
   return INNR_OK;
 }
 
@@ -1437,7 +1570,7 @@ int innr_cuda_binary_from_f32(const innr_cuda_corpus* f32_corpus, float threshol
   innr_cuda_corpus* c = *out;
   CorpusGuard guard(out);
   if (c->bytes) {
-    CU(launch_binary_from_pdx((const float*)f32_corpus->dev, f32_corpus->ld, f32_corpus->n, f32_corpus->d, threshold,
+    CU(launch_binary_from_pdx(pdx_view(f32_corpus), threshold,
                               (uint4*)c->dev, c->ld, ctx->stream, &g_launches));
     CU(cudaStreamSynchronize(ctx->stream));
   }
@@ -1700,7 +1833,7 @@ int innr_cuda_u8_from_f32(const innr_cuda_corpus* f32_corpus, float alpha, float
   innr_cuda_corpus* c = *out;
   CorpusGuard guard(out);
   if (c->bytes) {
-    CU(launch_u8_from_pdx((const float*)f32_corpus->dev, f32_corpus->ld, f32_corpus->n, f32_corpus->d, alpha, offset,
+    CU(launch_u8_from_pdx(pdx_view(f32_corpus), alpha, offset,
                           (uint4*)c->dev, c->ld, ctx->stream, &g_launches));
     CU(cudaStreamSynchronize(ctx->stream));
   }
@@ -1908,7 +2041,7 @@ int innr_cuda_ternary_from_f32(const innr_cuda_corpus* f32_corpus, float thresho
   innr_cuda_corpus* c = *out;
   CorpusGuard guard(out);
   if (c->bytes) {
-    CU(launch_ternary_from_pdx((const float*)f32_corpus->dev, f32_corpus->ld, f32_corpus->n, f32_corpus->d, threshold,
+    CU(launch_ternary_from_pdx(pdx_view(f32_corpus), threshold,
                                (uint4*)c->dev, c->ld, ctx->stream, &g_launches));
     CU(cudaStreamSynchronize(ctx->stream));
   }

@@ -14,6 +14,7 @@
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "pdx.cuh"
 
 namespace innr {
 
@@ -262,7 +263,7 @@ __global__ void generate_binary_kernel(uint64_t salt, uint64_t first_row, unsign
 
 // encode_binary (src/binary.rs:133-141) of every vector of a device-resident PDX f32 corpus straight into the
 // chunk-major code layout: thread (chunk c, vector i) reads 128 dimension rows (coalesced along i), bit = v > threshold
-__global__ void binary_from_pdx_kernel(const float* __restrict__ pdx, size_t ld_f, unsigned n, unsigned d,
+__global__ void binary_from_pdx_kernel(const PdxView pdx, unsigned n, unsigned d,
                                        float threshold, uint4* __restrict__ codes, size_t ld, unsigned chunks) {
   const size_t total = (size_t)chunks * ld;
   for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
@@ -273,7 +274,7 @@ __global__ void binary_from_pdx_kernel(const float* __restrict__ pdx, size_t ld_
 #pragma unroll 8
       for (int b = 0; b < 128; ++b) {
         const unsigned dd = 128 * c + b;
-        if (dd < d && pdx[(size_t)dd * ld_f + i] > threshold) w[b >> 5] |= 1u << (b & 31);
+        if (dd < d && pdx_load1(pdx, (size_t)dd * pdx.ld + i) > threshold) w[b >> 5] |= 1u << (b & 31);
       }
     }
     codes[t] = make_uint4(w[0], w[1], w[2], w[3]);
@@ -422,11 +423,11 @@ cudaError_t launch_generate_binary(uint64_t salt, uint64_t first_row, size_t n, 
   return cudaGetLastError();
 }
 
-cudaError_t launch_binary_from_pdx(const float* dev_pdx, size_t ld_f, size_t n, size_t d, float threshold,
+cudaError_t launch_binary_from_pdx(const PdxView& v, float threshold,
                                    uint4* dev_codes, size_t ld, cudaStream_t s, LaunchCounter* launches) {
-  if (n == 0 || d == 0) return cudaSuccess;
-  binary_from_pdx_kernel<<<148 * 16, 256, 0, s>>>(dev_pdx, ld_f, (unsigned)n, (unsigned)d, threshold, dev_codes, ld,
-                                                  (unsigned)((d + 127) / 128));
+  if (v.n == 0 || v.d == 0) return cudaSuccess;
+  binary_from_pdx_kernel<<<148 * 16, 256, 0, s>>>(v, (unsigned)v.n, (unsigned)v.d, threshold, dev_codes, ld,
+                                                  (unsigned)((v.d + 127) / 128));
   ++*launches;
   return cudaGetLastError();
 }

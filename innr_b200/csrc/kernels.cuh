@@ -32,6 +32,13 @@ struct Workspace {
   size_t tickets_cap = 0;
   unsigned long long* shared_thr = nullptr;  // launch-wide bound on the k-th key (common.cuh: SharedThreshold); all ones between launches
   int num_sms = 0;
+  // screened single-query kNN (launch_pdx_knn_screened): one optimistic bound per row, the candidate list and its
+  // ready-made keys, the k keys of the pessimistic bounds, and ctl = {candidate count, "the exact scan answers" flag}
+  float* sc_bounds = nullptr;
+  size_t sc_bounds_cap = 0;  // in floats
+  uint32_t* sc_cand = nullptr;
+  uint64_t* sc_keys = nullptr;
+  unsigned* sc_ctl = nullptr;
 };
 
 // Persistent grids stride tiles by gridDim: pick the largest grid <= max_ctas for which every CTA gets the same
@@ -43,16 +50,46 @@ inline unsigned balanced_grid(unsigned n_tiles, unsigned max_ctas) {
   return (n_tiles + waves - 1) / waves;
 }
 
+// An f32 corpus in the PDX layout (dimension-major, row pitch ld). Kernels read it through pdx.cuh only: plain corpora
+// hold data[dd * ld + i]; split corpora (hi != null) hold the high and low 16 bits of that element at hi[dd * ld + i] and
+// lo[dd * ld + i], two planes of one allocation of the plain size.
 struct PdxView {
-  const float* data;  // data[dd * ld + i]
+  const float* data;
   size_t n, d, ld;
   uint32_t index_base;
+  const uint16_t* hi = nullptr;
+  const uint16_t* lo = nullptr;
+};
+// a corpus being written: data for plain, hi / lo for split (same pitch ld)
+struct PdxDst {
+  float* data;
+  uint16_t* hi;
+  uint16_t* lo;
+  size_t ld;
+  PdxDst at_column(size_t i0) const { return PdxDst{data ? data + i0 : nullptr, hi ? hi + i0 : nullptr, lo ? lo + i0 : nullptr, ld}; }
 };
 
 // kNN: queries on device (nq x d row-major); writes nq x k sorted keys (sentinel padded) into dev_keys.
 // Returns cudaSuccess or the launch error; `launches` is incremented per kernel launched.
+// dev_run_flag (optional): the launch does nothing unless *dev_run_flag != 0 when it starts (read on the device)
 cudaError_t launch_pdx_knn(const PdxView& v, int mode, const float* dev_queries, size_t nq, size_t k,
-                           uint64_t* dev_keys, Workspace& ws, cudaStream_t s, LaunchCounter* launches);
+                           uint64_t* dev_keys, Workspace& ws, cudaStream_t s, LaunchCounter* launches,
+                           const unsigned* dev_run_flag = nullptr);
+// Screened single-query kNN of a split corpus (scan_f32.cu): the hi plane alone gives every row an interval that holds
+// its exact score, the rows whose interval reaches the k-th best pessimistic bound are rescored exactly from both planes.
+// Same keys as launch_pdx_knn. Needs the corpus' sidecar (dev_norms, dev_lo_norm, all finite), k <= 128,
+// d <= SCREEN_MAX_D and ws.sc_* sized for v.ld rows. More than SCREEN_CAP candidates, or a query whose norm is not finite
+// (cosine: below the reference's epsilon), hand the query to the full-read scan, queued behind on the device.
+constexpr size_t SCREEN_CAP = 4096;
+constexpr size_t SCREEN_MAX_D = 4096;
+cudaError_t launch_pdx_knn_screened(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+                                    const float* dev_query, size_t k, uint64_t* dev_keys, Workspace& ws, cudaStream_t s,
+                                    LaunchCounter* launches);
+// test hook: the screen's interval [lower, upper] for every row (host arrays of n floats); returns cudaErrorNotSupported
+// when the query cannot be screened
+cudaError_t launch_pdx_screen_debug_bounds(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+                                           const float* dev_query, float* host_lower, float* host_upper, Workspace& ws,
+                                           cudaStream_t s, LaunchCounter* launches);
 // batch_knn_filtered (src/batch.rs:820-882): L2, one query; dev_mask = one bit per local vector (LSB-first u32 words,
 // zero padded to ld/32 + 1 words); vectors whose bit is clear are neither read nor offered.
 cudaError_t launch_pdx_knn_filtered(const PdxView& v, const float* dev_query, const uint32_t* dev_mask, size_t k,
@@ -154,11 +191,19 @@ cudaError_t launch_pdx_knn_tc(const PdxView& v, const CUtensorMap& tm_xh, const 
                               std::vector<unsigned>* overflow_queries, KnnTcStats* stats);
 
 // layout / generator kernels (layout.cu)
-// n rows (row-major, device) -> columns [0, cols) of dev_pdx (cols >= n; columns past n are zero-filled)
-cudaError_t launch_transpose_rows_to_pdx(const float* dev_rows, size_t n, size_t d, float* dev_pdx, size_t ld,
-                                         size_t cols, cudaStream_t s, LaunchCounter* launches);
+// n rows (row-major, device) -> columns [0, cols) of dst (cols >= n; columns past n are zero-filled)
+cudaError_t launch_transpose_rows_to_pdx(const float* dev_rows, size_t n, size_t d, const PdxDst& dst, size_t cols,
+                                         cudaStream_t s, LaunchCounter* launches);
 cudaError_t launch_generate_f32_pdx(int generator, uint64_t salt, uint64_t first_row, size_t n, size_t d,
-                                    float* dev_pdx, size_t ld, cudaStream_t s, LaunchCounter* launches);
+                                    const PdxDst& dst, cudaStream_t s, LaunchCounter* launches);
+// `rows` dimension rows of a plain PDX block (row pitch n, device) -> dimension rows [0, rows) of dst (columns past n
+// zero-filled up to dst.ld)
+cudaError_t launch_pdx_rows_to_dst(const float* dev_src, size_t rows, size_t n, const PdxDst& dst, cudaStream_t s,
+                                   LaunchCounter* launches);
+// per-row sidecar of a split corpus: dev_norms[i] = the reference's norm (PDX_NORMS bits), dev_lo_norm[i] >= ||lo_i||_2
+// (lo_i = x_i minus its high half, rounded up); *dev_nonfinite != 0 when some row's norm or bound is not finite
+cudaError_t launch_split_sidecar(const PdxView& v, float* dev_norms, float* dev_lo_norm, unsigned* dev_nonfinite,
+                                 cudaStream_t s, LaunchCounter* launches);
 
 // binary codes (hamming.cu): chunk-major layout codes[c * ld + i] (uint4 = 128 bits), chunks = ceil(words/2)
 struct BinView {
@@ -183,7 +228,7 @@ cudaError_t launch_hamming_topk(const BinView& v, const uint64_t* dev_query_word
                                 uint64_t* dev_keys, Workspace& ws, cudaStream_t s, LaunchCounter* launches);
 cudaError_t launch_encode_binary(const float* dev_values, size_t n, float threshold, uint64_t* dev_words,
                                  cudaStream_t s, LaunchCounter* launches);
-cudaError_t launch_binary_from_pdx(const float* dev_pdx, size_t ld_f, size_t n, size_t d, float threshold,
+cudaError_t launch_binary_from_pdx(const PdxView& v, float threshold,
                                    uint4* dev_codes, size_t ld, cudaStream_t s, LaunchCounter* launches);
 
 // ternary codes (ternary.cu): chunk-major layout codes[c * ld + i] (uint4 = 64 two-bit values), chunks = ceil(dim/64)
@@ -194,7 +239,7 @@ struct TerView {
 };
 cudaError_t launch_ternary_pack(const uint64_t* dev_words_rowmajor, size_t n, size_t words, size_t dim, uint4* dev_codes,
                                 size_t ld, cudaStream_t s, LaunchCounter* launches);
-cudaError_t launch_ternary_from_pdx(const float* dev_pdx, size_t ld_f, size_t n, size_t d, float threshold, uint4* dev_codes,
+cudaError_t launch_ternary_from_pdx(const PdxView& v, float threshold, uint4* dev_codes,
                                     size_t ld, cudaStream_t s, LaunchCounter* launches);
 cudaError_t launch_encode_ternary(const float* dev_values, size_t n, float threshold, uint64_t* dev_words, cudaStream_t s,
                                   LaunchCounter* launches);
@@ -215,7 +260,7 @@ cudaError_t launch_generate_u8(uint64_t salt, uint64_t first_row, size_t n, size
                                uint4* dev_codes, size_t ld, cudaStream_t s, LaunchCounter* launches);
 cudaError_t launch_quantize_u8(const float* dev_values, size_t n, float alpha, float offset, uint8_t* dev_out,
                                cudaStream_t s, LaunchCounter* launches);
-cudaError_t launch_u8_from_pdx(const float* dev_pdx, size_t ld_f, size_t n, size_t d, float alpha, float offset,
+cudaError_t launch_u8_from_pdx(const PdxView& v, float alpha, float offset,
                                uint4* dev_codes, size_t ld, cudaStream_t s, LaunchCounter* launches);
 // mode 0: raw mixed dot, 1: asymmetric score
 cudaError_t launch_u8_scores(const U8View& v, int mode, const float* dev_query, float* dev_out,

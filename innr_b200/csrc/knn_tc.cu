@@ -37,6 +37,7 @@
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "pdx.cuh"
 #include "tc_common.cuh"
 
 namespace innr {
@@ -319,7 +320,7 @@ __global__ void __launch_bounds__(KT_THREADS, 1) knn_tc_filter_kernel(const __gr
 }
 
 // ---- once per corpus: Xh[i][k] = f16(x[k][i] / ||x_i||) from the PDX corpus and its exact norms ----------------------
-__global__ void knn_tc_build_xh_kernel(const float* __restrict__ pdx, size_t ld, unsigned n, unsigned d, unsigned d_pad,
+__global__ void knn_tc_build_xh_kernel(const PdxView pdx, unsigned n, unsigned d, unsigned d_pad,
                                        const float* __restrict__ norms, __half* __restrict__ xh,
                                        unsigned* __restrict__ nonfinite) {
   __shared__ float tile[32][33];
@@ -339,7 +340,7 @@ __global__ void knn_tc_build_xh_kernel(const float* __restrict__ pdx, size_t ld,
 #pragma unroll
     for (int r = 0; r < 4; ++r) {
       const unsigned dd = d0 + ty * 4 + r, i = i0 + tx;
-      tile[ty * 4 + r][tx] = (dd < d && i < n) ? pdx[(size_t)dd * ld + i] : 0.0f;
+      tile[ty * 4 + r][tx] = (dd < d && i < n) ? pdx_load1(pdx, (size_t)dd * pdx.ld + i) : 0.0f;
     }
     __syncthreads();
 #pragma unroll
@@ -437,7 +438,7 @@ __global__ void knn_tc_select_kernel(unsigned nq, unsigned k, const unsigned* __
 constexpr int RS_THREADS = 256;
 
 template <int R>
-__global__ void __launch_bounds__(RS_THREADS) knn_tc_rescore_kernel(const float* __restrict__ data, size_t ld, unsigned n,
+__global__ void __launch_bounds__(RS_THREADS) knn_tc_rescore_kernel(const PdxView data, unsigned n,
                                                                     unsigned d, unsigned index_base,
                                                                     const float* __restrict__ queries, int cosine,
                                                                     int l2, float eps, const float* __restrict__ norms,
@@ -506,7 +507,7 @@ __global__ void __launch_bounds__(RS_THREADS) knn_tc_rescore_kernel(const float*
       valid = ub >= bound;
     }
     if (valid) {
-      const float* p = data + i;
+      const size_t p = i, ld = data.ld;
       float acc = 0.0f, ss = 0.0f;
       unsigned dd = 0;
       // the reference's sequential unfused sums (src/batch.rs:257-265, 290-296, 676-681), 8 rows in flight per thread
@@ -515,7 +516,7 @@ __global__ void __launch_bounds__(RS_THREADS) knn_tc_rescore_kernel(const float*
       for (; dd + 8 <= d; dd += 8) {
         float v[8];
 #pragma unroll
-        for (int u = 0; u < 8; ++u) v[u] = __ldg(p + (size_t)(dd + u) * ld);
+        for (int u = 0; u < 8; ++u) v[u] = pdx_load1(data, p + (size_t)(dd + u) * ld);
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
           if (l2) {
@@ -528,7 +529,7 @@ __global__ void __launch_bounds__(RS_THREADS) knn_tc_rescore_kernel(const float*
         }
       }
       for (; dd < d; ++dd) {
-        const float v = __ldg(p + (size_t)dd * ld);
+        const float v = pdx_load1(data, p + (size_t)dd * ld);
         if (l2) {
           const float diff = __fsub_rn(sq[dd], v);
           acc = __fadd_rn(acc, __fmul_rn(diff, diff));
@@ -611,7 +612,7 @@ cudaError_t launch_knn_tc_build(const PdxView& v, const float* dev_norms, void* 
   const unsigned d_pad = (unsigned)knn_tc_dpad(v.d);
   cudaError_t e = cudaMemsetAsync(dev_scratch_u32, 0, 4, s);
   if (e != cudaSuccess) return e;
-  knn_tc_build_xh_kernel<<<(unsigned)((v.n + 31) / 32), dim3(32, 8), 0, s>>>(v.data, v.ld, (unsigned)v.n, (unsigned)v.d, d_pad,
+  knn_tc_build_xh_kernel<<<(unsigned)((v.n + 31) / 32), dim3(32, 8), 0, s>>>(v, (unsigned)v.n, (unsigned)v.d, d_pad,
                                                                              dev_norms, (__half*)dev_xh, dev_scratch_u32);
   ++*launches;
   e = cudaGetLastError();
@@ -817,11 +818,11 @@ cudaError_t launch_pdx_knn_tc(const PdxView& v, const CUtensorMap& tm_xh, const 
   // 3. exact rescoring + selection
   const size_t rs_smem = ((v.d + 3) & ~(size_t)3) * 4 + (size_t)(RS_THREADS / 32) * k * 8;
   if (k <= 32)
-    knn_tc_rescore_kernel<1><<<(unsigned)nq, RS_THREADS, rs_smem, s>>>(v.data, v.ld, (unsigned)v.n, (unsigned)v.d, v.index_base,
+    knn_tc_rescore_kernel<1><<<(unsigned)nq, RS_THREADS, rs_smem, s>>>(v, (unsigned)v.n, (unsigned)v.d, v.index_base,
                                                                        dev_queries, cosine, l2, a.eps, dev_norms, qflag, cnt, cand_idx,
                                                                        cand_lb, (int)k, dev_keys);
   else
-    knn_tc_rescore_kernel<4><<<(unsigned)nq, RS_THREADS, rs_smem, s>>>(v.data, v.ld, (unsigned)v.n, (unsigned)v.d, v.index_base,
+    knn_tc_rescore_kernel<4><<<(unsigned)nq, RS_THREADS, rs_smem, s>>>(v, (unsigned)v.n, (unsigned)v.d, v.index_base,
                                                                        dev_queries, cosine, l2, a.eps, dev_norms, qflag, cnt, cand_idx,
                                                                        cand_lb, (int)k, dev_keys);
   ++*launches;

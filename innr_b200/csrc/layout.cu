@@ -7,6 +7,7 @@
 // Generators are stateless so any row can be re-derived on the CPU by the oracle without holding the corpus.
 #include "common.cuh"
 #include "kernels.cuh"
+#include "pdx.cuh"
 
 namespace innr {
 
@@ -14,8 +15,8 @@ namespace {
 
 // rows: n x d row-major (a chunk of the corpus); pdx: first column of the chunk inside the PDX matrix (row pitch ld);
 // columns [0, cols) are written (cols >= n: the tail of the last chunk zero-fills the pitch padding)
-__global__ void transpose_rows_to_pdx_kernel(const float* __restrict__ rows, unsigned n, unsigned d,
-                                             float* __restrict__ pdx, size_t ld, unsigned cols) {
+__global__ void transpose_rows_to_pdx_kernel(const float* __restrict__ rows, unsigned n, unsigned d, const PdxDst dst,
+                                             unsigned cols) {
   __shared__ float tile[32][33];
   const unsigned i0 = blockIdx.x * 32, d0 = blockIdx.y * 32;
   // read rows[i][d0 + tx] coalesced along d
@@ -27,13 +28,13 @@ __global__ void transpose_rows_to_pdx_kernel(const float* __restrict__ rows, uns
   // write pdx[dd][i0 + tx] coalesced along i
   for (unsigned r = threadIdx.y; r < 32; r += blockDim.y) {
     unsigned dd = d0 + r, i = i0 + threadIdx.x;
-    if (dd < d && i < cols) pdx[(size_t)dd * ld + i] = tile[threadIdx.x][r];
+    if (dd < d && i < cols) pdx_store1(dst.data, dst.hi, dst.lo, (size_t)dd * dst.ld + i, tile[threadIdx.x][r]);
   }
 }
 
 __global__ void generate_f32_pdx_kernel(int generator, uint64_t salt, uint64_t first_row, unsigned n, unsigned d,
-                                        float* __restrict__ pdx, size_t ld) {
-  const size_t total = (size_t)d * ld;
+                                        const PdxDst dst) {
+  const size_t ld = dst.ld, total = (size_t)d * ld;
   for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
     const size_t dd = t / ld, i = t % ld;
     float v = 0.0f;
@@ -41,8 +42,35 @@ __global__ void generate_f32_pdx_kernel(int generator, uint64_t salt, uint64_t f
       const uint64_t row = first_row + i;
       v = generator == 0 ? ghash_value(salt, row * d + dd) : gref_value(salt + row, dd);
     }
-    pdx[t] = v;
+    pdx_store1(dst.data, dst.hi, dst.lo, t, v);
   }
+}
+
+__global__ void pdx_rows_to_dst_kernel(const float* __restrict__ src, unsigned rows, unsigned n, const PdxDst dst) {
+  const size_t total = (size_t)rows * dst.ld;
+  for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+    const size_t dd = t / dst.ld, i = t % dst.ld;
+    pdx_store1(dst.data, dst.hi, dst.lo, t, i < n ? src[dd * n + i] : 0.0f);
+  }
+}
+
+// r_i >= ||x_i - hi(x_i)||_2: the low halves are exact f32 differences, squared and summed rounding upward, so the
+// result bounds the true norm from above (also when the squares underflow). A norm or bound that is not finite
+// (inf / NaN elements, overflowing sums) marks the corpus as one the screened kNN must not take.
+__global__ void split_sidecar_kernel(const PdxView v, const float* __restrict__ norms, float* __restrict__ lo_norm,
+                                     unsigned* __restrict__ nonfinite) {
+  const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= v.n) return;
+  float acc = 0.0f;
+  for (unsigned dd = 0; dd < v.d; ++dd) {
+    const size_t off = (size_t)dd * v.ld + i;
+    const float x = pdx_load1(v, off), h = __uint_as_float((uint32_t)v.hi[off] << 16);
+    const float l = __fsub_rn(x, h);  // exact (Sterbenz; exact in the subnormal range too)
+    acc = __fmaf_ru(l, l, acc);
+  }
+  const float r = __fsqrt_ru(acc);
+  lo_norm[i] = r;
+  if (!isfinite(r) || !isfinite(norms[i])) atomicOr(nonfinite, 1u);
 }
 
 __global__ void generate_tokens_kernel(uint64_t salt, uint64_t first_row, size_t n_rows, unsigned dim,
@@ -54,19 +82,36 @@ __global__ void generate_tokens_kernel(uint64_t salt, uint64_t first_row, size_t
 
 }  // namespace
 
-cudaError_t launch_transpose_rows_to_pdx(const float* dev_rows, size_t n, size_t d, float* dev_pdx, size_t ld,
-                                         size_t cols, cudaStream_t s, LaunchCounter* launches) {
+cudaError_t launch_transpose_rows_to_pdx(const float* dev_rows, size_t n, size_t d, const PdxDst& dst, size_t cols,
+                                         cudaStream_t s, LaunchCounter* launches) {
   if (cols == 0 || d == 0) return cudaSuccess;
   dim3 grid((unsigned)((cols + 31) / 32), (unsigned)((d + 31) / 32));
-  transpose_rows_to_pdx_kernel<<<grid, dim3(32, 8), 0, s>>>(dev_rows, (unsigned)n, (unsigned)d, dev_pdx, ld, (unsigned)cols);
+  transpose_rows_to_pdx_kernel<<<grid, dim3(32, 8), 0, s>>>(dev_rows, (unsigned)n, (unsigned)d, dst, (unsigned)cols);
   ++*launches;
   return cudaGetLastError();
 }
 
 cudaError_t launch_generate_f32_pdx(int generator, uint64_t salt, uint64_t first_row, size_t n, size_t d,
-                                    float* dev_pdx, size_t ld, cudaStream_t s, LaunchCounter* launches) {
+                                    const PdxDst& dst, cudaStream_t s, LaunchCounter* launches) {
   if (n == 0 || d == 0) return cudaSuccess;
-  generate_f32_pdx_kernel<<<148 * 16, 256, 0, s>>>(generator, salt, first_row, (unsigned)n, (unsigned)d, dev_pdx, ld);
+  generate_f32_pdx_kernel<<<148 * 16, 256, 0, s>>>(generator, salt, first_row, (unsigned)n, (unsigned)d, dst);
+  ++*launches;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pdx_rows_to_dst(const float* dev_src, size_t rows, size_t n, const PdxDst& dst, cudaStream_t s,
+                                   LaunchCounter* launches) {
+  if (rows == 0) return cudaSuccess;
+  pdx_rows_to_dst_kernel<<<148 * 16, 256, 0, s>>>(dev_src, (unsigned)rows, (unsigned)n, dst);
+  ++*launches;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_split_sidecar(const PdxView& v, float* dev_norms, float* dev_lo_norm, unsigned* dev_nonfinite,
+                                 cudaStream_t s, LaunchCounter* launches) {
+  cudaError_t e = cudaMemsetAsync(dev_nonfinite, 0, sizeof(unsigned), s);
+  if (e != cudaSuccess || v.n == 0) return e;
+  split_sidecar_kernel<<<(unsigned)((v.n + 255) / 256), 256, 0, s>>>(v, dev_norms, dev_lo_norm, dev_nonfinite);
   ++*launches;
   return cudaGetLastError();
 }

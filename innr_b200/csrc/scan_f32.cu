@@ -18,9 +18,12 @@
 // Selection never materialises N scores: scores become 64-bit composite keys (common.cuh) and flow into a
 // per-warp register list, a CTA merge and a last-CTA merge -- one launch per query group.
 #include <algorithm>
+#include <cmath>
+#include <type_traits>
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "pdx.cuh"
 
 namespace innr {
 
@@ -32,7 +35,7 @@ constexpr int TILE = SCAN_THREADS * VPT;      // vectors per CTA tile
 constexpr float NORM_EPS = 1e-9f;             // crate::NORM_EPSILON, src/lib.rs:178
 
 struct PdxArgs {
-  const float* data;
+  PdxView v;
   unsigned long long ld;
   unsigned n, d, ld4;     // ld4 = ld (u32 copy for bounds checks; ld < 2^32)
   unsigned n_tiles;
@@ -50,6 +53,7 @@ struct PdxArgs {
   const uint32_t* perm;   // PDX_L2_PERM: the order in which the dimension rows are accumulated (batch_knn_reordered)
   float threshold;        // PDX_L2_PRUNE
   float one;              // 1.0f, opaque to the compiler (see add2_unfusable)
+  const unsigned* run_flag;  // non-null: the launch returns at once unless *run_flag != 0
 };
 
 template <int MODE>
@@ -95,6 +99,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) pdx_scan_kernel(const PdxArgs a_
   uint64_t* smem_keys = reinterpret_cast<uint64_t*>(s_perm + (PERM ? d_pad : 0u));
 
   const int lane = threadIdx.x & 31;
+  if (a_in.run_flag && *a_in.run_flag == 0) return;  // the whole grid leaves: no ticket is taken
 
   // query group of this CTA (grid.y): shifts the query, output and merge-workspace pointers
   PdxArgs a = a_in;
@@ -205,13 +210,15 @@ __global__ void __launch_bounds__(SCAN_THREADS) pdx_scan_kernel(const PdxArgs a_
         mx[3] = fmaxf(mx[3], p3);
       }
     };
-    if (active) {
-      const float* p = a.data + i0;
+    // the layout branch is taken once per tile, so each loop below holds loads of one kind only
+    auto rows = [&](auto split) {
+      constexpr bool SPLIT = decltype(split)::value;
+      size_t p = i0;
       unsigned dd = 0;
       for (; dd + U <= a.d; dd += U) {
         float4 v[U];
 #pragma unroll
-        for (int u = 0; u < U; ++u) v[u] = ldg_stream_f4(PERM ? p + (size_t)s_perm[dd + u] * a.ld : p + (size_t)u * a.ld);
+        for (int u = 0; u < U; ++u) v[u] = pdx_load4_as<SPLIT>(a.v, PERM ? i0 + (size_t)s_perm[dd + u] * a.ld : p + (size_t)u * a.ld);
         if (!PERM) p += (size_t)U * a.ld;
 #pragma unroll
         for (int u = 0; u < U; ++u) step(v[u], dd + u);
@@ -221,10 +228,14 @@ __global__ void __launch_bounds__(SCAN_THREADS) pdx_scan_kernel(const PdxArgs a_
         }
       }
       for (; dd < a.d; ++dd) {  // D % U tail
-        const float4 v = ldg_stream_f4(PERM ? p + (size_t)s_perm[dd] * a.ld : p);
+        const float4 v = pdx_load4_as<SPLIT>(a.v, PERM ? i0 + (size_t)s_perm[dd] * a.ld : p);
         if (!PERM) p += a.ld;
         step(v, dd);
       }
+    };
+    if (active) {
+      if (a.v.hi) rows(std::true_type{});
+      else rows(std::false_type{});
     }
     float acc[QB][VPT];
     float ss[VPT];
@@ -348,7 +359,7 @@ namespace {
 // multiple of 4, so the last float4 is in bounds); a prefix view (n << ld) scans only its own columns.
 PdxArgs base_args(const PdxView& v, const Workspace& ws, size_t k) {
   PdxArgs a{};
-  a.data = v.data;
+  a.v = v;
   a.ld = v.ld;
   a.ld4 = (unsigned)std::min<size_t>(v.ld, (v.n + 3) / 4 * 4);
   a.n = (unsigned)v.n;
@@ -366,8 +377,10 @@ PdxArgs base_args(const PdxView& v, const Workspace& ws, size_t k) {
 }  // namespace
 
 cudaError_t launch_pdx_knn(const PdxView& v, int mode, const float* dev_queries, size_t nq, size_t k,
-                           uint64_t* dev_keys, Workspace& ws, cudaStream_t s, LaunchCounter* launches) {
+                           uint64_t* dev_keys, Workspace& ws, cudaStream_t s, LaunchCounter* launches,
+                           const unsigned* dev_run_flag) {
   PdxArgs a = base_args(v, ws, k);
+  a.run_flag = dev_run_flag;
   const bool big_k = k > 32;
   // query blocking: 8 queries share one pass over the corpus when their lists fit in registers; several groups of 8
   // run as grid.y of ONE launch as long as their merge workspaces fit (small corpora / many queries: C1, sample pass)
@@ -476,29 +489,29 @@ constexpr int VAR_UV = 4;  // 128-value groups per step (512 values: 2 KB of sha
 // The warp loads 512 consecutive values per step (the next step's loads are issued before this step's chain runs),
 // parks them in shared memory, and every lane replays the chain from broadcast 128-bit reads.
 template <bool CENTERED>
-__device__ __forceinline__ float row_chain(const float* row, unsigned n, float mean, int lane, float4* buf) {
+__device__ __forceinline__ float row_chain(const PdxView& v, size_t row, unsigned n, float mean, int lane, float4* buf) {
   float acc = 0.0f;
   constexpr unsigned STEP = 128u * VAR_UV;
   const unsigned n_steps = n / STEP;
   float4 cur[VAR_UV], nxt[VAR_UV];
   if (n_steps) {
 #pragma unroll
-    for (int u = 0; u < VAR_UV; ++u) cur[u] = ldg_stream_f4(row + 128u * u + 4u * lane);
+    for (int u = 0; u < VAR_UV; ++u) cur[u] = pdx_load4(v, row + 128u * u + 4u * lane);
   }
   for (unsigned st = 0; st < n_steps; ++st) {
     if (st + 1 < n_steps) {
-      const float* p = row + (size_t)(st + 1) * STEP + 4u * lane;
+      const size_t p = row + (size_t)(st + 1) * STEP + 4u * lane;
 #pragma unroll
-      for (int u = 0; u < VAR_UV; ++u) nxt[u] = ldg_stream_f4(p + 128u * u);
+      for (int u = 0; u < VAR_UV; ++u) nxt[u] = pdx_load4(v, p + 128u * u);
     }
 #pragma unroll
     for (int u = 0; u < VAR_UV; ++u) {
-      float4 v = cur[u];
+      float4 x = cur[u];
       if (CENTERED) {  // computed once per value by the lane that loaded it
-        v.x = __fsub_rn(v.x, mean); v.y = __fsub_rn(v.y, mean); v.z = __fsub_rn(v.z, mean); v.w = __fsub_rn(v.w, mean);
-        v.x = __fmul_rn(v.x, v.x); v.y = __fmul_rn(v.y, v.y); v.z = __fmul_rn(v.z, v.z); v.w = __fmul_rn(v.w, v.w);
+        x.x = __fsub_rn(x.x, mean); x.y = __fsub_rn(x.y, mean); x.z = __fsub_rn(x.z, mean); x.w = __fsub_rn(x.w, mean);
+        x.x = __fmul_rn(x.x, x.x); x.y = __fmul_rn(x.y, x.y); x.z = __fmul_rn(x.z, x.z); x.w = __fmul_rn(x.w, x.w);
       }
-      buf[u * 32 + lane] = v;
+      buf[u * 32 + lane] = x;
     }
     __syncwarp();
 #pragma unroll 16
@@ -515,24 +528,24 @@ __device__ __forceinline__ float row_chain(const float* row, unsigned n, float m
   }
 #pragma unroll 8
   for (unsigned i = n_steps * STEP; i < n; ++i) {  // tail (< 512 values): every lane reads the same value
-    float x = __ldg(row + i);
+    float x = pdx_load1(v, row + i);
     if (CENTERED) { x = __fsub_rn(x, mean); x = __fmul_rn(x, x); }
     acc = __fadd_rn(acc, x);
   }
   return acc;
 }
 
-__global__ void __launch_bounds__(VAR_WARPS * 32) dimension_variance_kernel(const float* __restrict__ data, size_t ld,
-                                                                            unsigned n, unsigned d, float* __restrict__ out) {
+__global__ void __launch_bounds__(VAR_WARPS * 32) dimension_variance_kernel(const PdxView v, unsigned n, unsigned d,
+                                                                            float* __restrict__ out) {
   __shared__ float4 s_buf[VAR_WARPS][VAR_UV * 32];
   const unsigned dd = blockIdx.x * VAR_WARPS + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (dd >= d) return;
   float4* buf = s_buf[threadIdx.x >> 5];
-  const float* row = data + (size_t)dd * ld;
+  const size_t row = (size_t)dd * v.ld;
   const float nf = (float)n;                                     // let n = batch.num_vectors as f32;
-  const float mean = __fdiv_rn(row_chain<false>(row, n, 0.0f, lane, buf), nf);
-  const float var = __fdiv_rn(row_chain<true>(row, n, mean, lane, buf), nf);
+  const float mean = __fdiv_rn(row_chain<false>(v, row, n, 0.0f, lane, buf), nf);
+  const float var = __fdiv_rn(row_chain<true>(v, row, n, mean, lane, buf), nf);
   if (lane == 0) out[dd] = var;
 }
 
@@ -541,8 +554,8 @@ __global__ void __launch_bounds__(VAR_WARPS * 32) dimension_variance_kernel(cons
 cudaError_t launch_dimension_variance(const PdxView& v, float* dev_out, cudaStream_t s, LaunchCounter* launches) {
   if (v.d == 0) return cudaSuccess;
   if (v.n <= 1) return cudaMemsetAsync(dev_out, 0, v.d * sizeof(float), s);  // src/batch.rs:573-575
-  dimension_variance_kernel<<<(unsigned)((v.d + VAR_WARPS - 1) / VAR_WARPS), VAR_WARPS * 32, 0, s>>>(v.data, v.ld, (unsigned)v.n,
-                                                                                                  (unsigned)v.d, dev_out);
+  dimension_variance_kernel<<<(unsigned)((v.d + VAR_WARPS - 1) / VAR_WARPS), VAR_WARPS * 32, 0, s>>>(v, (unsigned)v.n, (unsigned)v.d,
+                                                                                                  dev_out);
   ++*launches;
   return cudaGetLastError();
 }
@@ -801,7 +814,7 @@ namespace {
 // src/scalar.rs:366-368, examples/binary_demo.rs:235-237). One thread per candidate, the reference's sequential unfused
 // arithmetic (same bits as the full scan); out-of-range candidates score the metric's worst value.
 template <int MODE>
-__global__ void __launch_bounds__(SCAN_THREADS) subset_scores_kernel(const float* __restrict__ data, size_t ld, unsigned n,
+__global__ void __launch_bounds__(SCAN_THREADS) subset_scores_kernel(const PdxView v, unsigned n,
                                                                     unsigned d, unsigned index_base,
                                                                     const float* __restrict__ query,
                                                                     const uint32_t* __restrict__ cand, unsigned m,
@@ -824,12 +837,11 @@ __global__ void __launch_bounds__(SCAN_THREADS) subset_scores_kernel(const float
     out[j] = MODE == PDX_L2 ? __int_as_float(0x7FC00000) : __int_as_float(0xFFC00000);  // sorts last under total_cmp
     return;
   }
-  const float* p = data + i;
   float acc = 0.0f, ss = 0.0f;
   for (unsigned dd = 0; dd < d; ++dd) {
-    const float v = __ldg(p + (size_t)dd * ld);
-    accumulate<MODE == PDX_COSINE_FUSED ? PDX_DOT : MODE>(sq[dd], v, acc);
-    if (MODE == PDX_COSINE_FUSED) ss = __fadd_rn(ss, __fmul_rn(v, v));
+    const float x = pdx_load1(v, (size_t)dd * v.ld + i);
+    accumulate<MODE == PDX_COSINE_FUSED ? PDX_DOT : MODE>(sq[dd], x, acc);
+    if (MODE == PDX_COSINE_FUSED) ss = __fadd_rn(ss, __fmul_rn(x, x));
   }
   float sc = acc;
   if (MODE == PDX_COSINE_FUSED) {
@@ -853,7 +865,7 @@ cudaError_t launch_subset_scores(const PdxView& v, int mode, const float* dev_qu
       cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);           \
       if (e != cudaSuccess) return e;                                                                               \
     }                                                                                                               \
-    kern<<<grid, SCAN_THREADS, smem, s>>>(v.data, v.ld, (unsigned)v.n, (unsigned)v.d, v.index_base, dev_query,      \
+    kern<<<grid, SCAN_THREADS, smem, s>>>(v, (unsigned)v.n, (unsigned)v.d, v.index_base, dev_query,                 \
                                           dev_cand, (unsigned)m, dev_out);                                          \
   }
   if (mode == PDX_DOT) INNR_SUBSET(PDX_DOT)
@@ -941,7 +953,7 @@ cudaError_t launch_merge_keys_big(const uint64_t* dev_in, size_t n_lists, size_t
 namespace {
 
 struct AdaptArgs {
-  const float* data;
+  PdxView v;
   unsigned long long ld;
   unsigned ld4;
   const float* query;
@@ -970,7 +982,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) adaptive_epoch_kernel(const Adap
     float4 acc = *reinterpret_cast<const float4*>(a.dist + i0);
     const float T = a.thr[0];
     unsigned ex = 0, e0 = 0, e1 = 0, e2 = 0, e3 = 0;
-    const float* p = a.data + (size_t)a.d0 * a.ld + i0;
+    size_t p = (size_t)a.d0 * a.ld + i0;
     auto step = [&](const float4& v, unsigned j) {
       const float q = sq[j];
       float df;
@@ -988,13 +1000,13 @@ __global__ void __launch_bounds__(SCAN_THREADS) adaptive_epoch_kernel(const Adap
     for (; j + U <= nd; j += U) {
       float4 v[U];
 #pragma unroll
-      for (int u = 0; u < U; ++u) v[u] = ldg_stream_f4(p + (size_t)u * a.ld);
+      for (int u = 0; u < U; ++u) v[u] = pdx_load4(a.v, p + (size_t)u * a.ld);
       p += (size_t)U * a.ld;
 #pragma unroll
       for (int u = 0; u < U; ++u) step(v[u], j + u);
     }
     for (; j < nd; ++j) {
-      const float4 v = ldg_stream_f4(p);
+      const float4 v = pdx_load4(a.v, p);
       p += a.ld;
       step(v, j);
     }
@@ -1088,7 +1100,7 @@ cudaError_t launch_adaptive_epoch(const PdxView& v, const float* dev_query, size
                                   const uint32_t* dev_mask_in, uint32_t* dev_mask_out, const float* dev_thr, uint32_t* dev_ev,
                                   unsigned* dev_pruned, int no_prune, cudaStream_t s, LaunchCounter* launches) {
   AdaptArgs a{};
-  a.data = v.data;
+  a.v = v;
   a.ld = v.ld;
   a.ld4 = (unsigned)std::min<size_t>(v.ld, (v.n + 3) / 4 * 4);
   a.query = dev_query;
@@ -1127,6 +1139,378 @@ cudaError_t launch_adaptive_revive(const uint64_t* dev_keys, size_t m, uint32_t*
 cudaError_t launch_topk_from_distances(const float* dev_dist, size_t n, size_t k, uint64_t* dev_keys,
                                        Workspace& ws, cudaStream_t s, LaunchCounter* launches) {
   return launch_topk_from_scores(dev_dist, 0, n, 0, k, dev_keys, ws, s, launches, nullptr, nullptr, 1, 1);
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Screened single-query kNN of a split corpus (DESIGN.md section 3.1). Three steps, all on the device:
+//  1. screen: stream the hi plane only; for each row an interval [lower, upper] that holds the reference's score.
+//     Selection on the pessimistic bound (lower for dot / cosine, upper for L2) gives T, its k-th best value; every row
+//     gets its optimistic bound written to ws.sc_bounds.
+//  2. compaction: the rows whose optimistic bound reaches T. At least k rows have a score at least as good as T, so
+//     every row of the top k (ties on the k-th score included) is among them.
+//  3. rescoring from both planes with the reference's sequential unfused arithmetic, selection on the scan's keys.
+// The bound (scores are d-term f32 sums; u = 2^-24, g = gamma of the launch >= (d + 2) u / (1 - (d + 2) u)):
+//  dot:    |ref - s| <= |q| (r + g (2 |v| + r)) + 2 d 2^-149, s = the screen's sum of q * hi (any order, fused);
+//          |v| <= (nrm (1 + 2u) + nu) (1 + g) with nu = sqrt(d 2^-149) (the reference norm's rounding and underflow).
+//  cosine: ref = RN(dot / P) with P = RN(qn * nrm) computed here with the reference's bits; RN(x / P) is monotone in x.
+//  L2:     a = |q - hi| from the screen's sum A: a^2 in [(A - eta)(1 - g), (A + eta)(1 + 2g)], the exact distance in
+//          [(a - r)^2, (a + r)^2], the reference's within (1 +- g) of it plus eta.
+// Every step rounds outward (RD / RU); a bound that is not finite, or a product |q| |v| past 2^100, makes the row a
+// candidate whatever T is.
+// ---------------------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int SC_VPT = 8;                       // vectors per thread: one 16 B load of the hi plane
+constexpr int SC_TILE = SCAN_THREADS * SC_VPT;  // vectors per CTA tile
+constexpr int SC_U = 8;                         // hi-plane rows in flight per thread
+constexpr int RS_WARPS = 4;                     // rescoring: warps per CTA, one candidate per warp
+
+struct ScreenArgs {
+  const uint16_t* hi;
+  unsigned long long ld;
+  unsigned n, d, ld8, n_tiles, index_base;
+  int k;
+  const float* query;
+  const float* norms;    // the reference's norm of each row
+  const float* lo_norm;  // r_i >= |lo_i|
+  float gamma, eta, nu;
+  uint64_t* partials;
+  uint64_t* group_partials;
+  unsigned* tickets;
+  uint64_t* tkeys;       // out: the k keys of the pessimistic bounds
+  float* opt;            // out: optimistic bound of every row
+  float* pess;           // out (test hook only, may be null): pessimistic bound of every row
+  unsigned* ctl;         // ctl[1] = 1: the query cannot be screened
+};
+
+__device__ __forceinline__ void hi8(const uint4& w, float (&h)[8]) {
+  const unsigned x[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    h[2 * t] = __uint_as_float(x[t] << 16);
+    h[2 * t + 1] = __uint_as_float(x[t] & 0xFFFF0000u);
+  }
+}
+
+template <int MODE>
+__device__ __forceinline__ void screen_bounds(float s, float nv, float r, float qn_ref, float qn_up, const ScreenArgs& a,
+                                              float& lower, float& upper) {
+  const float g = a.gamma;
+  if (MODE == PDX_L2) {
+    const float a2_up = __fmul_ru(__fadd_ru(s, a.eta), __fadd_ru(1.0f, __fmul_ru(2.0f, g)));
+    const float a2_lo = fmaxf(0.0f, __fmul_rd(__fsub_rd(s, a.eta), __fsub_rd(1.0f, g)));
+    const float t_lo = fmaxf(0.0f, __fsub_rd(__fsqrt_rd(a2_lo), r));
+    const float t_up = __fadd_ru(__fsqrt_ru(a2_up), r);
+    lower = fmaxf(0.0f, __fsub_rd(__fmul_rd(__fmul_rd(t_lo, t_lo), __fsub_rd(1.0f, g)), a.eta));
+    upper = __fadd_ru(__fmul_ru(__fmul_ru(t_up, t_up), __fadd_ru(1.0f, g)), a.eta);
+    if (!(upper <= 3.0e38f)) { lower = -INFINITY; upper = INFINITY; }
+    return;
+  }
+  const float v_up = __fmul_ru(__fadd_ru(__fmul_ru(nv, 1.0f + 2.0f / 16777216.0f), a.nu), __fadd_ru(1.0f, g));
+  const float e = __fadd_ru(__fmul_ru(qn_up, __fadd_ru(r, __fmul_ru(g, __fadd_ru(__fmul_ru(2.0f, v_up), r)))), __fmul_ru(2.0f, a.eta));
+  if (!(__fmul_ru(qn_up, v_up) <= 0x1p100f) || !(fabsf(s) <= 0x1p100f)) {
+    lower = -INFINITY;
+    upper = INFINITY;
+    return;
+  }
+  lower = __fsub_rd(s, e);
+  upper = __fadd_ru(s, e);
+  if (MODE == PDX_COSINE_FUSED) {
+    if (!(nv > NORM_EPS)) {  // the reference's score is exactly 0 (src/batch.rs:716-727)
+      lower = upper = 0.0f;
+      return;
+    }
+    const float p = __fmul_rn(qn_ref, nv);
+    lower = __fdiv_rd(lower, p);
+    upper = __fdiv_ru(upper, p);
+  }
+}
+
+template <int MODE, int R>
+__global__ void __launch_bounds__(SCAN_THREADS) pdx_screen_kernel(const ScreenArgs a) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const unsigned d_pad = (a.d + 31u) / 32u * 32u;
+  float* sq = reinterpret_cast<float*>(smem_raw);
+  float* s_qn = sq + d_pad;  // [0] the reference's query norm, [1] an upper bound on |q|
+  uint64_t* smem_keys = reinterpret_cast<uint64_t*>(s_qn + 4);
+  const int lane = threadIdx.x & 31;
+  for (unsigned dd = threadIdx.x; dd < d_pad; dd += blockDim.x) sq[dd] = dd < a.d ? a.query[dd] : 0.0f;
+  __syncthreads();
+  // both norms are d-long chains: the last thread computes them while the others stream (read after the first tile)
+  if (threadIdx.x == SCAN_THREADS - 1) {
+    float ss = 0.0f, su = 0.0f;
+    for (unsigned dd = 0; dd < a.d; ++dd) {
+      const float x = sq[dd];
+      ss = __fadd_rn(ss, __fmul_rn(x, x));
+      su = __fmaf_ru(x, x, su);
+    }
+    s_qn[0] = __fsqrt_rn(ss);
+    s_qn[1] = __fsqrt_ru(su);
+  }
+  bool qn_visible = false;
+  WarpList<R> lists[1];
+  lists[0].init();
+  uint64_t thr = KEY_SENTINEL;
+
+  for (unsigned tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
+    const unsigned i0 = tile * SC_TILE + threadIdx.x * SC_VPT;
+    const bool active = i0 < a.ld8;
+    float acc[SC_VPT];
+#pragma unroll
+    for (int j = 0; j < SC_VPT; ++j) acc[j] = 0.0f;
+    auto step = [&](const uint4& w, unsigned dd) {
+      float h[8];
+      hi8(w, h);
+      const float q = sq[dd];
+#pragma unroll
+      for (int j = 0; j < SC_VPT; ++j) {
+        if (MODE == PDX_L2) {
+          const float t = q - h[j];
+          acc[j] = fmaf(t, t, acc[j]);
+        } else {
+          acc[j] = fmaf(q, h[j], acc[j]);
+        }
+      }
+    };
+    if (active) {
+      const uint16_t* p = a.hi + i0;
+      unsigned dd = 0;
+      for (; dd + SC_U <= a.d; dd += SC_U) {
+        uint4 w[SC_U];
+#pragma unroll
+        for (int u = 0; u < SC_U; ++u) w[u] = ldg_stream_u4(reinterpret_cast<const uint4*>(p + (size_t)u * a.ld));
+        p += (size_t)SC_U * a.ld;
+#pragma unroll
+        for (int u = 0; u < SC_U; ++u) step(w[u], dd + u);
+      }
+      for (; dd < a.d; ++dd) {
+        step(ldg_stream_u4(reinterpret_cast<const uint4*>(p)), dd);
+        p += a.ld;
+      }
+    }
+    if (!qn_visible) {  // first tile of this CTA (CTA-uniform)
+      __syncthreads();
+      qn_visible = true;
+      const float qr = s_qn[0], qu = s_qn[1];
+      // a query the bound cannot take: every CTA sees the same and leaves before taking a ticket
+      if (!(qu <= 0x1p100f) || (MODE == PDX_COSINE_FUSED && !(qr >= NORM_EPS))) {
+        if (threadIdx.x == 0) a.ctl[1] = 1u;
+        return;
+      }
+    }
+    const float qn_ref = s_qn[0], qn_up = s_qn[1];
+    float nv[SC_VPT], r[SC_VPT];
+    if (active) {
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const float4 x = *reinterpret_cast<const float4*>(a.norms + i0 + 4 * h);
+        const float4 y = *reinterpret_cast<const float4*>(a.lo_norm + i0 + 4 * h);
+        nv[4 * h] = x.x; nv[4 * h + 1] = x.y; nv[4 * h + 2] = x.z; nv[4 * h + 3] = x.w;
+        r[4 * h] = y.x; r[4 * h + 1] = y.y; r[4 * h + 2] = y.z; r[4 * h + 3] = y.w;
+      }
+    }
+    float lo[SC_VPT], up[SC_VPT];
+#pragma unroll
+    for (int j = 0; j < SC_VPT; ++j) {
+      lo[j] = up[j] = 0.0f;
+      if (active) screen_bounds<MODE>(acc[j], nv[j], r[j], qn_ref, qn_up, a, lo[j], up[j]);
+    }
+    if (active) {
+      float* o = a.opt + i0;
+      const float* ob = (MODE == PDX_L2) ? lo : up;
+      *reinterpret_cast<float4*>(o) = make_float4(ob[0], ob[1], ob[2], ob[3]);
+      *reinterpret_cast<float4*>(o + 4) = make_float4(ob[4], ob[5], ob[6], ob[7]);
+      if (a.pess) {
+        const float* pb = (MODE == PDX_L2) ? up : lo;
+        for (int j = 0; j < SC_VPT; ++j) a.pess[i0 + j] = pb[j];
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < SC_VPT; ++j) {
+      const unsigned i = i0 + j;
+      const uint64_t key = (MODE == PDX_L2) ? make_key_asc(up[j], a.index_base + i) : make_key_desc(lo[j], a.index_base + i);
+      lists[0].offer(key, active && i < a.n, thr, a.k, lane);
+    }
+  }
+  block_finish<R, 1>(lists, 1, a.k, smem_keys, a.partials, a.group_partials, a.tkeys, a.tickets);
+}
+
+// rows whose optimistic bound reaches T (a NaN bound counts as reaching it), in any order: the rescoring selects on keys
+__global__ void __launch_bounds__(SCAN_THREADS) screen_compact_kernel(const float* __restrict__ opt, unsigned n, int l2,
+                                                                      const uint64_t* __restrict__ tkeys, int k,
+                                                                      unsigned index_base, uint32_t* __restrict__ cand,
+                                                                      unsigned* ctl) {
+  if (ctl[1]) return;
+  const uint64_t kth = tkeys[k - 1];
+  float t;
+  if (kth == KEY_SENTINEL) t = l2 ? INFINITY : -INFINITY;
+  else t = __uint_as_float(order_bits_to_f32_bits(l2 ? (uint32_t)(kth >> 32) : ~(uint32_t)(kth >> 32)));
+  const int lane = threadIdx.x & 31;
+  const unsigned stride = gridDim.x * blockDim.x, n_round = (n + 31u) / 32u * 32u;
+  for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_round; i += stride) {
+    bool hit = false;
+    if (i < n) {
+      const float b = opt[i];
+      hit = l2 ? !(b > t) : !(b < t);
+    }
+    const unsigned m = __ballot_sync(FULL_MASK, hit);
+    if (!m) continue;
+    unsigned base = 0;
+    if (lane == 0) base = atomicAdd(&ctl[0], (unsigned)__popc(m));
+    base = __shfl_sync(FULL_MASK, base, 0);
+    const unsigned pos = base + __popc(m & ((1u << lane) - 1u));
+    if (hit && pos < SCREEN_CAP) cand[pos] = index_base + i;
+  }
+}
+
+// One warp per candidate: the 32 lanes gather both planes of the row at once into shared memory, then one lane runs the
+// reference's sequential chain (cosine divides by RN(qn * nrm) with the cached norm: the same bits as the fused scan's).
+// Writes SCREEN_CAP ready-made keys (KEY_SENTINEL past the candidates); more than SCREEN_CAP candidates raise ctl[1].
+template <int MODE>
+__global__ void __launch_bounds__(RS_WARPS * 32) screen_rescore_kernel(const PdxView v, const float* __restrict__ query,
+                                                                       const float* __restrict__ norms,
+                                                                       const uint32_t* __restrict__ cand,
+                                                                       unsigned* ctl, uint64_t* __restrict__ keys) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const unsigned d = (unsigned)v.d, d_pad = (d + 3u) & ~3u;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float* sq = reinterpret_cast<float*>(smem_raw) + (size_t)2 * d_pad * warp;  // this warp's query copy, then its row
+  float* buf = sq + d_pad;
+  const unsigned j = blockIdx.x * RS_WARPS + warp;
+  const unsigned cnt = ctl[0], stop = ctl[1];
+  if (j == 0 && lane == 0 && cnt > SCREEN_CAP) ctl[1] = 1u;
+  if (stop || j >= min(cnt, (unsigned)SCREEN_CAP)) {
+    if (lane == 0) keys[j] = KEY_SENTINEL;
+    return;
+  }
+  for (unsigned dd = lane; dd < d; dd += 32) sq[dd] = query[dd];
+  const unsigned gid = cand[j], i = gid - v.index_base;
+  for (unsigned dd = lane; dd < d; dd += 32) buf[dd] = pdx_load1(v, (size_t)dd * v.ld + i);
+  __syncwarp();
+  if (lane != 0) return;
+  float acc = 0.0f, qss = 0.0f;
+  for (unsigned dd = 0; dd < d; ++dd) {
+    const float q = sq[dd], x = buf[dd];
+    accumulate<MODE == PDX_COSINE_FUSED ? PDX_DOT : MODE>(q, x, acc);
+    if (MODE == PDX_COSINE_FUSED) qss = __fadd_rn(qss, __fmul_rn(q, q));
+  }
+  float sc = acc;
+  if (MODE == PDX_COSINE_FUSED) {
+    const float qn = __fsqrt_rn(qss), nrm = norms[i];
+    sc = (!(qn < NORM_EPS) && nrm > NORM_EPS) ? __fdiv_rn(acc, __fmul_rn(qn, nrm)) : 0.0f;
+  }
+  keys[j] = MODE == PDX_L2 ? make_key_asc(sc, gid) : make_key_desc(sc, gid);
+}
+
+ScreenArgs screen_args(const PdxView& v, const float* dev_norms, const float* dev_lo_norm, const float* dev_query, size_t k,
+                       Workspace& ws) {
+  ScreenArgs a{};
+  a.hi = v.hi;
+  a.ld = v.ld;
+  a.n = (unsigned)v.n;
+  a.d = (unsigned)v.d;
+  a.ld8 = (unsigned)std::min<size_t>(v.ld, (v.n + 7) / 8 * 8);
+  a.n_tiles = (unsigned)(((size_t)a.ld8 + SC_TILE - 1) / SC_TILE);
+  a.index_base = v.index_base;
+  a.k = (int)k;
+  a.query = dev_query;
+  a.norms = dev_norms;
+  a.lo_norm = dev_lo_norm;
+  // gamma_(d+2) = (d + 2) u / (1 - (d + 2) u), u = 2^-24, rounded up to f32 (double has room to spare)
+  const double du = (double)(v.d + 2) * 0x1p-24;
+  a.gamma = (float)(du / (1.0 - du)) * (1.0f + 0x1p-20f);
+  a.eta = (float)((double)v.d * 0x1p-148) * (1.0f + 0x1p-20f) + 0x1p-149f;
+  a.nu = (float)std::sqrt((double)v.d * 0x1p-149) * (1.0f + 0x1p-20f);
+  a.partials = ws.partials;
+  a.group_partials = ws.group_partials;
+  a.tickets = ws.tickets;
+  a.tkeys = ws.sc_keys + SCREEN_CAP;
+  a.opt = ws.sc_bounds;
+  a.ctl = ws.sc_ctl;
+  return a;
+}
+
+template <int MODE, int R>
+cudaError_t launch_screen(const ScreenArgs& a, int num_sms, cudaStream_t s) {
+  auto kern = pdx_screen_kernel<MODE, R>;
+  const size_t smem = ((a.d + 31u) / 32u * 32u + 4) * sizeof(float) + (size_t)(SCAN_THREADS / 32) * a.k * sizeof(uint64_t);
+  static size_t smem_set_dev[16] = {};
+  size_t& smem_set = smem_set_dev[current_device_slot()];
+  if (smem > 48 * 1024 && smem > smem_set) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    smem_set = smem;
+  }
+  int occ = 0;
+  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, SCAN_THREADS, smem);
+  if (e != cudaSuccess) return e;
+  if (occ < 1) return cudaErrorInvalidConfiguration;
+  kern<<<balanced_grid(a.n_tiles, (unsigned)occ * (unsigned)num_sms), SCAN_THREADS, smem, s>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_screen_mode(int mode, const ScreenArgs& a, int num_sms, cudaStream_t s) {
+  const bool big = a.k > 32;
+  switch (mode) {
+    case PDX_DOT: return big ? launch_screen<PDX_DOT, 4>(a, num_sms, s) : launch_screen<PDX_DOT, 1>(a, num_sms, s);
+    case PDX_COSINE_FUSED:
+      return big ? launch_screen<PDX_COSINE_FUSED, 4>(a, num_sms, s) : launch_screen<PDX_COSINE_FUSED, 1>(a, num_sms, s);
+    case PDX_L2: return big ? launch_screen<PDX_L2, 4>(a, num_sms, s) : launch_screen<PDX_L2, 1>(a, num_sms, s);
+  }
+  return cudaErrorInvalidValue;
+}
+
+}  // namespace
+
+cudaError_t launch_pdx_knn_screened(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+                                    const float* dev_query, size_t k, uint64_t* dev_keys, Workspace& ws, cudaStream_t s,
+                                    LaunchCounter* launches) {
+  if (!v.hi || k == 0 || k > 128 || v.d == 0 || v.d > SCREEN_MAX_D || v.n < k || ws.sc_bounds_cap < v.ld)
+    return cudaErrorInvalidValue;
+  const ScreenArgs a = screen_args(v, dev_norms, dev_lo_norm, dev_query, k, ws);
+  cudaError_t e = cudaMemsetAsync(ws.sc_ctl, 0, 2 * sizeof(unsigned), s);
+  if (e != cudaSuccess) return e;
+  if ((e = launch_screen_mode(mode, a, ws.num_sms, s)) != cudaSuccess) return e;
+  screen_compact_kernel<<<(unsigned)std::min<size_t>((v.n + SCAN_THREADS - 1) / SCAN_THREADS, (size_t)ws.num_sms * 8), SCAN_THREADS, 0, s>>>(
+      ws.sc_bounds, (unsigned)v.n, mode == PDX_L2, a.tkeys, (int)k, v.index_base, ws.sc_cand, ws.sc_ctl);
+  const size_t rs_smem = (size_t)(2 * RS_WARPS) * ((v.d + 3) & ~(size_t)3) * sizeof(float);
+#define INNR_RESCORE(MODE)                                                                                              \
+  {                                                                                                                     \
+    auto kern = screen_rescore_kernel<MODE>;                                                                            \
+    if (rs_smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem)) != cudaSuccess) \
+      return e;                                                                                                         \
+    kern<<<(unsigned)(SCREEN_CAP / RS_WARPS), RS_WARPS * 32, rs_smem, s>>>(v, dev_query, dev_norms, ws.sc_cand, ws.sc_ctl, ws.sc_keys); \
+  }
+  if (mode == PDX_DOT) INNR_RESCORE(PDX_DOT)
+  else if (mode == PDX_L2) INNR_RESCORE(PDX_L2)
+  else INNR_RESCORE(PDX_COSINE_FUSED)
+#undef INNR_RESCORE
+  *launches += 3;
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  if ((e = launch_topk_from_scores(ws.sc_keys, 3, SCREEN_CAP, 0, k, dev_keys, ws, s, launches)) != cudaSuccess) return e;
+  // the exact full-read scan, which returns at once unless the screen handed the query over
+  return launch_pdx_knn(v, mode, dev_query, 1, k, dev_keys, ws, s, launches, ws.sc_ctl + 1);
+}
+
+cudaError_t launch_pdx_screen_debug_bounds(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+                                           const float* dev_query, float* host_lower, float* host_upper, Workspace& ws,
+                                           cudaStream_t s, LaunchCounter* launches) {
+  if (!v.hi || v.n == 0 || v.d == 0 || v.d > SCREEN_MAX_D || 2 * v.ld > ws.sc_bounds_cap) return cudaErrorInvalidValue;
+  ScreenArgs a = screen_args(v, dev_norms, dev_lo_norm, dev_query, 1, ws);
+  a.pess = ws.sc_bounds + v.ld;
+  cudaError_t e = cudaMemsetAsync(ws.sc_ctl, 0, 2 * sizeof(unsigned), s);
+  if (e != cudaSuccess) return e;
+  if ((e = launch_screen_mode(mode, a, ws.num_sms, s)) != cudaSuccess) return e;
+  ++*launches;
+  unsigned flag[2];
+  if ((e = cudaMemcpyAsync(flag, ws.sc_ctl, sizeof(flag), cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+  if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return e;
+  if (flag[1]) return cudaErrorNotSupported;
+  float* lower = mode == PDX_L2 ? a.opt : a.pess;
+  float* upper = mode == PDX_L2 ? a.pess : a.opt;
+  if ((e = cudaMemcpyAsync(host_lower, lower, v.n * sizeof(float), cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+  if ((e = cudaMemcpyAsync(host_upper, upper, v.n * sizeof(float), cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+  return cudaStreamSynchronize(s);
 }
 
 }  // namespace innr

@@ -12,6 +12,7 @@
 // q * 0.0 is -0.0 or NaN for negative / non-finite q, exactly as on the CPU).
 #include "common.cuh"
 #include "kernels.cuh"
+#include "pdx.cuh"
 
 namespace innr {
 
@@ -171,7 +172,7 @@ __global__ void ternary_pack_kernel(const uint64_t* __restrict__ words_rm, unsig
 }
 
 // encode_ternary of every vector of a device-resident PDX f32 corpus: thread (chunk c, vector i) reads 64 dimension rows
-__global__ void ternary_from_pdx_kernel(const float* __restrict__ pdx, size_t ld_f, unsigned n, unsigned d, float threshold,
+__global__ void ternary_from_pdx_kernel(const PdxView pdx, unsigned n, unsigned d, float threshold,
                                         uint4* __restrict__ codes, size_t ld, unsigned chunks) {
   const size_t total = (size_t)chunks * ld;
   for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
@@ -183,7 +184,7 @@ __global__ void ternary_from_pdx_kernel(const float* __restrict__ pdx, size_t ld
       for (int b = 0; b < 64; ++b) {
         const unsigned dd = 64 * c + b;
         if (dd < d) {
-          const float v = pdx[(size_t)dd * ld_f + i];
+          const float v = pdx_load1(pdx, (size_t)dd * pdx.ld + i);
           const unsigned bits = v > threshold ? 1u : (v < -threshold ? 2u : 0u);
           w[b >> 4] |= bits << (2 * (b & 15));
         }
@@ -221,11 +222,11 @@ cudaError_t launch_ternary_pack(const uint64_t* dev_words_rowmajor, size_t n, si
   return cudaGetLastError();
 }
 
-cudaError_t launch_ternary_from_pdx(const float* dev_pdx, size_t ld_f, size_t n, size_t d, float threshold, uint4* dev_codes,
+cudaError_t launch_ternary_from_pdx(const PdxView& v, float threshold, uint4* dev_codes,
                                     size_t ld, cudaStream_t s, LaunchCounter* launches) {
-  if (n == 0 || d == 0) return cudaSuccess;
-  ternary_from_pdx_kernel<<<148 * 16, 256, 0, s>>>(dev_pdx, ld_f, (unsigned)n, (unsigned)d, threshold, dev_codes, ld,
-                                                   (unsigned)((d + 63) / 64));
+  if (v.n == 0 || v.d == 0) return cudaSuccess;
+  ternary_from_pdx_kernel<<<148 * 16, 256, 0, s>>>(v, (unsigned)v.n, (unsigned)v.d, threshold, dev_codes, ld,
+                                                   (unsigned)((v.d + 63) / 64));
   ++*launches;
   return cudaGetLastError();
 }

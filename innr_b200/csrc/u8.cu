@@ -26,6 +26,7 @@
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "pdx.cuh"
 #include "tc_common.cuh"
 
 namespace innr {
@@ -498,7 +499,7 @@ __global__ void generate_u8_kernel(uint64_t salt, uint64_t first_row, unsigned n
 
 // quantize_u8 (src/scalar.rs:212-225) of a device-resident PDX f32 corpus straight into the chunk-major u8 layout:
 // thread (chunk c, vector i) reads 16 dimension rows (coalesced along i) and writes one uint4
-__global__ void u8_from_pdx_kernel(const float* __restrict__ pdx, size_t ld_f, unsigned n, unsigned d, float alpha,
+__global__ void u8_from_pdx_kernel(const PdxView pdx, unsigned n, unsigned d, float alpha,
                                    float offset, uint4* __restrict__ codes, size_t ld, unsigned chunks) {
   const size_t total = (size_t)chunks * ld;
   const float inv_alpha = __fdiv_rn(255.0f, alpha);
@@ -510,7 +511,7 @@ __global__ void u8_from_pdx_kernel(const float* __restrict__ pdx, size_t ld_f, u
 #pragma unroll
       for (int e = 0; e < 16; ++e) {
         const unsigned dd = 16 * c + e;
-        if (dd < d) w[e >> 2] |= quantize_one(pdx[(size_t)dd * ld_f + i], offset, inv_alpha) << (8 * (e & 3));
+        if (dd < d) w[e >> 2] |= quantize_one(pdx_load1(pdx, (size_t)dd * pdx.ld + i), offset, inv_alpha) << (8 * (e & 3));
       }
     }
     codes[t] = make_uint4(w[0], w[1], w[2], w[3]);
@@ -584,11 +585,11 @@ cudaError_t launch_generate_u8(uint64_t salt, uint64_t first_row, size_t n, size
   return cudaGetLastError();
 }
 
-cudaError_t launch_u8_from_pdx(const float* dev_pdx, size_t ld_f, size_t n, size_t d, float alpha, float offset,
+cudaError_t launch_u8_from_pdx(const PdxView& v, float alpha, float offset,
                                uint4* dev_codes, size_t ld, cudaStream_t s, LaunchCounter* launches) {
-  if (n == 0 || d == 0) return cudaSuccess;
-  u8_from_pdx_kernel<<<148 * 16, 256, 0, s>>>(dev_pdx, ld_f, (unsigned)n, (unsigned)d, alpha, offset, dev_codes, ld,
-                                              (unsigned)((d + 15) / 16));
+  if (v.n == 0 || v.d == 0) return cudaSuccess;
+  u8_from_pdx_kernel<<<148 * 16, 256, 0, s>>>(v, (unsigned)v.n, (unsigned)v.d, alpha, offset, dev_codes, ld,
+                                              (unsigned)((v.d + 15) / 16));
   ++*launches;
   return cudaGetLastError();
 }
