@@ -89,7 +89,8 @@ int innr_cuda_knn_tc_debug_bounds(const innr_cuda_corpus* c, int metric, const f
 /* Test hook for the screened single-query kNN of a split corpus: the interval [lower, upper] the screen gives every row
  * for this query, exactly as production computes it (n floats each). The tests assert lower <= reference score <= upper
  * on adversarial rows. INNR_EUNSUPPORTED when the corpus is not split, has a non-finite row or the query cannot be
- * screened (norm not finite; cosine: below the reference's epsilon). */
+ * screened (norm not finite or above 2^100, largest element outside [2^-100, 2^100]; cosine: norm below the
+ * reference's epsilon). */
 int innr_cuda_knn_screen_debug_bounds(const innr_cuda_corpus* c, int metric, const float* query, size_t query_len,
                                       float* out_lower, float* out_upper);
 /* number of kernels the library has launched so far (bench.py's gpu_launches counter) */
@@ -97,9 +98,11 @@ int innr_cuda_launch_count(uint64_t* out_count);
 
 /* ---- f32 VerticalBatch (PDX) corpus: src/batch.rs:88-220 ------------------------------------- */
 /* Owned corpora of at least f32_split_min_rows rows (innr_cuda_set_option; default 1,000,000) are stored split: the
- * same bytes as two 16-bit planes (high halves, then low halves, same pitch), which lets a single-query kNN read only
- * the high halves before it rescores a few dozen rows exactly. Every entry gives the same bits on either layout;
- * corpus_info's ld and device_bytes keep their meaning. Wrapped device memory stays as the caller laid it out. */
+ * same bytes as two 16-bit planes (high halves, then low halves, same pitch), plus an 8-bit sketch of every element
+ * (one byte per element plus 8 bytes per row: +25 % device memory, 7.68 GB for 10M x 768), which lets a single-query
+ * kNN read only the sketch before it rescores a few dozen rows exactly. Every entry gives the same bits on either
+ * layout; corpus_info's ld and device_bytes (the f32 matrix alone) keep their meaning. Wrapped device memory stays as
+ * the caller laid it out. */
 /* host_pdx: the buffer VerticalBatch::data() returns (src/batch.rs:212): data[d*n + i]. */
 int innr_cuda_upload_f32_pdx(const float* host_pdx, size_t n, size_t d, uint64_t index_base,
                              innr_cuda_corpus** out);

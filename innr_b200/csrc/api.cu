@@ -40,9 +40,10 @@ struct innr_cuda_corpus {
   bool tmap_valid = false;
   // f32 PDX, split layout (pdx.cuh): the low-half plane (the high halves start at `dev`); null for plain corpora
   uint16_t* lo_plane = nullptr;
-  // f32 PDX, split corpora: the screened kNN's per-row sidecar (built with the corpus): dev_norms (the reference's norm
-  // bits), dev_lo_norm (r_i >= |lo_i|); `screen` = both finite for every row
-  float* dev_lo_norm = nullptr;
+  // f32 PDX, split corpora: the screened kNN's sidecar (built with the corpus): dev_norms (the reference's norm bits) and
+  // the 8-bit sketch (PdxSketch: d * ld code bytes, then ld scales and ld residual bounds; sketch_of); `screen` = norms,
+  // scales and bounds finite for every row
+  uint8_t* dev_sketch = nullptr;
   bool screen = false;
   // f32 PDX: lazily built operands of the tensor-core filter path (knn_tc.cu): exact norms, f16 unit vectors + TMA map
   int tc_state = 0;  // 0 not built, 1 ready, -1 unusable (non-finite norms / no memory): exact scan only
@@ -357,7 +358,7 @@ void destroy_corpus(innr_cuda_corpus* c) {
   if (c->owns && c->dev) cudaFree(c->dev);
   if (c->dev_offsets) cudaFree(c->dev_offsets);
   if (c->dev_norms) cudaFree(c->dev_norms);
-  if (c->dev_lo_norm) cudaFree(c->dev_lo_norm);
+  if (c->dev_sketch) cudaFree(c->dev_sketch);
   if (c->dev_xh) cudaFree(c->dev_xh);
   if (c->dev_order) cudaFree(c->dev_order);
   delete c;
@@ -542,17 +543,22 @@ static int alloc_pdx(DeviceCtx& ctx, size_t n, size_t d, uint64_t index_base, in
   return INNR_OK;
 }
 
+static PdxSketch sketch_of(const innr_cuda_corpus* c) {
+  float* rows = (float*)(c->dev_sketch + c->d * c->ld);  // d * ld is a multiple of 64: 16 B aligned
+  return PdxSketch{c->dev_sketch, rows, rows + c->ld};
+}
+
 // After a split corpus is written: its sidecar. The norms pass writes whole float4 groups (up to ld entries), the
-// screen reads whole groups of 8: both arrays have ld (+ the tensor-core path's 16 B of scratch) entries.
+// screen reads whole groups of 16: the per-row arrays have ld (+ the tensor-core path's 16 B of scratch) entries.
 static int build_sidecar(innr_cuda_corpus* c, DeviceCtx* ctx) {
   if (!c->lo_plane) return INNR_OK;
   CU(cudaMalloc((void**)&c->dev_norms, c->ld * sizeof(float) + 16));
-  CU(cudaMalloc((void**)&c->dev_lo_norm, c->ld * sizeof(float)));
+  CU(cudaMalloc((void**)&c->dev_sketch, c->d * c->ld + 2 * c->ld * sizeof(float)));
   const PdxView v = pdx_view(c);
   CU(launch_pdx_scores(v, PDX_NORMS, nullptr, nullptr, c->dev_norms, ctx->ws, ctx->stream, &g_launches));
   CU(ctx->h_counts.reserve(64));
   unsigned* flag = (unsigned*)(c->dev_norms + c->ld);
-  CU(launch_split_sidecar(v, c->dev_norms, c->dev_lo_norm, flag, ctx->stream, &g_launches));
+  CU(launch_pdx_sketch(v, c->dev_norms, sketch_of(c), flag, ctx->stream, &g_launches));
   CU(cudaMemcpyAsync(ctx->h_counts.p, flag, sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   c->screen = *(unsigned*)ctx->h_counts.p == 0;
@@ -869,7 +875,7 @@ static int knn_screened(innr_cuda_corpus* c, Workspace& w, int mode, const float
                         cudaStream_t s) {
   int rc = ensure_screen_scratch(w, c->ld);
   if (rc) return rc;
-  CU(launch_pdx_knn_screened(pdx_view(c), mode, c->dev_norms, c->dev_lo_norm, dev_query, k, dev_keys, w, s, &g_launches));
+  CU(launch_pdx_knn_screened(pdx_view(c), mode, c->dev_norms, sketch_of(c), dev_query, k, dev_keys, w, s, &g_launches));
   return INNR_OK;
 }
 // the plain fused scan (k <= 128, no tensor-core filter) needs a Workspace and nothing else: either lane will do
@@ -971,7 +977,7 @@ extern "C" int innr_cuda_knn_screen_debug_bounds(const innr_cuda_corpus* c, int 
   if (rc) return rc;
   CU(ctx->d_query.reserve((c->d + 4) * sizeof(float)));
   CU(cudaMemcpyAsync(ctx->d_query.p, query, c->d * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-  cudaError_t e = launch_pdx_screen_debug_bounds(pdx_view(c), mode, c->dev_norms, c->dev_lo_norm, (const float*)ctx->d_query.p,
+  cudaError_t e = launch_pdx_screen_debug_bounds(pdx_view(c), mode, c->dev_norms, sketch_of(c), (const float*)ctx->d_query.p,
                                                  out_lower, out_upper, ctx->ws, ctx->stream, &g_launches);
   if (e == cudaErrorNotSupported) return fail(INNR_EUNSUPPORTED, "the query cannot be screened");
   CU(e);

@@ -103,6 +103,11 @@ __device__ __forceinline__ uint64_t add2_unfusable(uint64_t a, uint64_t b, uint6
   asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(one2), "l"(b));
   return r;
 }
+__device__ __forceinline__ uint64_t fma2_rn(uint64_t a, uint64_t b, uint64_t c) {
+  uint64_t r;
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
+  return r;
+}
 __device__ __forceinline__ uint64_t add2_rn(uint64_t a, uint64_t b) {
   uint64_t r;
   asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));

@@ -1,12 +1,14 @@
-"""dev: A/B of the single-query f32 kNN on the plain layout (full read) against the split layout (screen on the hi plane +
-exact rescoring), at C2a (10M x 768, G-hash, cosine top-10) and at one 8-GPU shard (1.25M rows). Both corpora are
-generated on the device; the calls alternate back to back for several rounds. Prints per-call CUDA-event times, the
-per-kernel times of the split path (torch.profiler, in a run of its own), candidates per query (from the screen's
-bounds), bit-equality of the keys over 16 queries, and a full-read scores-mode (batch_dot) A/B.
+"""dev: A/B of the single-query f32 kNN on the plain layout (full read) against the split layout (screen on the 8-bit
+sketch + exact rescoring), at C2a (10M x 768, G-hash, cosine top-10) and at one 8-GPU shard (1.25M rows). Both corpora
+are generated on the device; the calls alternate back to back for several rounds. Prints per-call CUDA-event times, the
+per-phase kernel times of the split path (torch.profiler, in a run of its own: screen, compaction, rescoring, selection,
+the fallback full-read launch that returns at once) with the bytes the screen moves and its rate, candidates per query
+(from the screen's bounds), bit-equality of the keys over 16 queries, and a full-read scores-mode (batch_dot) A/B.
 Usage: python innr_b200/csrc/dev/split_scan_ab.py [out_dir]"""
 import ctypes as C
 import json
 import os
+import re
 import subprocess
 import sys
 
@@ -26,6 +28,15 @@ D, K, ROUNDS, CALLS = 768, 10, 6, 40
 q = torch.from_numpy(synth.ghash_f32(synth.SALT_QUERY, 0, 16 * D).reshape(16, D)).cuda()
 stream = torch.cuda.current_stream()
 report = {"gpu": gpu, "sizes": {}}
+# kernel name (profiler keys look like "void innr::(anonymous namespace)::pdx_screen_kernel<1, 1>(...)") -> phase
+PHASES = {"pdx_screen_kernel": "screen", "screen_compact_kernel": "compaction", "screen_rescore_kernel": "rescoring",
+          "topk_scores_kernel": "selection", "pdx_scan_kernel": "fallback_full_read_noop"}
+
+
+def kernel_name(key):
+    key = key.replace("(anonymous namespace)::", "")
+    m = re.match(r"(?:void\s+)?([\w:]+)", key)
+    return m.group(1).split("::")[-1] if m else key
 
 
 def call(db, i, out):
@@ -75,7 +86,8 @@ for n in (10_000_000, 1_250_000):
     phases = {}
     for ev in prof.key_averages():
         if ev.device_type.name == "CUDA" and ev.count:
-            name = ev.key.split("(")[0].split("<")[0].split("::")[-1]
+            name = kernel_name(ev.key)
+            name = PHASES.get(name, name)
             t = getattr(ev, "device_time_total", None) or getattr(ev, "cuda_time_total", 0)
             phases[name] = phases.get(name, 0.0) + t / 20 / 1000.0   # ms per call
     # full-read scores mode (both planes through the load helper against the f32 loads)
@@ -89,14 +101,19 @@ for n in (10_000_000, 1_250_000):
             L.call("innr_cuda_last_kernel_ms", C.byref(ms))
             scores[name].append(ms.value)
     ib.set_option("kernel_timing", 0)
-    hi_bytes = n * D * 2
+    f32_bytes = n * D * 4
+    # the screen reads the sketch (1 B per element) and 16 B per row: scale, residual bound, reference norm, and writes
+    # the 4 B optimistic bound
+    screen_bytes = n * D + n * 16
     med = {k: float(np.median(v)) for k, v in rounds.items()}
     res = {"n": n, "keys_bit_equal_16_queries": equal, "ms_per_call": rounds, "median_ms": med,
            "speedup": med["plain"] / med["split"], "candidates_per_query": cands,
            "split_kernels_ms_per_call": phases,
-           "screen_tb_per_s": hi_bytes / (phases.get("pdx_screen_kernel", float("nan")) / 1e3) / 1e12,
-           "plain_tb_per_s": 2 * hi_bytes / (med["plain"] / 1e3) / 1e12,
-           "bytes_moved_split": hi_bytes + n * 12, "bytes_moved_plain": 2 * hi_bytes,
+           "screen_bytes": screen_bytes,
+           "screen_tb_per_s": screen_bytes / (phases.get("screen", float("nan")) / 1e3) / 1e12,
+           "split_call_tb_per_s": screen_bytes / (med["split"] / 1e3) / 1e12,
+           "plain_tb_per_s": f32_bytes / (med["plain"] / 1e3) / 1e12,
+           "bytes_moved_split": screen_bytes, "bytes_moved_plain": f32_bytes,
            "scores_mode_kernel_ms": scores}
     report["sizes"][str(n)] = res
     print(json.dumps(res, indent=1))

@@ -75,19 +75,28 @@ struct PdxDst {
 cudaError_t launch_pdx_knn(const PdxView& v, int mode, const float* dev_queries, size_t nq, size_t k,
                            uint64_t* dev_keys, Workspace& ws, cudaStream_t s, LaunchCounter* launches,
                            const unsigned* dev_run_flag = nullptr);
-// Screened single-query kNN of a split corpus (scan_f32.cu): the hi plane alone gives every row an interval that holds
-// its exact score, the rows whose interval reaches the k-th best pessimistic bound are rescored exactly from both planes.
-// Same keys as launch_pdx_knn. Needs the corpus' sidecar (dev_norms, dev_lo_norm, all finite), k <= 128,
-// d <= SCREEN_MAX_D and ws.sc_* sized for v.ld rows. More than SCREEN_CAP candidates, or a query whose norm is not finite
-// (cosine: below the reference's epsilon), hand the query to the full-read scan, queued behind on the device.
+// The screened kNN's 8-bit sketch of a split corpus, one allocation built with it (layout.cu, addressing in pdx.cuh):
+// codes[dd * ld + i] = 128 + round(x / scale[i]) clamped to [1, 255], scale[i] = absmax_i / 127 (0 for a zero row),
+// resid[i] >= || x_i - scale[i] (code_i - 128) ||_2 (rounded outward), for the ld columns of the corpus.
+struct PdxSketch {
+  uint8_t* codes;
+  float* scale;
+  float* resid;
+};
+// Screened single-query kNN of a split corpus (scan_f32.cu): the sketch alone gives every row an interval that holds its
+// exact score, the rows whose interval reaches the k-th best pessimistic bound are rescored exactly from both planes.
+// Same keys as launch_pdx_knn. Needs the corpus' sidecar (dev_norms and the sketch, all finite), k <= 128,
+// d <= SCREEN_MAX_D and ws.sc_* sized for v.ld rows. More than SCREEN_CAP candidates, or a query the screen cannot take
+// (norm not finite, largest element outside [2^-100, 2^100], cosine: norm below the reference's epsilon), hand the
+// query to the full-read scan, queued behind on the device.
 constexpr size_t SCREEN_CAP = 4096;
 constexpr size_t SCREEN_MAX_D = 4096;
-cudaError_t launch_pdx_knn_screened(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+cudaError_t launch_pdx_knn_screened(const PdxView& v, int mode, const float* dev_norms, const PdxSketch& sk,
                                     const float* dev_query, size_t k, uint64_t* dev_keys, Workspace& ws, cudaStream_t s,
                                     LaunchCounter* launches);
 // test hook: the screen's interval [lower, upper] for every row (host arrays of n floats); returns cudaErrorNotSupported
 // when the query cannot be screened
-cudaError_t launch_pdx_screen_debug_bounds(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+cudaError_t launch_pdx_screen_debug_bounds(const PdxView& v, int mode, const float* dev_norms, const PdxSketch& sk,
                                            const float* dev_query, float* host_lower, float* host_upper, Workspace& ws,
                                            cudaStream_t s, LaunchCounter* launches);
 // batch_knn_filtered (src/batch.rs:820-882): L2, one query; dev_mask = one bit per local vector (LSB-first u32 words,
@@ -200,10 +209,10 @@ cudaError_t launch_generate_f32_pdx(int generator, uint64_t salt, uint64_t first
 // zero-filled up to dst.ld)
 cudaError_t launch_pdx_rows_to_dst(const float* dev_src, size_t rows, size_t n, const PdxDst& dst, cudaStream_t s,
                                    LaunchCounter* launches);
-// per-row sidecar of a split corpus: dev_norms[i] = the reference's norm (PDX_NORMS bits), dev_lo_norm[i] >= ||lo_i||_2
-// (lo_i = x_i minus its high half, rounded up); *dev_nonfinite != 0 when some row's norm or bound is not finite
-cudaError_t launch_split_sidecar(const PdxView& v, float* dev_norms, float* dev_lo_norm, unsigned* dev_nonfinite,
-                                 cudaStream_t s, LaunchCounter* launches);
+// the sketch of a split corpus (PdxSketch) from the corpus and its reference norms (dev_norms, PDX_NORMS bits);
+// *dev_nonfinite != 0 when some row's norm, scale or residual bound is not finite
+cudaError_t launch_pdx_sketch(const PdxView& v, const float* dev_norms, const PdxSketch& sk, unsigned* dev_nonfinite,
+                              cudaStream_t s, LaunchCounter* launches);
 
 // binary codes (hamming.cu): chunk-major layout codes[c * ld + i] (uint4 = 128 bits), chunks = ceil(words/2)
 struct BinView {

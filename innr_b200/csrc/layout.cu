@@ -54,23 +54,30 @@ __global__ void pdx_rows_to_dst_kernel(const float* __restrict__ src, unsigned r
   }
 }
 
-// r_i >= ||x_i - hi(x_i)||_2: the low halves are exact f32 differences, squared and summed rounding upward, so the
-// result bounds the true norm from above (also when the squares underflow). A norm or bound that is not finite
-// (inf / NaN elements, overflowing sums) marks the corpus as one the screened kNN must not take.
-__global__ void split_sidecar_kernel(const PdxView v, const float* __restrict__ norms, float* __restrict__ lo_norm,
-                                     unsigned* __restrict__ nonfinite) {
-  const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= v.n) return;
+// The sketch, one thread per column of the pitch (padding columns are zero: code 128, scale 0, bound 0). Two passes over
+// the row: absmax, then codes and the residual bound. Any code is valid because r is computed against the code stored:
+// the exact residual x - s c lies between its RD and RU roundings, and the squares are summed rounding upward, so r
+// bounds the true norm from above (also where the squares underflow). A row of zeros or of subnormals below 127 * 2^-150
+// gets s = 0, codes 128 and r = its norm. NaN elements do not enter the absmax but make r NaN.
+__global__ void pdx_sketch_kernel(const PdxView v, const float* __restrict__ norms, const PdxSketch sk,
+                                  unsigned* __restrict__ nonfinite) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= v.ld) return;
+  float m = 0.0f;
+  for (unsigned dd = 0; dd < v.d; ++dd) m = fmaxf(m, fabsf(pdx_load1(v, (size_t)dd * v.ld + i)));
+  const float s = __fdiv_rn(m, 127.0f);
   float acc = 0.0f;
   for (unsigned dd = 0; dd < v.d; ++dd) {
-    const size_t off = (size_t)dd * v.ld + i;
-    const float x = pdx_load1(v, off), h = __uint_as_float((uint32_t)v.hi[off] << 16);
-    const float l = __fsub_rn(x, h);  // exact (Sterbenz; exact in the subnormal range too)
-    acc = __fmaf_ru(l, l, acc);
+    const float x = pdx_load1(v, (size_t)dd * v.ld + i);
+    const float c = s > 0.0f ? fminf(fmaxf(rintf(__fdiv_rn(x, s)), -127.0f), 127.0f) : 0.0f;
+    sk.codes[pdx_sketch_off(v.ld, dd, i)] = (uint8_t)((int)c + 128);
+    const float e = fmaxf(fabsf(__fmaf_rd(-s, c, x)), fabsf(__fmaf_ru(-s, c, x)));
+    acc = __fmaf_ru(e, e, acc);
   }
   const float r = __fsqrt_ru(acc);
-  lo_norm[i] = r;
-  if (!isfinite(r) || !isfinite(norms[i])) atomicOr(nonfinite, 1u);
+  sk.scale[i] = s;
+  sk.resid[i] = r;
+  if (i < v.n && (!isfinite(s) || !isfinite(r) || !isfinite(norms[i]))) atomicOr(nonfinite, 1u);
 }
 
 __global__ void generate_tokens_kernel(uint64_t salt, uint64_t first_row, size_t n_rows, unsigned dim,
@@ -107,11 +114,11 @@ cudaError_t launch_pdx_rows_to_dst(const float* dev_src, size_t rows, size_t n, 
   return cudaGetLastError();
 }
 
-cudaError_t launch_split_sidecar(const PdxView& v, float* dev_norms, float* dev_lo_norm, unsigned* dev_nonfinite,
-                                 cudaStream_t s, LaunchCounter* launches) {
+cudaError_t launch_pdx_sketch(const PdxView& v, const float* dev_norms, const PdxSketch& sk, unsigned* dev_nonfinite,
+                              cudaStream_t s, LaunchCounter* launches) {
   cudaError_t e = cudaMemsetAsync(dev_nonfinite, 0, sizeof(unsigned), s);
-  if (e != cudaSuccess || v.n == 0) return e;
-  split_sidecar_kernel<<<(unsigned)((v.n + 255) / 256), 256, 0, s>>>(v, dev_norms, dev_lo_norm, dev_nonfinite);
+  if (e != cudaSuccess || v.ld == 0) return e;
+  pdx_sketch_kernel<<<(unsigned)((v.ld + 255) / 256), 256, 0, s>>>(v, dev_norms, sk, dev_nonfinite);
   ++*launches;
   return cudaGetLastError();
 }

@@ -3,8 +3,9 @@
 // Plain: data[dd * ld + i] (f32). Split (owned corpora of at least f32_split_min_rows rows): the same bytes as two u16
 // planes of the same pitch, hi[dd * ld + i] = the high 16 bits of the f32 (sign, exponent, 7 mantissa bits) and
 // lo[dd * ld + i] = its low 16 bits. Joining the halves gives back the f32 bit for bit, so every reader computes what it
-// computes on a plain corpus; the screened single-query kNN (scan_f32.cu) reads the hi plane alone. The layout is the
-// same for every thread of a launch, so the branch below is uniform.
+// computes on a plain corpus. The layout is the same for every thread of a launch, so the branch below is uniform.
+// A split corpus also has an 8-bit sketch (PdxSketch, built in layout.cu, read by the screened single-query kNN in
+// scan_f32.cu) in the same dimension-major order and pitch: pdx_sketch_off.
 #pragma once
 #include "common.cuh"
 #include "kernels.cuh"
@@ -48,5 +49,9 @@ __device__ __forceinline__ void pdx_store1(float* dst_f, uint16_t* dst_hi, uint1
     dst_f[off] = x;
   }
 }
+
+// the sketch code of element dd of row i: one byte per element, so one 16 B load holds 16 consecutive rows of one
+// dimension and the next dimension is ld bytes further on
+__device__ __forceinline__ size_t pdx_sketch_off(size_t ld, size_t dd, size_t i) { return dd * ld + i; }
 
 }  // namespace innr

@@ -1143,36 +1143,37 @@ cudaError_t launch_topk_from_distances(const float* dev_dist, size_t n, size_t k
 
 // ---------------------------------------------------------------------------------------------------------
 // Screened single-query kNN of a split corpus (DESIGN.md section 3.1). Three steps, all on the device:
-//  1. screen: stream the hi plane only; for each row an interval [lower, upper] that holds the reference's score.
+//  1. screen: stream the 8-bit sketch only; for each row an interval [lower, upper] that holds the reference's score.
 //     Selection on the pessimistic bound (lower for dot / cosine, upper for L2) gives T, its k-th best value; every row
 //     gets its optimistic bound written to ws.sc_bounds.
 //  2. compaction: the rows whose optimistic bound reaches T. At least k rows have a score at least as good as T, so
 //     every row of the top k (ties on the k-th score included) is among them.
 //  3. rescoring from both planes with the reference's sequential unfused arithmetic, selection on the scan's keys.
-// The bound (scores are d-term f32 sums; u = 2^-24, g = gamma of the launch >= (d + 2) u / (1 - (d + 2) u)):
-//  dot:    |ref - s| <= |q| (r + g (2 |v| + r)) + 2 d 2^-149, s = the screen's sum of q * hi (any order, fused);
-//          |v| <= (nrm (1 + 2u) + nu) (1 + g) with nu = sqrt(d 2^-149) (the reference norm's rounding and underflow).
+// The bound (u = 2^-24, g = gamma of the launch >= (d + 2) u / (1 - (d + 2) u); row v = s (b - 128) + e with the sketch's
+// scale s, codes b in [1, 255] and |e| <= r):
+//  S = the screen's sum of q * b (fused, any order, scaled by a power of two): |S - sum q b| <= 255 g sum|q| + d 2^-p;
+//  Q = the sequential sum of q: |Q - sum q| <= g sum|q|; so q.v lies in s [S - 128 Q -+ E1] -+ |q| r with
+//  E1 = 383 g sum|q| + d 2^-p.
+//  dot:    + the reference's own rounding g |q| |v| + eta, |v| <= (nrm (1 + 2u) + nu) (1 + g), nu = sqrt(d 2^-149);
 //  cosine: ref = RN(dot / P) with P = RN(qn * nrm) computed here with the reference's bits; RN(x / P) is monotone in x.
-//  L2:     a = |q - hi| from the screen's sum A: a^2 in [(A - eta)(1 - g), (A + eta)(1 + 2g)], the exact distance in
-//          [(a - r)^2, (a + r)^2], the reference's within (1 +- g) of it plus eta.
+//  L2:     |q|^2 - 2 q.v + |v|^2 with |v|^2 >= ((nrm (1 - 2u))^2 - eta)(1 - g), the reference's within (1 +- g) plus eta.
 // Every step rounds outward (RD / RU); a bound that is not finite, or a product |q| |v| past 2^100, makes the row a
 // candidate whatever T is.
 // ---------------------------------------------------------------------------------------------------------
 namespace {
 
-constexpr int SC_VPT = 8;                       // vectors per thread: one 16 B load of the hi plane
-constexpr int SC_TILE = SCAN_THREADS * SC_VPT;  // vectors per CTA tile
-constexpr int SC_U = 8;                         // hi-plane rows in flight per thread
+constexpr int SC_VPT = 16;                      // rows per thread: one 16 B load of the sketch
+constexpr int SC_TILE = SCAN_THREADS * SC_VPT;  // rows per CTA tile
+constexpr int SC_U = 8;                         // sketch loads in flight per thread
 constexpr int RS_WARPS = 4;                     // rescoring: warps per CTA, one candidate per warp
 
 struct ScreenArgs {
-  const uint16_t* hi;
+  PdxSketch sk;
   unsigned long long ld;
-  unsigned n, d, ld8, n_tiles, index_base;
+  unsigned n, d, ld16, n_tiles, index_base;
   int k;
   const float* query;
   const float* norms;    // the reference's norm of each row
-  const float* lo_norm;  // r_i >= |lo_i|
   float gamma, eta, nu;
   uint64_t* partials;
   uint64_t* group_partials;
@@ -1183,69 +1184,110 @@ struct ScreenArgs {
   unsigned* ctl;         // ctl[1] = 1: the query cannot be screened
 };
 
-__device__ __forceinline__ void hi8(const uint4& w, float (&h)[8]) {
-  const unsigned x[4] = {w.x, w.y, w.z, w.w};
-#pragma unroll
-  for (int t = 0; t < 4; ++t) {
-    h[2 * t] = __uint_as_float(x[t] << 16);
-    h[2 * t + 1] = __uint_as_float(x[t] & 0xFFFF0000u);
-  }
-}
+// the query's side of the bound, in shared memory (written by one thread while the others stream)
+struct alignas(16) ScreenQuery {
+  float qn_ref, qn_up;  // the reference's |q| bits, an upper bound on |q|
+  float qq_lo, qq_hi;   // bounds on |q|^2
+  float q128;           // 128 Q
+  float e1;             // E1
+  float gq;             // an upper bound on g |q|
+  float unscale;        // 2^(149 - p): the screen's sums are q * b scaled by 2^(p - 149)
+  unsigned wmax[SCAN_THREADS / 32];  // per warp: the bits of max |q_j|
+};
 
 template <int MODE>
-__device__ __forceinline__ void screen_bounds(float s, float nv, float r, float qn_ref, float qn_up, const ScreenArgs& a,
-                                              float& lower, float& upper) {
+__device__ __forceinline__ void screen_bounds(float acc, float s, float r, float nv, const ScreenQuery& c,
+                                              const ScreenArgs& a, float& lower, float& upper) {
   const float g = a.gamma;
-  if (MODE == PDX_L2) {
-    const float a2_up = __fmul_ru(__fadd_ru(s, a.eta), __fadd_ru(1.0f, __fmul_ru(2.0f, g)));
-    const float a2_lo = fmaxf(0.0f, __fmul_rd(__fsub_rd(s, a.eta), __fsub_rd(1.0f, g)));
-    const float t_lo = fmaxf(0.0f, __fsub_rd(__fsqrt_rd(a2_lo), r));
-    const float t_up = __fadd_ru(__fsqrt_ru(a2_up), r);
-    lower = fmaxf(0.0f, __fsub_rd(__fmul_rd(__fmul_rd(t_lo, t_lo), __fsub_rd(1.0f, g)), a.eta));
-    upper = __fadd_ru(__fmul_ru(__fmul_ru(t_up, t_up), __fadd_ru(1.0f, g)), a.eta);
-    if (!(upper <= 3.0e38f)) { lower = -INFINITY; upper = INFINITY; }
-    return;
-  }
-  const float v_up = __fmul_ru(__fadd_ru(__fmul_ru(nv, 1.0f + 2.0f / 16777216.0f), a.nu), __fadd_ru(1.0f, g));
-  const float e = __fadd_ru(__fmul_ru(qn_up, __fadd_ru(r, __fmul_ru(g, __fadd_ru(__fmul_ru(2.0f, v_up), r)))), __fmul_ru(2.0f, a.eta));
-  if (!(__fmul_ru(qn_up, v_up) <= 0x1p100f) || !(fabsf(s) <= 0x1p100f)) {
+  const float v_up = __fmul_ru(__fadd_ru(__fmul_ru(nv, 1.0f + 0x1p-23f), a.nu), __fadd_ru(1.0f, g));
+  if (!(__fmul_ru(c.qn_up, v_up) <= 0x1p100f)) {
     lower = -INFINITY;
     upper = INFINITY;
     return;
   }
-  lower = __fsub_rd(s, e);
-  upper = __fadd_ru(s, e);
+  const float m_lo = __fsub_rd(__fsub_rd(__fmul_rd(acc, c.unscale), c.q128), c.e1);
+  const float m_hi = __fadd_ru(__fsub_ru(__fmul_ru(acc, c.unscale), c.q128), c.e1);
+  const float qr = __fmul_ru(c.qn_up, r);
+  const float x_lo = __fsub_rd(__fmul_rd(s, m_lo), qr);  // the exact q.v lies in [x_lo, x_hi]
+  const float x_hi = __fadd_ru(__fmul_ru(s, m_hi), qr);
+  if (MODE == PDX_L2) {
+    const float n_lo = __fmul_rd(nv, 1.0f - 0x1p-23f);
+    const float vv_lo = fmaxf(0.0f, __fmul_rd(__fsub_rd(__fmul_rd(n_lo, n_lo), a.eta), __fsub_rd(1.0f, g)));
+    const float l_lo = fmaxf(0.0f, __fadd_rd(__fsub_rd(c.qq_lo, 2.0f * x_hi), vv_lo));
+    const float l_hi = __fadd_ru(__fsub_ru(c.qq_hi, 2.0f * x_lo), __fmul_ru(v_up, v_up));
+    lower = fmaxf(0.0f, __fsub_rd(__fmul_rd(l_lo, __fsub_rd(1.0f, g)), a.eta));
+    upper = __fadd_ru(__fmul_ru(l_hi, __fadd_ru(1.0f, g)), a.eta);
+    if (!(upper <= 3.0e38f)) { lower = -INFINITY; upper = INFINITY; }
+    return;
+  }
+  const float e = __fmaf_ru(c.gq, v_up, a.eta);
+  lower = __fsub_rd(x_lo, e);
+  upper = __fadd_ru(x_hi, e);
   if (MODE == PDX_COSINE_FUSED) {
     if (!(nv > NORM_EPS)) {  // the reference's score is exactly 0 (src/batch.rs:716-727)
       lower = upper = 0.0f;
       return;
     }
-    const float p = __fmul_rn(qn_ref, nv);
+    const float p = __fmul_rn(c.qn_ref, nv);
     lower = __fdiv_rd(lower, p);
     upper = __fdiv_ru(upper, p);
   }
 }
 
+// The query is pre-scaled by 2^p so that max |q_j| 2^p lies in [2^126, 2^127), and each code enters as the f32 whose
+// bits are the byte (b 2^-149, exact): PRMT + FFMA2 per byte pair, no conversion. The scaled products stay below 2^-14
+// and their sums below 2^-2 (d <= 4096), so nothing overflows; an operation whose result falls below 2^-126 errs by at
+// most 2^-150 absolutely, d 2^-149 in all, d 2^-p once unscaled. Scaling q up by powers of two is exact; queries with
+// max |q_j| outside [2^-100, 2^100] (NaN included) are not screened.
 template <int MODE, int R>
 __global__ void __launch_bounds__(SCAN_THREADS) pdx_screen_kernel(const ScreenArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const unsigned d_pad = (a.d + 31u) / 32u * 32u;
-  float* sq = reinterpret_cast<float*>(smem_raw);
-  float* s_qn = sq + d_pad;  // [0] the reference's query norm, [1] an upper bound on |q|
-  uint64_t* smem_keys = reinterpret_cast<uint64_t*>(s_qn + 4);
+  float* sq = reinterpret_cast<float*>(smem_raw);  // the query as given
+  float* sqs = sq + d_pad;                          // pre-scaled by 2^p
+  ScreenQuery* sc = reinterpret_cast<ScreenQuery*>(sqs + d_pad);
+  uint64_t* smem_keys = reinterpret_cast<uint64_t*>(sc + 1);
   const int lane = threadIdx.x & 31;
-  for (unsigned dd = threadIdx.x; dd < d_pad; dd += blockDim.x) sq[dd] = dd < a.d ? a.query[dd] : 0.0f;
+  unsigned mb = 0;
+  for (unsigned dd = threadIdx.x; dd < d_pad; dd += blockDim.x) {
+    const float x = dd < a.d ? a.query[dd] : 0.0f;
+    sq[dd] = x;
+    mb = max(mb, __float_as_uint(x) & 0x7FFFFFFFu);
+  }
+  mb = __reduce_max_sync(FULL_MASK, mb);
+  if (lane == 0) sc->wmax[threadIdx.x >> 5] = mb;
   __syncthreads();
-  // both norms are d-long chains: the last thread computes them while the others stream (read after the first tile)
+#pragma unroll
+  for (int w = 0; w < SCAN_THREADS / 32; ++w) mb = max(mb, sc->wmax[w]);
+  // a query that cannot be pre-scaled: every CTA sees the same and leaves before taking a ticket
+  if (!(mb >= 0x0D800000u && mb <= 0x71800000u)) {  // 2^-100, 2^100
+    if (threadIdx.x == 0) a.ctl[1] = 1u;
+    return;
+  }
+  const int p = 253 - (int)(mb >> 23);  // 126 - the exponent of max |q_j|: 26 .. 226
+  const float f1 = __uint_as_float((unsigned)(p / 2 + 127) << 23), f2 = __uint_as_float((unsigned)(p - p / 2 + 127) << 23);
+  for (unsigned dd = threadIdx.x; dd < d_pad; dd += blockDim.x) sqs[dd] = __fmul_rn(__fmul_rn(sq[dd], f1), f2);
+  __syncthreads();
+  // the query's d-long chains: the last thread computes them while the others stream (read after the first tile)
   if (threadIdx.x == SCAN_THREADS - 1) {
-    float ss = 0.0f, su = 0.0f;
+    float ss = 0.0f, su = 0.0f, sl = 0.0f, qs = 0.0f, sa = 0.0f;
     for (unsigned dd = 0; dd < a.d; ++dd) {
       const float x = sq[dd];
       ss = __fadd_rn(ss, __fmul_rn(x, x));
       su = __fmaf_ru(x, x, su);
+      sl = __fmaf_rd(x, x, sl);
+      qs = __fadd_rn(qs, x);
+      sa = __fadd_ru(sa, fabsf(x));
     }
-    s_qn[0] = __fsqrt_rn(ss);
-    s_qn[1] = __fsqrt_ru(su);
+    const float us = __uint_as_float((unsigned)(276 - p) << 23);
+    sc->qn_ref = __fsqrt_rn(ss);
+    sc->qn_up = __fsqrt_ru(su);
+    sc->qq_lo = sl;
+    sc->qq_hi = su;
+    sc->q128 = 128.0f * qs;  // exact: |qs| <= sum|q| <= 2^112
+    sc->e1 = __fadd_ru(__fmul_ru(a.gamma, __fmul_ru(383.0f, sa)), __fmul_ru(__uint_as_float(a.d), us));  // d 2^-149 us
+    sc->gq = __fmul_ru(a.gamma, sc->qn_up);
+    sc->unscale = us;
   }
   bool qn_visible = false;
   WarpList<R> lists[1];
@@ -1254,82 +1296,71 @@ __global__ void __launch_bounds__(SCAN_THREADS) pdx_screen_kernel(const ScreenAr
 
   for (unsigned tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
     const unsigned i0 = tile * SC_TILE + threadIdx.x * SC_VPT;
-    const bool active = i0 < a.ld8;
-    float acc[SC_VPT];
+    const bool active = i0 < a.ld16;
+    uint64_t acc[SC_VPT / 2];  // rows (2j, 2j + 1)
 #pragma unroll
-    for (int j = 0; j < SC_VPT; ++j) acc[j] = 0.0f;
-    auto step = [&](const uint4& w, unsigned dd) {
-      float h[8];
-      hi8(w, h);
-      const float q = sq[dd];
+    for (int j = 0; j < SC_VPT / 2; ++j) acc[j] = 0;
+    auto step = [&](const uint4& w, float q) {
+      const uint64_t q2 = pack2(q, q);
+      const unsigned x[4] = {w.x, w.y, w.z, w.w};
 #pragma unroll
-      for (int j = 0; j < SC_VPT; ++j) {
-        if (MODE == PDX_L2) {
-          const float t = q - h[j];
-          acc[j] = fmaf(t, t, acc[j]);
-        } else {
-          acc[j] = fmaf(q, h[j], acc[j]);
-        }
+      for (int t = 0; t < 4; ++t) {
+        const float b0 = __uint_as_float(__byte_perm(x[t], 0u, 0x4440u)), b1 = __uint_as_float(__byte_perm(x[t], 0u, 0x4441u));
+        const float b2 = __uint_as_float(__byte_perm(x[t], 0u, 0x4442u)), b3 = __uint_as_float(__byte_perm(x[t], 0u, 0x4443u));
+        acc[2 * t] = fma2_rn(q2, pack2(b0, b1), acc[2 * t]);
+        acc[2 * t + 1] = fma2_rn(q2, pack2(b2, b3), acc[2 * t + 1]);
       }
     };
     if (active) {
-      const uint16_t* p = a.hi + i0;
+      const uint8_t* p = a.sk.codes + pdx_sketch_off(a.ld, 0, i0);
+      const size_t next = pdx_sketch_off(a.ld, 1, 0);  // one dimension on
       unsigned dd = 0;
       for (; dd + SC_U <= a.d; dd += SC_U) {
         uint4 w[SC_U];
 #pragma unroll
-        for (int u = 0; u < SC_U; ++u) w[u] = ldg_stream_u4(reinterpret_cast<const uint4*>(p + (size_t)u * a.ld));
-        p += (size_t)SC_U * a.ld;
+        for (int u = 0; u < SC_U; ++u) w[u] = ldg_stream_u4(reinterpret_cast<const uint4*>(p + u * next));
+        p += SC_U * next;
 #pragma unroll
-        for (int u = 0; u < SC_U; ++u) step(w[u], dd + u);
+        for (int u = 0; u < SC_U; ++u) step(w[u], sqs[dd + u]);
       }
-      for (; dd < a.d; ++dd) {
-        step(ldg_stream_u4(reinterpret_cast<const uint4*>(p)), dd);
-        p += a.ld;
-      }
+      for (; dd < a.d; ++dd, p += next) step(ldg_stream_u4(reinterpret_cast<const uint4*>(p)), sqs[dd]);
     }
     if (!qn_visible) {  // first tile of this CTA (CTA-uniform)
       __syncthreads();
       qn_visible = true;
-      const float qr = s_qn[0], qu = s_qn[1];
-      // a query the bound cannot take: every CTA sees the same and leaves before taking a ticket
+      const float qr = sc->qn_ref, qu = sc->qn_up;
       if (!(qu <= 0x1p100f) || (MODE == PDX_COSINE_FUSED && !(qr >= NORM_EPS))) {
         if (threadIdx.x == 0) a.ctl[1] = 1u;
         return;
       }
     }
-    const float qn_ref = s_qn[0], qn_up = s_qn[1];
-    float nv[SC_VPT], r[SC_VPT];
-    if (active) {
 #pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const float4 x = *reinterpret_cast<const float4*>(a.norms + i0 + 4 * h);
-        const float4 y = *reinterpret_cast<const float4*>(a.lo_norm + i0 + 4 * h);
-        nv[4 * h] = x.x; nv[4 * h + 1] = x.y; nv[4 * h + 2] = x.z; nv[4 * h + 3] = x.w;
-        r[4 * h] = y.x; r[4 * h + 1] = y.y; r[4 * h + 2] = y.z; r[4 * h + 3] = y.w;
+    for (int h = 0; h < SC_VPT / 4; ++h) {
+      const unsigned ih = i0 + 4 * h;
+      float lo[4] = {0.0f, 0.0f, 0.0f, 0.0f}, up[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+      if (active) {
+        const float4 s4 = *reinterpret_cast<const float4*>(a.sk.scale + ih);
+        const float4 r4 = *reinterpret_cast<const float4*>(a.sk.resid + ih);
+        const float4 n4 = *reinterpret_cast<const float4*>(a.norms + ih);
+        const float s[4] = {s4.x, s4.y, s4.z, s4.w}, r[4] = {r4.x, r4.y, r4.z, r4.w}, nv[4] = {n4.x, n4.y, n4.z, n4.w};
+        float x[4];
+        unpack2(acc[2 * h], x[0], x[1]);
+        unpack2(acc[2 * h + 1], x[2], x[3]);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) screen_bounds<MODE>(x[j], s[j], r[j], nv[j], *sc, a, lo[j], up[j]);
+        const float* ob = (MODE == PDX_L2) ? lo : up;
+        *reinterpret_cast<float4*>(a.opt + ih) = make_float4(ob[0], ob[1], ob[2], ob[3]);
+        if (a.pess) {
+          const float* pb = (MODE == PDX_L2) ? up : lo;
+          for (int j = 0; j < 4; ++j) a.pess[ih + j] = pb[j];
+        }
       }
-    }
-    float lo[SC_VPT], up[SC_VPT];
 #pragma unroll
-    for (int j = 0; j < SC_VPT; ++j) {
-      lo[j] = up[j] = 0.0f;
-      if (active) screen_bounds<MODE>(acc[j], nv[j], r[j], qn_ref, qn_up, a, lo[j], up[j]);
-    }
-    if (active) {
-      float* o = a.opt + i0;
-      const float* ob = (MODE == PDX_L2) ? lo : up;
-      *reinterpret_cast<float4*>(o) = make_float4(ob[0], ob[1], ob[2], ob[3]);
-      *reinterpret_cast<float4*>(o + 4) = make_float4(ob[4], ob[5], ob[6], ob[7]);
-      if (a.pess) {
-        const float* pb = (MODE == PDX_L2) ? up : lo;
-        for (int j = 0; j < SC_VPT; ++j) a.pess[i0 + j] = pb[j];
+      for (int j = 0; j < 4; ++j) {
+        const unsigned i = ih + j;
+        const uint64_t key = (MODE == PDX_L2) ? make_key_asc(up[j], a.index_base + i) : make_key_desc(lo[j], a.index_base + i);
+        lists[0].offer(key, active && i < a.n, thr, a.k, lane);
       }
-    }
-#pragma unroll
-    for (int j = 0; j < SC_VPT; ++j) {
-      const unsigned i = i0 + j;
-      const uint64_t key = (MODE == PDX_L2) ? make_key_asc(up[j], a.index_base + i) : make_key_desc(lo[j], a.index_base + i);
-      lists[0].offer(key, active && i < a.n, thr, a.k, lane);
     }
   }
   block_finish<R, 1>(lists, 1, a.k, smem_keys, a.partials, a.group_partials, a.tkeys, a.tickets);
@@ -1402,20 +1433,19 @@ __global__ void __launch_bounds__(RS_WARPS * 32) screen_rescore_kernel(const Pdx
   keys[j] = MODE == PDX_L2 ? make_key_asc(sc, gid) : make_key_desc(sc, gid);
 }
 
-ScreenArgs screen_args(const PdxView& v, const float* dev_norms, const float* dev_lo_norm, const float* dev_query, size_t k,
+ScreenArgs screen_args(const PdxView& v, const float* dev_norms, const PdxSketch& sk, const float* dev_query, size_t k,
                        Workspace& ws) {
   ScreenArgs a{};
-  a.hi = v.hi;
+  a.sk = sk;
   a.ld = v.ld;
   a.n = (unsigned)v.n;
   a.d = (unsigned)v.d;
-  a.ld8 = (unsigned)std::min<size_t>(v.ld, (v.n + 7) / 8 * 8);
-  a.n_tiles = (unsigned)(((size_t)a.ld8 + SC_TILE - 1) / SC_TILE);
+  a.ld16 = (unsigned)std::min<size_t>(v.ld, (v.n + 15) / 16 * 16);
+  a.n_tiles = (unsigned)(((size_t)a.ld16 + SC_TILE - 1) / SC_TILE);
   a.index_base = v.index_base;
   a.k = (int)k;
   a.query = dev_query;
   a.norms = dev_norms;
-  a.lo_norm = dev_lo_norm;
   // gamma_(d+2) = (d + 2) u / (1 - (d + 2) u), u = 2^-24, rounded up to f32 (double has room to spare)
   const double du = (double)(v.d + 2) * 0x1p-24;
   a.gamma = (float)(du / (1.0 - du)) * (1.0f + 0x1p-20f);
@@ -1433,7 +1463,8 @@ ScreenArgs screen_args(const PdxView& v, const float* dev_norms, const float* de
 template <int MODE, int R>
 cudaError_t launch_screen(const ScreenArgs& a, int num_sms, cudaStream_t s) {
   auto kern = pdx_screen_kernel<MODE, R>;
-  const size_t smem = ((a.d + 31u) / 32u * 32u + 4) * sizeof(float) + (size_t)(SCAN_THREADS / 32) * a.k * sizeof(uint64_t);
+  const size_t smem = (size_t)2 * ((a.d + 31u) / 32u * 32u) * sizeof(float) + sizeof(ScreenQuery) +
+                      (size_t)(SCAN_THREADS / 32) * a.k * sizeof(uint64_t);
   static size_t smem_set_dev[16] = {};
   size_t& smem_set = smem_set_dev[current_device_slot()];
   if (smem > 48 * 1024 && smem > smem_set) {
@@ -1462,12 +1493,12 @@ cudaError_t launch_screen_mode(int mode, const ScreenArgs& a, int num_sms, cudaS
 
 }  // namespace
 
-cudaError_t launch_pdx_knn_screened(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+cudaError_t launch_pdx_knn_screened(const PdxView& v, int mode, const float* dev_norms, const PdxSketch& sk,
                                     const float* dev_query, size_t k, uint64_t* dev_keys, Workspace& ws, cudaStream_t s,
                                     LaunchCounter* launches) {
-  if (!v.hi || k == 0 || k > 128 || v.d == 0 || v.d > SCREEN_MAX_D || v.n < k || ws.sc_bounds_cap < v.ld)
+  if (!v.hi || !sk.codes || k == 0 || k > 128 || v.d == 0 || v.d > SCREEN_MAX_D || v.n < k || ws.sc_bounds_cap < v.ld)
     return cudaErrorInvalidValue;
-  const ScreenArgs a = screen_args(v, dev_norms, dev_lo_norm, dev_query, k, ws);
+  const ScreenArgs a = screen_args(v, dev_norms, sk, dev_query, k, ws);
   cudaError_t e = cudaMemsetAsync(ws.sc_ctl, 0, 2 * sizeof(unsigned), s);
   if (e != cudaSuccess) return e;
   if ((e = launch_screen_mode(mode, a, ws.num_sms, s)) != cudaSuccess) return e;
@@ -1492,11 +1523,12 @@ cudaError_t launch_pdx_knn_screened(const PdxView& v, int mode, const float* dev
   return launch_pdx_knn(v, mode, dev_query, 1, k, dev_keys, ws, s, launches, ws.sc_ctl + 1);
 }
 
-cudaError_t launch_pdx_screen_debug_bounds(const PdxView& v, int mode, const float* dev_norms, const float* dev_lo_norm,
+cudaError_t launch_pdx_screen_debug_bounds(const PdxView& v, int mode, const float* dev_norms, const PdxSketch& sk,
                                            const float* dev_query, float* host_lower, float* host_upper, Workspace& ws,
                                            cudaStream_t s, LaunchCounter* launches) {
-  if (!v.hi || v.n == 0 || v.d == 0 || v.d > SCREEN_MAX_D || 2 * v.ld > ws.sc_bounds_cap) return cudaErrorInvalidValue;
-  ScreenArgs a = screen_args(v, dev_norms, dev_lo_norm, dev_query, 1, ws);
+  if (!v.hi || !sk.codes || v.n == 0 || v.d == 0 || v.d > SCREEN_MAX_D || 2 * v.ld > ws.sc_bounds_cap)
+    return cudaErrorInvalidValue;
+  ScreenArgs a = screen_args(v, dev_norms, sk, dev_query, 1, ws);
   a.pess = ws.sc_bounds + v.ld;
   cudaError_t e = cudaMemsetAsync(ws.sc_ctl, 0, 2 * sizeof(unsigned), s);
   if (e != cudaSuccess) return e;
