@@ -302,6 +302,20 @@ int innr_cuda_maxsim(const innr_cuda_corpus* c, const float* q_tokens, size_t n_
                      int cosine_flag, float* out_scores_host);
 int innr_cuda_maxsim_dev(const innr_cuda_corpus* c, const float* dev_q_tokens, size_t n_q, int cosine_flag,
                          float* dev_scores, void* stream);
+/* Top-k documents per query: n_queries queries of n_q tokens each (q_tokens n_queries x n_q x q_dim), the k best
+ * documents by the MaxSim score of innr_cuda_maxsim, descending under f32::total_cmp, exact ties -> lower global index
+ * (index_base + doc). The scores are innr_cuda_maxsim's bit for bit, so a result equals a stable descending total_cmp
+ * sort of its output, truncated to k; a NaN total is the canonical positive NaN and sorts first. min(k, n_docs)
+ * results per query at row stride k; k == 0, n_queries == 0 or an empty corpus -> *out_count = 0. Any k. Batches are
+ * scored in chunks (the score scratch is bounded whatever n_queries is); two queries of <= 32 tokens share a pass. */
+int innr_cuda_maxsim_topk(const innr_cuda_corpus* c, const float* q_tokens, size_t n_queries, size_t n_q, size_t q_dim,
+                          int cosine_flag, size_t k, uint64_t* out_idx, float* out_score, size_t* out_count);
+/* Device form: n_queries x k descending composite keys into dev_keys on `stream`, sentinel-padded like every *_keys_dev
+ * (also when n_docs < k); they feed innr_cuda_exchange_merge_dev / innr_cuda_merge_keys_dev with a descending metric
+ * (INNR_METRIC_DOT). The score vectors live in the device's scratch, so this call is ordered behind (and ahead of)
+ * every other call that uses it. */
+int innr_cuda_maxsim_topk_keys_dev(const innr_cuda_corpus* c, const float* dev_q_tokens, size_t n_queries, size_t n_q,
+                                   int cosine_flag, size_t k, uint64_t* dev_keys, void* stream);
 
 /* ---- cross-GPU exchange of per-shard top-k lists without a collective library (SURVEY 8e; csrc/exchange.cu) ---------
  * Every rank owns a small mailbox in its device memory and maps every peer's (CUDA IPC between processes,
@@ -344,6 +358,10 @@ int innr_cuda_hamming_topk_sharded(const innr_cuda_corpus* const* shards, size_t
 int innr_cuda_batch_knn_u8_sharded(const innr_cuda_corpus* const* shards, size_t n_shards, const float* queries,
                                    size_t n_queries, size_t query_len, size_t k, uint64_t* out_idx, float* out_score,
                                    size_t* out_count);
+/* token shards (each a document range with its index_base): equals innr_cuda_maxsim_topk over the whole document set */
+int innr_cuda_maxsim_topk_sharded(const innr_cuda_corpus* const* shards, size_t n_shards, const float* q_tokens,
+                                  size_t n_queries, size_t n_q, size_t q_dim, int cosine_flag, size_t k, uint64_t* out_idx,
+                                  float* out_score, size_t* out_count);
 /* ---- asynchronous host-buffer top-k ------------------------------------------------------------------------
  * The entries above synchronise before they return. These queue the same call -- same arguments, same checks, same
  * results -- and hand back a ticket; innr_cuda_ticket_wait blocks until THAT call is complete, writes min(k, N)
@@ -360,6 +378,9 @@ int innr_cuda_hamming_topk_async(const innr_cuda_corpus* c, const uint64_t* quer
                                  size_t query_dim_bits, size_t k, innr_cuda_ticket** out_ticket);
 int innr_cuda_batch_knn_u8_async(const innr_cuda_corpus* c, const float* queries, size_t n_queries, size_t query_len,
                                  size_t k, innr_cuda_ticket** out_ticket);
+/* each of the two slots owns its MaxSim score vectors: two calls in flight never share scratch */
+int innr_cuda_maxsim_topk_async(const innr_cuda_corpus* c, const float* q_tokens, size_t n_queries, size_t n_q,
+                                size_t q_dim, int cosine_flag, size_t k, innr_cuda_ticket** out_ticket);
 int innr_cuda_ticket_wait(innr_cuda_ticket* t, uint64_t* out_idx, float* out_score, uint32_t* out_dist,
                           size_t* out_count);
 /* The same for row shards on pairwise distinct devices (the peer-mapped exchange route of the *_sharded entries):
@@ -377,6 +398,9 @@ int innr_cuda_hamming_topk_sharded_async(const innr_cuda_corpus* const* shards, 
                                          size_t k, innr_cuda_ticket** out_ticket);
 int innr_cuda_batch_knn_u8_sharded_async(const innr_cuda_corpus* const* shards, size_t n_shards, const float* queries,
                                          size_t n_queries, size_t query_len, size_t k, innr_cuda_ticket** out_ticket);
+int innr_cuda_maxsim_topk_sharded_async(const innr_cuda_corpus* const* shards, size_t n_shards, const float* q_tokens,
+                                        size_t n_queries, size_t n_q, size_t q_dim, int cosine_flag, size_t k,
+                                        innr_cuda_ticket** out_ticket);
 
 /* ---- timing hook: device time (ms) of the last host-facing call's kernels, measured with CUDA events on the
  *      launching stream. Off by default (the two timed event records cost a short call ~15 us): enable with

@@ -673,6 +673,31 @@ impl TokenCorpus {
         })?;
         Ok(out)
     }
+
+    /// The `k` best documents for one query token set: `(index, score)` descending under `f32::total_cmp`, exact ties ->
+    /// lower index (`index_base + doc`). The scores are `maxsim`'s bit for bit, so this is a stable descending
+    /// `total_cmp` sort of `maxsim`'s output truncated to `k`, without copying `num_docs` floats to the host.
+    pub fn maxsim_topk(&self, q_tokens: &[f32], n_q: usize, cosine: bool, k: usize) -> Result<Vec<(usize, f32)>> {
+        assert_eq!(q_tokens.len(), n_q * self.dim, "dimension mismatch (query)"); // src/maxsim.rs:103-106
+        let (mut idx, mut sc) = knn_buffers(1, k);
+        let mut count = 0usize;
+        check(unsafe {
+            innr_cuda_maxsim_topk(self.h.0, q_tokens.as_ptr(), 1, n_q, self.dim, cosine as c_int, k, idx.as_mut_ptr(), sc.as_mut_ptr(), &mut count)
+        })?;
+        Ok(idx.into_iter().zip(sc).take(count).map(|(i, s)| (i as usize, s)).collect())
+    }
+
+    /// `maxsim_topk` of several queries of `n_q` tokens each (`n_queries x n_q x dim`): per query `(indices, scores)`,
+    /// the same as one `maxsim_topk` call per query.
+    pub fn maxsim_topk_batch(&self, q_tokens: &[f32], n_queries: usize, n_q: usize, cosine: bool, k: usize) -> Result<Vec<(Vec<usize>, Vec<f32>)>> {
+        assert_eq!(q_tokens.len(), n_queries * n_q * self.dim, "dimension mismatch (query)");
+        let (mut idx, mut sc) = knn_buffers(n_queries, k);
+        let mut count = 0usize;
+        check(unsafe {
+            innr_cuda_maxsim_topk(self.h.0, q_tokens.as_ptr(), n_queries, n_q, self.dim, cosine as c_int, k, idx.as_mut_ptr(), sc.as_mut_ptr(), &mut count)
+        })?;
+        Ok(split_results(idx, sc, n_queries, k, count))
+    }
 }
 
 // ------------------------------------------------------------------------------------------------ ternary codes

@@ -17,7 +17,8 @@ from .batch import (BatchKnnResult, DeviceBatch, VerticalBatch, batch_cosine, ba
 from .binary import (BinaryCorpus, PackedBinary, binary_dot, binary_dot_all, binary_hamming, binary_jaccard,  # noqa: F401
                      binary_jaccard_all, binary_topk, encode_binary, hamming_all,
                      hamming_topk, hamming_topk_many)
-from .maxsim import TokenCorpus, maxsim, maxsim_corpus, maxsim_corpus_batch, maxsim_cosine  # noqa: F401
+from .maxsim import (TokenCorpus, maxsim, maxsim_corpus, maxsim_corpus_batch, maxsim_cosine, maxsim_topk,  # noqa: F401
+                     maxsim_topk_batch)
 from .scalar import (QuantizationParams, QuantizedU8, QueryContext, U8Corpus, asymmetric_dot_u8,  # noqa: F401
                      asymmetric_dot_u8_all, asymmetric_dot_u8_precomputed, batch_knn_u8, batch_knn_u8_many,
                      mixed_dot_u8_all, mixed_dot_u8_f32, quantize_u8, query_context)

@@ -111,6 +111,11 @@ SIGNATURES = {
     "innr_cuda_maxsim_batch": [vp, f32p, sz, sz, sz, ci, f32p],
     "innr_cuda_maxsim_batch_dev": [vp, vp, sz, sz, ci, vp, vp],
     "innr_cuda_maxsim_dev": [vp, vp, sz, ci, vp, vp],
+    "innr_cuda_maxsim_topk": [vp, f32p, sz, sz, sz, ci, sz, u64p, f32p, szp],
+    "innr_cuda_maxsim_topk_keys_dev": [vp, vp, sz, sz, ci, sz, vp, vp],
+    "innr_cuda_maxsim_topk_async": [vp, f32p, sz, sz, sz, ci, sz, handle_p],
+    "innr_cuda_maxsim_topk_sharded": [vp, sz, f32p, sz, sz, sz, ci, sz, u64p, f32p, szp],
+    "innr_cuda_maxsim_topk_sharded_async": [vp, sz, f32p, sz, sz, sz, ci, sz, handle_p],
 }
 STRING_GETTERS = ("innr_cuda_last_error", "innr_cuda_backend_name")
 

@@ -70,6 +70,9 @@ struct innr_cuda_ticket {
   cudaEvent_t done = nullptr;
   void *d_query = nullptr, *d_keys = nullptr, *h_in = nullptr, *h_out = nullptr;  // h_*: pinned
   size_t d_query_cap = 0, d_keys_cap = 0, h_in_cap = 0, h_out_cap = 0;
+  // MaxSim top-k: the slot's own score vectors (a chunk of queries x n_docs), so two calls in flight never share them
+  void* d_scores = nullptr;
+  size_t d_scores_cap = 0;
   // a sharded call (innr_cuda_*_sharded_async): this is the root's ticket, `siblings` are the other devices' (released
   // with it), the merged keys come out of the exchange launch into d_merged, rows are k wide, and the exchange's status
   // word travels behind the keys
@@ -461,6 +464,7 @@ int innr_cuda_shutdown(void) {
       if (t.h_in) cudaFreeHost(t.h_in);
       if (t.h_out) cudaFreeHost(t.h_out);
       if (t.d_merged) cudaFree(t.d_merged);
+      if (t.d_scores) cudaFree(t.d_scores);
       if (t.done) cudaEventDestroy(t.done);
       if (t.stream) cudaStreamDestroy(t.stream);
     }
@@ -2345,6 +2349,86 @@ int innr_cuda_maxsim_dev(const innr_cuda_corpus* c, const float* dev_q_tokens, s
   return maxsim_common(c, ctx, dev_q_tokens, n_q, cosine_flag, dev_scores, (cudaStream_t)stream);
 }
 
+// MaxSim top-k: the score vectors of a chunk of queries (maxsim_batch_common: pairs of <= 32-token queries still share
+// a corpus pass), then one selection per query over its vector (launch_topk_from_scores kind 1: descending under
+// total_cmp, ties -> lower index, rounds of 128 for any k). The keys are those of a stable descending sort of
+// innr_cuda_maxsim's output. The scratch holds one chunk, so it is bounded by MAXSIM_TOPK_SCRATCH (or two score vectors)
+// whatever the batch size.
+constexpr size_t MAXSIM_TOPK_SCRATCH = 64ull << 20;
+static size_t maxsim_topk_chunk(const innr_cuda_corpus* c, size_t nq) {
+  size_t rows = MAXSIM_TOPK_SCRATCH / (c->n * sizeof(float));
+  rows = rows < 2 ? 2 : rows & ~(size_t)1;  // even: a chunk boundary never splits a pair
+  return rows < nq ? rows : nq;
+}
+// Writes min(k, n) keys per query at row stride k, the rest of each row sentinel-padded; dev_scores holds
+// maxsim_topk_chunk(c, nq) * n floats. Needs c->n > 0 and lane 0 of ctx (launch_topk_from_scores uses ctx->ws).
+static int maxsim_topk_keys(const innr_cuda_corpus* c, DeviceCtx* ctx, const float* dev_q, size_t nq, size_t n_q, int cosine,
+                            size_t k, uint64_t* dev_keys, float* dev_scores, cudaStream_t s) {
+  const size_t kk = k < c->n ? k : c->n;
+  if (kk < k) CU(cudaMemsetAsync(dev_keys, 0xFF, nq * k * sizeof(uint64_t), s));
+  const size_t chunk = maxsim_topk_chunk(c, nq);
+  for (size_t q0 = 0; q0 < nq; q0 += chunk) {
+    const size_t m = nq - q0 < chunk ? nq - q0 : chunk;
+    int rc = maxsim_batch_common(c, ctx, dev_q + q0 * n_q * c->d, m, n_q, cosine, dev_scores, s);
+    if (rc) return rc;
+    for (size_t j = 0; j < m; ++j) {
+      rc = big_k_from_scores(ctx, dev_scores + j * c->n, 1, c->n, c->index_base, kk, dev_keys + (q0 + j) * k, s);
+      if (rc) return rc;
+    }
+  }
+  return INNR_OK;
+}
+
+int innr_cuda_maxsim_topk(const innr_cuda_corpus* c, const float* q_tokens, size_t n_queries, size_t n_q, size_t q_dim,
+                          int cosine_flag, size_t k, uint64_t* out_idx, float* out_score, size_t* out_count) {
+  if (!c || c->kind != 3) return fail(INNR_EINVAL, "need a token corpus");
+  if (n_q && c->total_tokens && q_dim != c->d) return fail(INNR_EINVAL, "dimension mismatch (doc)");  // src/maxsim.rs:107-110
+  if (out_count) *out_count = 0;
+  if (c->n == 0 || k == 0 || n_queries == 0) return INNR_OK;
+  if (!out_idx || !out_score || (n_q * q_dim && !q_tokens)) return fail(INNR_EINVAL, "null argument");
+  const size_t kk = k < c->n ? k : c->n;
+  EntryGuard lk(c->device);
+  DeviceCtx* ctx;
+  int rc = ctx_for(c, &ctx);
+  if (rc) return rc;
+  const size_t qfloats = n_queries * n_q * c->d;
+  CU(ctx->d_query.reserve((qfloats + 4) * sizeof(float)));
+  CU(ctx->d_keys.reserve(n_queries * kk * sizeof(uint64_t)));
+  CU(ctx->d_scores.reserve(maxsim_topk_chunk(c, n_queries) * c->n * sizeof(float)));
+  if (qfloats && c->total_tokens)
+    CU(cudaMemcpyAsync(ctx->d_query.p, q_tokens, qfloats * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  Timed tm(*ctx);
+  rc = maxsim_topk_keys(c, ctx, (const float*)ctx->d_query.p, n_queries, n_q, cosine_flag, kk, (uint64_t*)ctx->d_keys.p,
+                        (float*)ctx->d_scores.p, ctx->stream);
+  if (rc) return rc;
+  tm.stop();
+  rc = fetch_keys(*ctx, n_queries, kk, tm, [&](const uint64_t* keys) {
+    for (size_t q = 0; q < n_queries; ++q) decode_keys_f32(keys + q * kk, kk, true, out_idx + q * k, out_score + q * k);
+  });
+  if (rc) return rc;
+  if (out_count) *out_count = kk;
+  return INNR_OK;
+}
+
+int innr_cuda_maxsim_topk_keys_dev(const innr_cuda_corpus* c, const float* dev_q_tokens, size_t n_queries, size_t n_q,
+                                   int cosine_flag, size_t k, uint64_t* dev_keys, void* stream) {
+  if (!c || c->kind != 3) return fail(INNR_EINVAL, "need a token corpus");
+  if (k == 0 || n_queries == 0) return INNR_OK;
+  if (!dev_keys || (n_q * c->d && c->total_tokens && !dev_q_tokens)) return fail(INNR_EINVAL, "null argument");
+  EntryGuard lk(c->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  DeviceCtx* ctx;
+  int rc = ctx_for_dev(c, &ctx, s);  // lane 0: the score vectors live in the device's scratch
+  if (rc) return rc;
+  DevRelease rel(*ctx, s);
+  if (c->n == 0) {
+    CU(cudaMemsetAsync(dev_keys, 0xFF, n_queries * k * sizeof(uint64_t), s));
+    return INNR_OK;
+  }
+  CU(ctx->d_scores.reserve(maxsim_topk_chunk(c, n_queries) * c->n * sizeof(float)));
+  return maxsim_topk_keys(c, ctx, dev_q_tokens, n_queries, n_q, cosine_flag, k, dev_keys, (float*)ctx->d_scores.p, s);
+}
+
 // ------------------------------------------------------------------------------------------ asynchronous host-buffer calls
 // The host-facing top-k entries synchronise before they return, so a caller with one query per call pays the ramp at
 // both ends of every launch and leaves the GPU idle while it decodes. The _async forms queue the same work (query
@@ -2510,6 +2594,41 @@ int innr_cuda_batch_knn_u8_async(const innr_cuda_corpus* c, const float* queries
     if (rc) return rc;
     DevRelease rel(*ctx, t->stream, lane);
     rc = u8_keys(c, ctx, (const float*)t->d_query, n_queries, kk, (uint64_t*)t->d_keys, t->stream, lane);
+    if (rc) return rc;
+  }
+  rc = async_finish(t);
+  if (rc) return rc;
+  *out_ticket = t;
+  return INNR_OK;
+}
+
+int innr_cuda_maxsim_topk_async(const innr_cuda_corpus* c, const float* q_tokens, size_t n_queries, size_t n_q,
+                                size_t q_dim, int cosine_flag, size_t k, innr_cuda_ticket** out_ticket) {
+  if (!out_ticket) return fail(INNR_EINVAL, "null out_ticket");
+  *out_ticket = nullptr;
+  if (!c || c->kind != 3) return fail(INNR_EINVAL, "need a token corpus");
+  if (n_q && c->total_tokens && q_dim != c->d) return fail(INNR_EINVAL, "dimension mismatch (doc)");  // src/maxsim.rs:107-110
+  const bool empty = c->n == 0 || k == 0 || n_queries == 0;
+  if (!empty && n_q * q_dim && !q_tokens) return fail(INNR_EINVAL, "null argument");
+  const size_t kk = empty ? 0 : (k < c->n ? k : c->n);
+  EntryGuard lk(c->device);
+  DeviceCtx* ctx;
+  innr_cuda_ticket* t;
+  const size_t qbytes = (empty || !c->total_tokens) ? 0 : n_queries * n_q * c->d * sizeof(float);
+  int rc = async_begin(c, &ctx, &t, qbytes, n_queries, k, kk);
+  if (rc) return rc;
+  t->metric = INNR_METRIC_DOT;  // descending keys
+  if (!empty) {
+    if (qbytes) {
+      std::memcpy(t->h_in, q_tokens, qbytes);
+      CU(cudaMemcpyAsync(t->d_query, t->h_in, qbytes, cudaMemcpyHostToDevice, t->stream));
+    }
+    if ((rc = grow(&t->d_scores, &t->d_scores_cap, maxsim_topk_chunk(c, n_queries) * c->n * sizeof(float), false))) return rc;
+    rc = ensure_ctx(c->device, &ctx, WS_DEV, t->stream);  // lane 0: the selection uses ctx->ws
+    if (rc) return rc;
+    DevRelease rel(*ctx, t->stream);
+    rc = maxsim_topk_keys(c, ctx, (const float*)t->d_query, n_queries, n_q, cosine_flag, kk, (uint64_t*)t->d_keys,
+                          (float*)t->d_scores, t->stream);
     if (rc) return rc;
   }
   rc = async_finish(t);
@@ -3271,6 +3390,81 @@ int innr_cuda_batch_knn_u8_sharded(const innr_cuda_corpus* const* shards, size_t
   return INNR_OK;
 }
 
+// Token shards (one document range each): the argument checks of innr_cuda_maxsim_topk over the union of the shards.
+static int check_token_shards(const innr_cuda_corpus* const* shards, size_t n_shards, size_t n_q, size_t q_dim,
+                              size_t* n_total) {
+  if (!shards || n_shards == 0) return fail(INNR_EINVAL, "no shards");
+  size_t tokens = 0;
+  *n_total = 0;
+  for (size_t i = 0; i < n_shards; ++i) {
+    if (!shards[i] || shards[i]->kind != 3) return fail(INNR_EINVAL, "need token shards");
+    if (shards[i]->d != shards[0]->d) return fail(INNR_EINVAL, "shards differ in dimension");
+    *n_total += shards[i]->n;
+    tokens += shards[i]->total_tokens;
+  }
+  if (n_q && tokens && q_dim != shards[0]->d) return fail(INNR_EINVAL, "dimension mismatch (doc)");  // src/maxsim.rs:107-110
+  return INNR_OK;
+}
+
+int innr_cuda_maxsim_topk_sharded(const innr_cuda_corpus* const* shards, size_t n_shards, const float* q_tokens,
+                                  size_t n_queries, size_t n_q, size_t q_dim, int cosine_flag, size_t k, uint64_t* out_idx,
+                                  float* out_score, size_t* out_count) {
+  if (out_count) *out_count = 0;
+  size_t n_total = 0;
+  int rc = check_token_shards(shards, n_shards, n_q, q_dim, &n_total);
+  if (rc) return rc;
+  if (n_total == 0 || k == 0 || n_queries == 0) return INNR_OK;
+  if (!out_idx || !out_score || (n_q * q_dim && !q_tokens)) return fail(INNR_EINVAL, "null argument");
+  const size_t kk = k < n_total ? k : n_total;
+  // distinct devices: every shard scores and selects on its own stream, the lists meet in the root's mailbox
+  if (ShardGroup* g = shard_group_for(shards, n_shards)) {
+    const float none = 0.0f;
+    const size_t qbytes = n_queries * n_q * shards[0]->d * sizeof(float);
+    rc = sharded_via_exchange(g, shards, n_shards, qbytes ? (const void*)q_tokens : (const void*)&none, qbytes, n_queries, k,
+                              INNR_METRIC_DOT, false,
+                              [&](size_t i, DeviceCtx* ctx, void* dq, uint64_t* dk) -> int {
+                                const innr_cuda_corpus* c = shards[i];
+                                if (c->n == 0) {
+                                  CU(cudaMemsetAsync(dk, 0xFF, n_queries * k * sizeof(uint64_t), ctx->stream));
+                                  return INNR_OK;
+                                }
+                                CU(ctx->d_scores.reserve(maxsim_topk_chunk(c, n_queries) * c->n * sizeof(float)));
+                                return maxsim_topk_keys(c, ctx, (const float*)dq, n_queries, n_q, cosine_flag, k, dk,
+                                                        (float*)ctx->d_scores.p, ctx->stream);
+                              },
+                              out_idx, out_score, nullptr);
+    if (rc == INNR_OK) {
+      if (out_count) *out_count = kk;
+      return INNR_OK;
+    }
+    if (rc != INNR_EUNSUPPORTED) return rc;
+  }
+  std::vector<ShardOut> outs(n_shards);
+  rc = run_shards(n_shards, [&](size_t i, ShardOut& o) {
+    o.idx.assign(n_queries * k, 0);
+    o.score.assign(n_queries * k, 0.0f);
+    return innr_cuda_maxsim_topk(shards[i], q_tokens, n_queries, n_q, q_dim, cosine_flag, k, o.idx.data(), o.score.data(),
+                                 &o.count);
+  }, outs);
+  if (rc) return rc;
+  std::vector<std::pair<uint64_t, float>> all;
+  for (size_t q = 0; q < n_queries; ++q) {
+    all.clear();
+    for (size_t i = 0; i < n_shards; ++i)
+      for (size_t j = 0; j < outs[i].count; ++j) {
+        const float sc = outs[i].score[q * k + j];
+        all.emplace_back(((uint64_t)(~host_order_bits(sc)) << 32) | outs[i].idx[q * k + j], sc);
+      }
+    std::sort(all.begin(), all.end(), [](const auto& a, const auto& b) { return a.first < b.first; });
+    for (size_t j = 0; j < kk; ++j) {
+      out_idx[q * k + j] = all[j].first & 0xFFFFFFFFull;
+      out_score[q * k + j] = all[j].second;
+    }
+  }
+  if (out_count) *out_count = kk;
+  return INNR_OK;
+}
+
 // ---- asynchronous forms of the sharded entries (exchange route only: shards on pairwise distinct devices) ------------
 int innr_cuda_batch_knn_sharded_async(const innr_cuda_corpus* const* shards, size_t n_shards, int metric,
                                       const float* queries, size_t n_queries, size_t query_len, size_t k,
@@ -3372,6 +3566,38 @@ int innr_cuda_batch_knn_u8_sharded_async(const innr_cuda_corpus* const* shards, 
           return INNR_OK;
         }
         return u8_keys(c, ctx, (const float*)dq, n_queries, k, dk, s, lane);
+      },
+      out_ticket);
+}
+
+int innr_cuda_maxsim_topk_sharded_async(const innr_cuda_corpus* const* shards, size_t n_shards, const float* q_tokens,
+                                        size_t n_queries, size_t n_q, size_t q_dim, int cosine_flag, size_t k,
+                                        innr_cuda_ticket** out_ticket) {
+  if (!out_ticket) return fail(INNR_EINVAL, "null out_ticket");
+  *out_ticket = nullptr;
+  size_t n_total = 0;
+  int rc = check_token_shards(shards, n_shards, n_q, q_dim, &n_total);
+  if (rc) return rc;
+  if (n_total == 0 || k == 0 || n_queries == 0) return INNR_OK;  // empty result: no ticket
+  if (n_q * q_dim && !q_tokens) return fail(INNR_EINVAL, "null argument");
+  ShardGroup* g = shard_group_for(shards, n_shards);
+  if (!g) return fail(INNR_EUNSUPPORTED, "asynchronous sharded calls need two or more shards on pairwise distinct devices with peer access");
+  const float none = 0.0f;
+  const size_t qbytes = n_queries * n_q * shards[0]->d * sizeof(float);
+  return sharded_async_via_exchange(
+      g, shards, n_shards, qbytes ? (const void*)q_tokens : (const void*)&none, qbytes, n_queries, k,
+      k < n_total ? k : n_total, INNR_METRIC_DOT, [&](size_t) { return false; },  // lane 0: scratch score vectors
+      [&](size_t i, DeviceCtx* ctx, void* dq, uint64_t* dk, cudaStream_t s, int) -> int {
+        const innr_cuda_corpus* c = shards[i];
+        if (c->n == 0) {
+          CU(cudaMemsetAsync(dk, 0xFF, n_queries * k * sizeof(uint64_t), s));
+          return INNR_OK;
+        }
+        // the score vectors belong to the asynchronous slot this call runs in (the one whose stream is `s`)
+        innr_cuda_ticket* t = ctx->async_slot[0].stream == s ? &ctx->async_slot[0] : &ctx->async_slot[1];
+        int r = grow(&t->d_scores, &t->d_scores_cap, maxsim_topk_chunk(c, n_queries) * c->n * sizeof(float), false);
+        if (r) return r;
+        return maxsim_topk_keys(c, ctx, (const float*)dq, n_queries, n_q, cosine_flag, k, dk, (float*)t->d_scores, s);
       },
       out_ticket);
 }

@@ -72,6 +72,29 @@ def maxsim_corpus_batch(queries, corpus: TokenCorpus, cosine: bool = False) -> n
     return out
 
 
+def maxsim_topk(query_tokens, corpus: TokenCorpus, k: int, cosine: bool = False):
+    """The k best documents for one query token set: (indices uint64[min(k, num_docs)], scores float32[...]), scores
+    descending under f32::total_cmp, exact ties -> lower index (index_base + doc). The scores are maxsim_corpus's bit
+    for bit: the result is a stable descending total_cmp sort of its output, truncated to k, computed on the device."""
+    q = _tokens(query_tokens, "query")
+    idx, sc = maxsim_topk_batch(q.reshape(1, q.shape[0], q.shape[1]), corpus, k, cosine)
+    return idx[0], sc[0]
+
+
+def maxsim_topk_batch(queries, corpus: TokenCorpus, k: int, cosine: bool = False):
+    """`queries`: (n_queries, n_q, dim). Returns (indices uint64[n_queries, min(k, num_docs)], scores float32[...]);
+    row i equals maxsim_topk(queries[i], ...)."""
+    q = np.ascontiguousarray(queries, dtype=np.float32)
+    assert q.ndim == 3, "queries must be (n_queries, n_q, dim)"
+    nq, kk = q.shape[0], max(int(k), 1)
+    idx = np.zeros((nq, kk), np.uint64)
+    sc = np.zeros((nq, kk), np.float32)
+    cnt = C.c_size_t(0)
+    L.call("innr_cuda_maxsim_topk", corpus.h, q.ctypes.data_as(L.f32p), nq, q.shape[1], q.shape[2] if q.shape[1] else 0,
+           1 if cosine else 0, k, idx.ctypes.data_as(L.u64p), sc.ctypes.data_as(L.f32p), C.byref(cnt))
+    return idx[:, :cnt.value], sc[:, :cnt.value]
+
+
 def _pair(query_tokens, doc_tokens, cosine: bool) -> float:
     q, d = _tokens(query_tokens, "query"), _tokens(doc_tokens, "doc")
     if q.shape[0] == 0 or d.shape[0] == 0:

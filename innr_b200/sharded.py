@@ -122,11 +122,12 @@ class PeerExchange:
 
 
 class ShardedKnn:
-    """One rank's view of a row-sharded corpus. kind: 'f32' (DeviceBatch), 'u8' (U8Corpus), 'binary' (BinaryCorpus).
-    `exchange`: a connected PeerExchange (keys travel through peer-mapped mailboxes, one launch) or None (one NCCL
-    `all_gather_into_tensor` of k keys per rank + the merge launch)."""
+    """One rank's view of a row-sharded corpus. kind: 'f32' (DeviceBatch), 'u8' (U8Corpus), 'binary' (BinaryCorpus),
+    'maxsim' (TokenCorpus, a document range; metric 'dot' or 'cosine'; queries of `query_tokens` tokens each, passed as
+    nq x query_tokens x dim floats). `exchange`: a connected PeerExchange (keys travel through peer-mapped mailboxes, one
+    launch) or None (one NCCL `all_gather_into_tensor` of k keys per rank + the merge launch)."""
 
-    def __init__(self, shard, kind: str = "f32", metric: str = "cosine", group=None, exchange=None):
+    def __init__(self, shard, kind: str = "f32", metric: str = "cosine", group=None, exchange=None, query_tokens: int = 0):
         import torch
         import torch.distributed as dist
         self.torch, self.dist = torch, dist
@@ -134,6 +135,8 @@ class ShardedKnn:
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.exchange = exchange
         self._metric_id = {"dot": L.METRIC_DOT, "cosine": L.METRIC_COSINE, "l2": L.METRIC_L2}[metric]
+        assert kind != "maxsim" or metric in ("dot", "cosine"), "MaxSim ranks by dot or cosine"
+        self.query_tokens = int(query_tokens)
         self._bufs = {}
 
     def _buffers(self, nq: int, k: int, device):
@@ -159,14 +162,7 @@ class ShardedKnn:
         t = self.torch
         stream = C.c_void_p(t.cuda.current_stream().cuda_stream)
         b = self._buffers(nq, k, dev_queries.device)
-        qp = C.c_void_p(dev_queries.data_ptr())
-        lp = b["p"]["local"]
-        if self.kind == "f32":
-            L.call("innr_cuda_batch_knn_keys_dev", self.shard.h, self._metric_id, qp, nq, k, lp, stream)
-        elif self.kind == "u8":
-            L.call("innr_cuda_batch_knn_u8_keys_dev", self.shard.h, qp, nq, k, lp, stream)
-        else:
-            L.call("innr_cuda_hamming_topk_keys_dev", self.shard.h, qp, nq, k, lp, stream)
+        self._keys(dev_queries, nq, k, b["local"], stream)
         if self.exchange is not None and self.exchange.fits(nq, k):
             # publish / wait / merge / decode in ONE launch, no collective call
             if self.kind == "binary":
@@ -197,12 +193,18 @@ class ShardedKnn:
             L.call("innr_cuda_batch_knn_keys_dev", self.shard.h, self._metric_id, qp, nq, k, lp, stream)
         elif self.kind == "u8":
             L.call("innr_cuda_batch_knn_u8_keys_dev", self.shard.h, qp, nq, k, lp, stream)
+        elif self.kind == "maxsim":
+            L.call("innr_cuda_maxsim_topk_keys_dev", self.shard.h, qp, nq, self.query_tokens, int(self.metric == "cosine"), k,
+                   lp, stream)
         else:
             L.call("innr_cuda_hamming_topk_keys_dev", self.shard.h, qp, nq, k, lp, stream)
 
     def knn_dev_pipelined(self, dev_queries, nq: int, k: int, overlap_scans: bool = True, host_queries=None,
                           host_out: bool = False):
-        """Throughput form of knn_dev for a stream of independent queries. Two things overlap here that knn_dev serialises:
+        """Throughput form of knn_dev for a stream of independent queries. Two things overlap here that knn_dev serialises
+        (kind 'maxsim': only the second -- its tcgen05 kernel fills every SM and its score vectors live in the library's
+        one scratch lane, so two MaxSim scans cannot overlap; overlap_scans is ignored and the scans stay on torch's
+        current stream, while the exchange still runs on the side stream):
 
         * consecutive shard scans. They alternate between two scan streams (the library keeps two workspaces per device
           for exactly this, api.cu `lane`), so the CTAs of scan i + 1 fill the SMs as the last CTAs of scan i retire and
@@ -225,6 +227,8 @@ class ShardedKnn:
         pinned host tensors behind the merge, on its stream -- the returned (idx, score) are then those HOST tensors,
         complete when `event` is. One host synchronisation per batch of calls instead of one per call."""
         t = self.torch
+        if self.kind == "maxsim":
+            overlap_scans = False
         if host_queries is not None and ((self.exchange is None and self.world > 1) or k > 128
                                          or (self.exchange is not None and not self.exchange.fits(nq, k))):
             dev_queries = host_queries.to(f"cuda:{t.cuda.current_device()}", non_blocking=True)
@@ -320,8 +324,8 @@ class ShardedKnn:
         """End-to-end call with HOST buffers: H2D of the queries, shard scan, allgather, merge, D2H of the result."""
         t = self.torch
         q = np.ascontiguousarray(queries_host)
-        if q.ndim == 1:
-            q = q.reshape(1, -1)
+        if q.ndim == 1 or (self.kind == "maxsim" and q.ndim == 2):
+            q = q.reshape((1,) + q.shape)
         nq = q.shape[0]
         src = t.from_numpy(q.view(np.int64) if self.kind == "binary" else q)
         dq = src.to(f"cuda:{t.cuda.current_device()}", non_blocking=True)
@@ -377,4 +381,20 @@ def batch_knn_u8_sharded(queries, shards, k: int):
     cnt = C.c_size_t(0)
     L.call("innr_cuda_batch_knn_u8_sharded", _handle_array(shards), len(shards), qs.ctypes.data_as(L.f32p), nq, qlen, k,
            idx.ctypes.data_as(L.u64p), sc.ctypes.data_as(L.f32p), C.byref(cnt))
+    return idx[:, :cnt.value], sc[:, :cnt.value]
+
+
+def maxsim_topk_sharded(queries, shards, k: int, cosine: bool = False):
+    """maxsim_topk_batch over TokenCorpus shards (document ranges, each with its index_base; on distinct devices the
+    lists meet in the peer-mapped exchange, otherwise one host thread per shard and a host merge). `queries`:
+    (n_queries, n_q, dim). Equals the unsharded call over the whole document set."""
+    qs = np.ascontiguousarray(queries, dtype=np.float32)
+    assert qs.ndim == 3, "queries must be (n_queries, n_q, dim)"
+    nq = qs.shape[0]
+    kk = max(k, 1)
+    idx = np.zeros((nq, kk), np.uint64)
+    sc = np.zeros((nq, kk), np.float32)
+    cnt = C.c_size_t(0)
+    L.call("innr_cuda_maxsim_topk_sharded", _handle_array(shards), len(shards), qs.ctypes.data_as(L.f32p), nq, qs.shape[1],
+           qs.shape[2], 1 if cosine else 0, k, idx.ctypes.data_as(L.u64p), sc.ctypes.data_as(L.f32p), C.byref(cnt))
     return idx[:, :cnt.value], sc[:, :cnt.value]

@@ -87,6 +87,17 @@ def submit_knn_u8(queries, corpus, k: int) -> Ticket:
     return Ticket(h, "u8", nq, k)
 
 
+def submit_maxsim_topk(queries, corpus, k: int, cosine: bool = False) -> Ticket:
+    """maxsim_topk_batch over a TokenCorpus (`queries`: (n_queries, n_q, dim)), queued. Each of the device's two slots
+    owns its score vectors, so two calls in flight never share scratch."""
+    qs = np.ascontiguousarray(queries, dtype=np.float32)
+    assert qs.ndim == 3, "queries must be (n_queries, n_q, dim)"
+    h = C.c_void_p()
+    L.call("innr_cuda_maxsim_topk_async", corpus.h, qs.ctypes.data_as(L.f32p), qs.shape[0], qs.shape[1], qs.shape[2],
+           1 if cosine else 0, k, C.byref(h))
+    return Ticket(h, "maxsim", qs.shape[0], k)
+
+
 # ---- row shards on different devices of this process (innr_cuda_*_sharded_async): one ticket per call ------------------
 def _shard_handles(shards):
     return (C.c_void_p * len(shards))(*[sh.h for sh in shards])
@@ -123,3 +134,12 @@ def submit_knn_u8_sharded(queries, shards, k: int) -> Ticket:
     L.call("innr_cuda_batch_knn_u8_sharded_async", _shard_handles(shards), len(shards), qs.ctypes.data_as(L.f32p), nq, qlen, k,
            C.byref(h))
     return Ticket(h, "u8", nq, k)
+
+
+def submit_maxsim_topk_sharded(queries, shards, k: int, cosine: bool = False) -> Ticket:
+    qs = np.ascontiguousarray(queries, dtype=np.float32)
+    assert qs.ndim == 3, "queries must be (n_queries, n_q, dim)"
+    h = C.c_void_p()
+    L.call("innr_cuda_maxsim_topk_sharded_async", _shard_handles(shards), len(shards), qs.ctypes.data_as(L.f32p), qs.shape[0],
+           qs.shape[1], qs.shape[2], 1 if cosine else 0, k, C.byref(h))
+    return Ticket(h, "maxsim", qs.shape[0], k)
