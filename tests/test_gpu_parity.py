@@ -1449,7 +1449,9 @@ def tc_small(ib):
 def test_knn_tc_filter_path_is_exact(tc_small, oracle, n, d, nq):
     """Large query batches go through tcgen05 as a pruning filter (csrc/knn_tc.cu); the exact rescoring must make the
     result bit-identical to the reference (indices AND scores), including zero / tiny / huge vectors and queries,
-    duplicates (ties -> lower index first) and queries the filter hands to the exact scan."""
+    duplicates (ties -> lower index first) and queries the filter hands to the exact scan. At these sizes (<= 300 K
+    rows) the prefix schedule is short: the n/256 pass and, for k > 32, the n/128 pass never run. The schedule itself
+    is covered at product shape by tests/test_gpu_knn_tc_passes.py."""
     ib = tc_small
     rows = rand_rows(n, d, n + d)
     rows[17] = 0.0                      # zero-norm vector -> cosine 0.0
