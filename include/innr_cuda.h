@@ -93,6 +93,22 @@ int innr_cuda_knn_tc_debug_bounds(const innr_cuda_corpus* c, int metric, const f
  * reference's epsilon). */
 int innr_cuda_knn_screen_debug_bounds(const innr_cuda_corpus* c, int metric, const float* query, size_t query_len,
                                       float* out_lower, float* out_upper);
+/* Statistics of the last batch_knn_u8 call that took the tensor-core filter (u8_tc.cu; options "u8_tc", "u8_tc_min_n",
+ * "u8_tc_min_queries", "u8_tc_max_k" of innr_cuda_set_option select it, results never depend on them): device time of the
+ * final filter passes and of the whole call (ms), integer operations those passes issued (2 x rows x padded d x padded
+ * queries; calls run in batches of 1024 queries, summed over the batches), pairs
+ * re-scored exactly, queries answered by the exact scan instead, filter passes. Any pointer may be NULL. Kept apart from
+ * innr_cuda_knn_tc_last_stats, which reports f32 calls only. */
+int innr_cuda_u8_tc_last_stats(float* out_filter_ms, float* out_total_ms, double* out_filter_ops,
+                               uint64_t* out_candidates, uint32_t* out_exact_scan_queries, int* out_passes);
+/* Test hook for the u8 filter's bound: runs the operands + the dense first pass of the filter and returns, for every
+ * query and every row < min(n, 4096), the score interval [lower, upper] exactly as production computes it (row-major
+ * n_queries x *out_rows each), and per query 1 when the filter does not answer it (a non-finite or all-zero query,
+ * largest |element| outside [2^-100, 2^100], non-finite offset * query_sum). The tests assert
+ * lower <= reference score <= upper on adversarial inputs. At most 1024 queries. INNR_EUNSUPPORTED when the corpus
+ * cannot take the filter (alpha / 255 not finite and positive, d > 8192). */
+int innr_cuda_u8_tc_debug_bounds(const innr_cuda_corpus* c, const float* queries, size_t n_queries, size_t query_len,
+                                 float* out_lower, float* out_upper, size_t* out_rows, uint32_t* out_qflags);
 /* number of kernels the library has launched so far (bench.py's gpu_launches counter) */
 int innr_cuda_launch_count(uint64_t* out_count);
 

@@ -45,8 +45,10 @@ struct innr_cuda_corpus {
   // scales and bounds finite for every row
   uint8_t* dev_sketch = nullptr;
   bool screen = false;
-  // f32 PDX: lazily built operands of the tensor-core filter path (knn_tc.cu): exact norms, f16 unit vectors + TMA map
+  // f32 PDX: lazily built operands of the tensor-core filter path (knn_tc.cu): exact norms, f16 unit vectors + TMA map;
+  // u8: the row radii of its filter path (u8_tc.cu, dev_radius)
   int tc_state = 0;  // 0 not built, 1 ready, -1 unusable (non-finite norms / no memory): exact scan only
+  float* dev_radius = nullptr;
   float* dev_norms = nullptr;
   void* dev_xh = nullptr;
   CUtensorMap tm_xh;
@@ -160,6 +162,13 @@ struct Options {
   size_t knn_tc_min_queries = 2;  // measured at 10M x 768: filter call 2.6 ms for 2..64 queries, 8-query scan pass 6.3 ms
   size_t f32_split_min_rows = 1000000;  // owned f32 corpora from this many rows are stored split (DESIGN.md section 2)
   bool maxsim_tc = true;
+  bool u8_tc = true;
+  // measured at C5 (50M x 384, DESIGN.md section 3.10): k = 10, 8 queries 7.8 ms against 18.8 ms on the pair kernel, 2 queries
+  // 7.8 against 4.8. Above k = 32 the candidate lists overflow for most queries (k = 100, 1024 queries: 978 re-run on the
+  // scan, slower than the pair kernel), so larger k stay on the scan.
+  size_t u8_tc_min_n = 100000;
+  size_t u8_tc_min_queries = 8;
+  size_t u8_tc_max_k = 32;
   bool kernel_timing = false;
 } g_opt;
 
@@ -170,6 +179,7 @@ std::mutex g_dev_mu[MAX_DEVICES];
 DeviceCtx g_ctx[MAX_DEVICES];
 LaunchCounter g_launches{0};
 KnnTcStats g_tc_stats;
+KnnTcStats g_u8tc_stats;  // the last u8 filter call (kept apart: knn_tc_last_stats reports f32 calls only)
 thread_local int t_device = -1;
 thread_local std::string t_err;
 std::mutex& dev_mu(int d) { return g_dev_mu[(d >= 0 && d < MAX_DEVICES) ? d : 0]; }
@@ -363,6 +373,7 @@ void destroy_corpus(innr_cuda_corpus* c) {
   if (c->dev_norms) cudaFree(c->dev_norms);
   if (c->dev_sketch) cudaFree(c->dev_sketch);
   if (c->dev_xh) cudaFree(c->dev_xh);
+  if (c->dev_radius) cudaFree(c->dev_radius);
   if (c->dev_order) cudaFree(c->dev_order);
   delete c;
 }
@@ -491,6 +502,10 @@ int innr_cuda_set_option(const char* name, double value) {
   else if (n == "knn_tc_min_queries") g_opt.knn_tc_min_queries = (size_t)value;
   else if (n == "f32_split_min_rows") g_opt.f32_split_min_rows = (size_t)value;
   else if (n == "maxsim_tc") g_opt.maxsim_tc = value != 0;
+  else if (n == "u8_tc") g_opt.u8_tc = value != 0;
+  else if (n == "u8_tc_min_n") g_opt.u8_tc_min_n = (size_t)value;
+  else if (n == "u8_tc_min_queries") g_opt.u8_tc_min_queries = (size_t)value;
+  else if (n == "u8_tc_max_k") g_opt.u8_tc_max_k = (size_t)value;
   else if (n == "kernel_timing") g_opt.kernel_timing = value != 0;
   else if (n == "u8_scaled_chains") u8_set_scaled_chains(value != 0);
   else return fail(INNR_EINVAL, "unknown option: " + n);
@@ -505,6 +520,17 @@ int innr_cuda_knn_tc_last_stats(float* out_filter_ms, float* out_total_ms, doubl
   if (out_candidates) *out_candidates = g_tc_stats.candidates;
   if (out_exact_scan_queries) *out_exact_scan_queries = g_tc_stats.overflowed;
   if (out_passes) *out_passes = g_tc_stats.passes;
+  return INNR_OK;
+}
+int innr_cuda_u8_tc_last_stats(float* out_filter_ms, float* out_total_ms, double* out_filter_ops,
+                               uint64_t* out_candidates, uint32_t* out_exact_scan_queries, int* out_passes) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  if (out_filter_ms) *out_filter_ms = g_u8tc_stats.filter_ms;
+  if (out_total_ms) *out_total_ms = g_u8tc_stats.total_ms;
+  if (out_filter_ops) *out_filter_ops = g_u8tc_stats.filter_flops;
+  if (out_candidates) *out_candidates = g_u8tc_stats.candidates;
+  if (out_exact_scan_queries) *out_exact_scan_queries = g_u8tc_stats.overflowed;
+  if (out_passes) *out_passes = g_u8tc_stats.passes;
   return INNR_OK;
 }
 int innr_cuda_launch_count(uint64_t* out_count) {
@@ -1920,8 +1946,52 @@ int innr_cuda_asymmetric_dot_u8_all(const innr_cuda_corpus* c, const float* quer
   return u8_scores(c, 1, query, query_len, out_host, "asymmetric_dot_u8: dimension mismatch");
 }
 
+// Large batches go through the tensor-core filter (u8_tc.cu: exact results, see there) when the corpus qualifies;
+// innr_cuda_set_option("u8_tc", 0) disables it. Single queries always take the scan.
+static bool u8_takes_tc_filter(const innr_cuda_corpus* c, size_t nq, size_t k) {
+  return g_opt.u8_tc && c->n >= g_opt.u8_tc_min_n && nq >= g_opt.u8_tc_min_queries && nq >= 2 && k <= g_opt.u8_tc_max_k &&
+         u8_tc_supported(u8_view(c), nq, k);
+}
+// the pair / single-query scans need a Workspace and nothing else: either lane will do
+static bool u8_is_scan_only(const innr_cuda_corpus* c, size_t nq, size_t k) {
+  return k <= MAX_FUSED_K && !u8_takes_tc_filter(c, nq, k);
+}
+// The row radii of the filter path, built on first use (the handle stays immutable: a cache of the same data). On failure
+// (no memory) the corpus stays on the exact scan.
+static int u8_tc_prepare(innr_cuda_corpus* c, cudaStream_t s) {
+  if (c->tc_state != 0) return INNR_OK;
+  c->tc_state = -1;
+  if (cudaMalloc(&c->dev_radius, c->n * sizeof(float)) != cudaSuccess) {
+    cudaGetLastError();  // out of memory is not an error of the call: exact scan
+    c->dev_radius = nullptr;
+    return INNR_OK;
+  }
+  CU(launch_u8_tc_radius(u8_view(c), c->dev_radius, s, &g_launches));
+  c->tc_state = 1;
+  return INNR_OK;
+}
 static int u8_keys(const innr_cuda_corpus* c, DeviceCtx* ctx, const float* dev_queries, size_t nq, size_t k,
                    uint64_t* dev_keys, cudaStream_t s, int lane = 0) {
+  if (u8_takes_tc_filter(c, nq, k)) {  // lane 0: the filter's scratch
+    innr_cuda_corpus* cm = const_cast<innr_cuda_corpus*>(c);
+    int rc = u8_tc_prepare(cm, s);
+    if (rc) return rc;
+    if (c->tc_state == 1) {
+      CU(ctx->d_tcws.reserve(u8_tc_workspace_bytes(c->d, nq, false)));
+      CU(ctx->h_counts.reserve((nq < 1024 ? nq : 1024) * sizeof(unsigned)));
+      std::vector<unsigned> overflow;
+      KnnTcStats st;
+      CU(launch_u8_knn_tc(u8_view(c), c->dev_radius, dev_queries, nq, k, dev_keys, ctx->d_tcws.p, (unsigned*)ctx->h_counts.p,
+                          ctx->ws, s, &g_launches, &overflow, &st));
+      {
+        std::lock_guard<std::mutex> lg(g_mu);
+        g_u8tc_stats = st;
+      }
+      for (unsigned q : overflow)
+        CU(launch_u8_knn(u8_view(c), dev_queries + (size_t)q * c->d, 1, k, dev_keys + (size_t)q * k, ctx->ws, s, &g_launches));
+      return INNR_OK;
+    }
+  }
   if (k <= MAX_FUSED_K) {
     CU(launch_u8_knn(u8_view(c), dev_queries, nq, k, dev_keys, ctx->lane_ws(lane), s, &g_launches));
     return INNR_OK;
@@ -1973,7 +2043,7 @@ int innr_cuda_batch_knn_u8_keys_dev(const innr_cuda_corpus* c, const float* dev_
   cudaStream_t s = (cudaStream_t)stream;
   DeviceCtx* ctx;
   int lane = 0;
-  int rc = ctx_for_dev(c, &ctx, s, k <= MAX_FUSED_K, &lane);
+  int rc = ctx_for_dev(c, &ctx, s, u8_is_scan_only(c, n_queries, k), &lane);
   if (rc) return rc;
   DevRelease rel(*ctx, s, lane);
   if (c->n == 0 || c->d == 0) {
@@ -1981,6 +2051,32 @@ int innr_cuda_batch_knn_u8_keys_dev(const innr_cuda_corpus* c, const float* dev_
     return INNR_OK;
   }
   return u8_keys(c, ctx, dev_queries, n_queries, k, dev_keys, s, lane);
+}
+
+// Test hook for the u8 filter's bound (tests/test_gpu_u8_tc.py): the score interval [lower, upper] of the dense first
+// pass for rows < min(n, 4096), row-major n_queries x *out_rows, exactly as the filter computes it, plus the per-query flag
+// (1 = the filter does not answer this query: it goes to the exact scan). INNR_EUNSUPPORTED when the corpus cannot take
+// the filter path (alpha / 255 not finite and positive, d > 8192, no memory).
+extern "C" int innr_cuda_u8_tc_debug_bounds(const innr_cuda_corpus* c, const float* queries, size_t n_queries, size_t query_len,
+                                            float* out_lower, float* out_upper, size_t* out_rows, uint32_t* out_qflags) {
+  if (!c || c->kind != 2) return fail(INNR_EINVAL, "need a u8 corpus");
+  if (query_len != c->d) return fail(INNR_EINVAL, "asymmetric_dot_u8_precomputed: dimension mismatch");
+  if (!queries || !out_lower || !out_upper || !out_rows || !out_qflags || n_queries == 0) return fail(INNR_EINVAL, "null argument");
+  if (n_queries > 1024) return fail(INNR_EINVAL, "at most 1024 queries per call");
+  if (!u8_tc_supported(u8_view(c), n_queries, 1)) return fail(INNR_EUNSUPPORTED, "corpus cannot take the u8 filter path");
+  EntryGuard lk(c->device);
+  DeviceCtx* ctx;
+  int rc = ctx_for(c, &ctx);
+  if (rc) return rc;
+  rc = u8_tc_prepare(const_cast<innr_cuda_corpus*>(c), ctx->stream);
+  if (rc) return rc;
+  if (c->tc_state != 1) return fail(INNR_EUNSUPPORTED, "corpus cannot take the u8 filter path (no memory)");
+  CU(ctx->d_query.reserve((n_queries * c->d + 4) * sizeof(float)));
+  CU(ctx->d_tcws.reserve(u8_tc_workspace_bytes(c->d, n_queries, true)));
+  CU(cudaMemcpyAsync(ctx->d_query.p, queries, n_queries * c->d * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  CU(launch_u8_tc_debug_bounds(u8_view(c), c->dev_radius, (const float*)ctx->d_query.p, n_queries, ctx->d_tcws.p, out_lower,
+                               out_upper, out_rows, out_qflags, ctx->ws.num_sms, ctx->stream, &g_launches));
+  return INNR_OK;
 }
 
 // ------------------------------------------------------------------------------------------ ternary codes
@@ -2590,7 +2686,7 @@ int innr_cuda_batch_knn_u8_async(const innr_cuda_corpus* c, const float* queries
     std::memcpy(t->h_in, queries, qbytes);
     CU(cudaMemcpyAsync(t->d_query, t->h_in, qbytes, cudaMemcpyHostToDevice, t->stream));
     int lane = 0;
-    rc = ensure_ctx(c->device, &ctx, kk <= MAX_FUSED_K ? WS_DEV_SCAN : WS_DEV, t->stream, &lane);
+    rc = ensure_ctx(c->device, &ctx, u8_is_scan_only(c, n_queries, kk) ? WS_DEV_SCAN : WS_DEV, t->stream, &lane);
     if (rc) return rc;
     DevRelease rel(*ctx, t->stream, lane);
     rc = u8_keys(c, ctx, (const float*)t->d_query, n_queries, kk, (uint64_t*)t->d_keys, t->stream, lane);
@@ -3558,7 +3654,7 @@ int innr_cuda_batch_knn_u8_sharded_async(const innr_cuda_corpus* const* shards, 
   if (!g) return fail(INNR_EUNSUPPORTED, "asynchronous sharded calls need two or more shards on pairwise distinct devices with peer access");
   return sharded_async_via_exchange(
       g, shards, n_shards, queries, n_queries * query_len * sizeof(float), n_queries, k, k < n_total ? k : n_total,
-      INNR_METRIC_DOT, [&](size_t) { return true; },
+      INNR_METRIC_DOT, [&](size_t i) { return shards[i]->n == 0 || u8_is_scan_only(shards[i], n_queries, k); },
       [&](size_t i, DeviceCtx* ctx, void* dq, uint64_t* dk, cudaStream_t s, int lane) -> int {
         const innr_cuda_corpus* c = shards[i];
         if (c->n == 0) {

@@ -280,6 +280,21 @@ cudaError_t launch_ternary_topk(const TerView& v, int op, const uint64_t* dev_qu
 void u8_set_scaled_chains(bool on);  // off = always the de-biasing path (tests compare both)
 cudaError_t launch_u8_knn(const U8View& v, const float* dev_queries, size_t nq, size_t k, uint64_t* dev_keys,
                           Workspace& ws, cudaStream_t s, LaunchCounter* launches);
+// tensor-core filter path for u8 query batches (u8_tc.cu): exact results, k <= 128; statistics in KnnTcStats
+// (filter_flops = integer operations of the final pass)
+bool u8_tc_supported(const U8View& v, size_t nq, size_t k);
+size_t u8_tc_workspace_bytes(size_t d, size_t nq, bool debug);
+// once per corpus: dev_radius[i] = ||b_i - 128||_2 rounded up (n floats)
+cudaError_t launch_u8_tc_radius(const U8View& v, float* dev_radius, cudaStream_t s, LaunchCounter* launches);
+// test hook: score interval of the dense first pass (rows < min(n, 4096)) for every query; see u8_tc.cu
+cudaError_t launch_u8_tc_debug_bounds(const U8View& v, const float* dev_radius, const float* dev_queries, size_t nq,
+                                      void* workspace, float* host_lower, float* host_upper, size_t* out_rows,
+                                      unsigned* host_qflags, int num_sms, cudaStream_t s, LaunchCounter* launches);
+// host_counts: pinned buffer of nq unsigned; overflow_queries receives the queries the filter could not answer
+// (the caller re-runs them on the exact scan). Synchronises the stream once at the end.
+cudaError_t launch_u8_knn_tc(const U8View& v, const float* dev_radius, const float* dev_queries, size_t nq, size_t k,
+                             uint64_t* dev_keys, void* workspace, unsigned* host_counts, Workspace& ws, cudaStream_t s,
+                             LaunchCounter* launches, std::vector<unsigned>* overflow_queries, KnnTcStats* stats);
 
 // MaxSim (maxsim.cu)
 struct TokView {

@@ -39,6 +39,7 @@
 #include "kernels.cuh"
 #include "pdx.cuh"
 #include "tc_common.cuh"
+#include "tc_filter.cuh"
 
 namespace innr {
 
@@ -64,7 +65,7 @@ constexpr int QR_STAGES = 7;    // 7 x 16 KB ring + 96 KB of Q + barriers and pe
 constexpr int KT_MAX_STAGES = 8;
 constexpr float COS_NORM_EPS = 1e-9f;   // src/batch.rs:721-727
 constexpr float TINY_NORM = 1e-30f;     // below this a vector / query is not normalised (handled by the exact path)
-constexpr unsigned CAND_CAP = 4096;
+using tcf::CAND_CAP;
 
 struct KtShared {
   uint64_t full[KT_MAX_STAGES], empty[KT_MAX_STAGES], acc_full[2], acc_empty[2], q_full;
@@ -406,34 +407,6 @@ __global__ void knn_tc_prep_queries_kernel(const float* __restrict__ q, unsigned
   }
 }
 
-// ---- between passes: threshold of the next pass = k-th largest lower bound among the appended pairs ------------------
-// one warp per query; also resets the counter for the next pass
-template <int R>
-__global__ void knn_tc_select_kernel(unsigned nq, unsigned k, const unsigned* __restrict__ qflag,
-                                     unsigned* __restrict__ cand_count, const float* __restrict__ cand_lb,
-                                     float* __restrict__ thr) {
-  const unsigned q = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  const int lane = threadIdx.x & 31;
-  if (q >= nq) return;
-  if (qflag[q]) return;  // thr stays +inf
-  unsigned cnt = cand_count[q];
-  if (cnt > CAND_CAP) cnt = CAND_CAP;  // any k stored pairs give a valid bound
-  WarpList<R> list;
-  list.init();
-  uint64_t t = KEY_SENTINEL;
-  for (unsigned c0 = 0; c0 < cnt; c0 += 32) {
-    const unsigned c = c0 + lane;
-    const bool valid = c < cnt;
-    const float lb = valid ? cand_lb[(size_t)q * CAND_CAP + c] : 0.0f;
-    list.offer(make_key_desc(lb, c), valid, t, (int)k, lane);
-  }
-  const uint64_t kth = list.at((int)k - 1);
-  if (lane == 0) {
-    thr[q] = (kth == KEY_SENTINEL) ? -INFINITY : __uint_as_float(order_bits_to_f32_bits(~(uint32_t)(kth >> 32)));
-    cand_count[q] = 0;
-  }
-}
-
 // ---- exact rescoring + selection: one CTA per query -------------------------------------------------------------------
 constexpr int RS_THREADS = 256;
 
@@ -574,16 +547,15 @@ KnnTcPlan make_plan(size_t d, size_t nq) {
   KnnTcPlan p{};
   p.nq_pad = (unsigned)((nq + 15) / 16 * 16);
   p.d_pad = (unsigned)knn_tc_dpad(d);
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o += (bytes + 1023) / 1024 * 1024; return r; };
-  p.off_qh = take((size_t)p.nq_pad * p.d_pad * 2);
-  p.off_qflag = take((size_t)p.nq_pad * 4);
-  p.off_thr = take((size_t)p.nq_pad * 4);
-  p.off_cnt = take((size_t)p.nq_pad * 4);
-  p.off_qaux = take((size_t)p.nq_pad * 3 * 4);
-  p.off_idx = take((size_t)p.nq_pad * CAND_CAP * 4);
-  p.off_lb = take((size_t)p.nq_pad * CAND_CAP * 4);
-  p.total = o;
+  tcf::WsCursor w;
+  p.off_qh = w.take((size_t)p.nq_pad * p.d_pad * 2);
+  p.off_qflag = w.take((size_t)p.nq_pad * 4);
+  p.off_thr = w.take((size_t)p.nq_pad * 4);
+  p.off_cnt = w.take((size_t)p.nq_pad * 4);
+  p.off_qaux = w.take((size_t)p.nq_pad * 3 * 4);
+  p.off_idx = w.take((size_t)p.nq_pad * CAND_CAP * 4);
+  p.off_lb = w.take((size_t)p.nq_pad * CAND_CAP * 4);
+  p.total = w.o;
   return p;
 }
 
@@ -717,12 +689,9 @@ cudaError_t launch_pdx_knn_tc(const PdxView& v, const CUtensorMap& tm_xh, const 
   tmark();
 
   // 1. operands, first-pass thresholds, zeroed counters
-  // The dense first pass keeps every pair of its rows. For k <= 32, 1024 rows are enough: the k-th best of a 1024-row
-  // sample lets about rows_next / 1024 * k pairs per query through the next pass, and the selection over 1024 pairs
-  // costs a quarter of what it cost over 4096 (0.15 ms of the 1024-query call). Larger k keep 4096.
+  // the dense first pass keeps every pair of its rows (tc_filter.cuh)
   static const int first_env = getenv("INNR_KNN_TC_FIRST") ? atoi(getenv("INNR_KNN_TC_FIRST")) : 0;
-  const size_t first_rows = std::min<size_t>(v.n, first_env > 0 ? std::min<size_t>((size_t)first_env, CAND_CAP)
-                                                                : (k <= 32 ? (size_t)1024 : (size_t)CAND_CAP));
+  const size_t first_rows = tcf::first_rows(v.n, k, first_env);
   knn_tc_prep_queries_kernel<<<p.nq_pad, 128, 0, s>>>(dev_queries, (unsigned)nq, (unsigned)v.d, p.nq_pad, p.d_pad, cosine, l2, qh,
                                                       qflag, thr, cnt, qaux, (unsigned)first_rows);
   ++*launches;
@@ -744,42 +713,8 @@ cudaError_t launch_pdx_knn_tc(const PdxView& v, const CUtensorMap& tm_xh, const 
     attr_set = true;
   }
   size_t levels[6];
-  int n_levels = 0;
-  {
-    size_t cur = first_rows;
-    levels[n_levels++] = cur;
-    static const int sched = getenv("INNR_KNN_TC_SCHED") ? atoi(getenv("INNR_KNN_TC_SCHED")) : 0;
-    // Prefixes between the dense pass and the whole corpus. Measured at 10M x 768, 1024 queries, k = 10 (whole call,
-    // ms; `profiles/r02_knn_tc_schedules.log`): n/256, n/32 14.8-15.3 | n/128, n/16 (round 1) 15.6-15.9 | n/32 only
-    // 15.0-15.4 | n/64 only 15.5 | n/128 only 16.8. Fewer / smaller prefixes cost less themselves but leave a looser
-    // threshold: the next pass appends more pairs, and every append drags its whole warp through the 32-column slow
-    // path (1.7 M pairs: +2.3 ms on the final pass).
-    // 0 (default): n/256, n/32 for k <= 32, n/128, n/16 above | 1: n/32 | 2: n/64, n/8 | 3: n/128 | 4: n/64 | 6: n/128, n/16
-    const bool fine = sched == 0 ? k <= 32 : false;
-    const size_t mids[2] = {sched == 1 ? 0 : (sched == 2 || sched == 4 ? v.n / 64 : (fine ? v.n / 256 : v.n / 128)),
-                            sched == 1 ? v.n / 32 : (sched == 2 ? v.n / 8 : (sched == 3 || sched == 4 ? 0 : (fine ? v.n / 32 : v.n / 16)))};
-    for (size_t nx : mids)
-      if (nx >= 4 * cur) {
-        cur = (nx + VT - 1) / VT * VT;
-        levels[n_levels++] = cur;
-      }
-    // a pass over `next` rows with the threshold of a `cur`-row sample appends about next / cur * k pairs per query:
-    // keep that under half of the list (CAND_CAP) with extra prefixes where the standard ones leave a larger step
-    // (small corpora, where n/256 and n/32 are below the 4 x rule)
-    const size_t g_safe = std::max<size_t>(4, (size_t)(CAND_CAP / 2) / k);
-    size_t extra[3];
-    int n_extra = 0;
-    for (size_t top = v.n; top / cur > g_safe && n_extra < 3;) {  // from the top down: the extra prefixes stay small
-      top = ((top + g_safe - 1) / g_safe + VT - 1) / VT * VT;
-      if (top <= cur) break;
-      extra[n_extra++] = top;
-    }
-    while (n_extra > 0 && n_levels < 5) {
-      cur = extra[--n_extra];
-      levels[n_levels++] = cur;
-    }
-    if (v.n > cur) levels[n_levels++] = v.n;
-  }
+  static const int sched = getenv("INNR_KNN_TC_SCHED") ? atoi(getenv("INNR_KNN_TC_SCHED")) : 0;
+  const int n_levels = tcf::levels(v.n, k, first_rows, sched, levels);
   KtArgs a{};
   a.n_qgroups = (p.nq_pad + QT - 1) / QT;
   a.kblocks = (p.d_pad + KB - 1) / KB;
@@ -808,8 +743,7 @@ cudaError_t launch_pdx_knn_tc(const PdxView& v, const CUtensorMap& tm_xh, const 
     if (last) {
       cudaEventRecord(ev[2], s);
     } else {
-      if (k <= 32) knn_tc_select_kernel<1><<<(unsigned)((nq + 3) / 4), 128, 0, s>>>((unsigned)nq, (unsigned)k, qflag, cnt, cand_lb, thr);
-      else knn_tc_select_kernel<4><<<(unsigned)((nq + 3) / 4), 128, 0, s>>>((unsigned)nq, (unsigned)k, qflag, cnt, cand_lb, thr);
+      tcf::launch_select(nq, k, qflag, cnt, cand_lb, thr, s);
       ++*launches;
       if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }

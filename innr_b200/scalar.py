@@ -210,6 +210,24 @@ def batch_knn_u8_many(queries, corpus: U8Corpus, k: int):
     return idx[:, :cnt.value], sc[:, :cnt.value]
 
 
+def u8_tc_debug_bounds(queries, corpus: U8Corpus):
+    """Test hook (include/innr_cuda.h: innr_cuda_u8_tc_debug_bounds): the u8 tensor-core filter's score interval for
+    every (query, row < min(N, 4096)) pair exactly as production computes it. Returns (lower[nq, rows], upper[nq, rows],
+    qflags[nq])."""
+    qs = np.ascontiguousarray(queries, dtype=np.float32)
+    if qs.ndim == 1:
+        qs = qs.reshape(1, -1)
+    nq, qlen = qs.shape
+    lower = np.zeros((nq, 4096), np.float32)
+    upper = np.zeros((nq, 4096), np.float32)
+    rows = C.c_size_t(0)
+    flags = np.zeros(nq, np.uint32)
+    L.call("innr_cuda_u8_tc_debug_bounds", corpus.h, qs.ctypes.data_as(L.f32p), nq, qlen, lower.ctypes.data_as(L.f32p),
+           upper.ctypes.data_as(L.f32p), C.byref(rows), flags.ctypes.data_as(L.u32p))
+    r = rows.value
+    return lower.reshape(-1)[:nq * r].reshape(nq, r), upper.reshape(-1)[:nq * r].reshape(nq, r), flags
+
+
 def batch_knn_u8(query, corpus, params: QuantizationParams, k: int):  # src/scalar.rs:370-393 -> Vec<(usize, f32)>
     if not isinstance(corpus, U8Corpus):
         if len(corpus) == 0 or k == 0:
