@@ -109,6 +109,15 @@ int innr_cuda_u8_tc_last_stats(float* out_filter_ms, float* out_total_ms, double
  * cannot take the filter (alpha / 255 not finite and positive, d > 8192). */
 int innr_cuda_u8_tc_debug_bounds(const innr_cuda_corpus* c, const float* queries, size_t n_queries, size_t query_len,
                                  float* out_lower, float* out_upper, size_t* out_rows, uint32_t* out_qflags);
+/* Statistics of the last binary top-k call that took the tensor-core filter (bin_tc.cu: Hamming, binary_dot and
+ * binary_jaccard query batches; options "bin_tc", "bin_tc_min_n", "bin_tc_min_queries", "bin_tc_max_k" of
+ * innr_cuda_set_option select it, results never depend on them): device time of the final filter passes and of the whole
+ * call (ms), integer operations those passes issued (2 x rows x padded bits x padded queries, summed over the batches of
+ * 1024 queries), candidate keys the final passes kept, queries whose final list overflowed (answered by the exact scan
+ * instead), filter passes. The filter never makes the host wait: the statistics stay on the device until this call, which
+ * waits for that filter call to finish. Any pointer may be NULL. */
+int innr_cuda_bin_tc_last_stats(float* out_filter_ms, float* out_total_ms, double* out_filter_ops,
+                                uint64_t* out_candidates, uint32_t* out_exact_scan_queries, int* out_passes);
 /* number of kernels the library has launched so far (bench.py's gpu_launches counter) */
 int innr_cuda_launch_count(uint64_t* out_count);
 
@@ -249,6 +258,17 @@ int innr_cuda_hamming_topk(const innr_cuda_corpus* c, const uint64_t* query_word
                            size_t* out_count);
 int innr_cuda_hamming_topk_keys_dev(const innr_cuda_corpus* c, const uint64_t* dev_query_words,
                                     size_t n_queries, size_t k, uint64_t* dev_keys, void* stream);
+/* innr_cuda_binary_topk for n_queries query codes (host, n_queries x ceil(dim/64) u64) in one call: the same indices,
+ * scores and order as n_queries calls of innr_cuda_binary_topk, rows at stride k (out_idx / out_score n_queries x k,
+ * *out_count = min(k, n) per row). Batches run on the tensor cores (bin_tc.cu) when they qualify. */
+int innr_cuda_binary_topk_batch(const innr_cuda_corpus* c, int op, const uint64_t* query_words, size_t n_queries,
+                                size_t query_dim_bits, size_t k, uint64_t* out_idx, float* out_score, size_t* out_count);
+/* Device-resident form of innr_cuda_binary_topk_batch: dev_query_words n_queries x 2 ceil(dim/128) u64 (zero padded to
+ * whole 128-bit chunks, padding bits masked), dev_keys n_queries x k keys (dot: (~count << 32) | index; Jaccard: the
+ * descending f32 key of the quotient), sentinel padded past n. Enqueued on `stream`; never makes the host wait.
+ * INNR_EUNSUPPORTED for zero-dimensional codes (use innr_cuda_binary_topk_batch). */
+int innr_cuda_binary_topk_keys_dev(const innr_cuda_corpus* c, int op, const uint64_t* dev_query_words, size_t n_queries,
+                                   size_t k, uint64_t* dev_keys, void* stream);
 /* encode_binary (src/binary.rs:133-141): bit i = values[i] > threshold; out_words ceil(n/64) u64 */
 int innr_cuda_encode_binary(const float* values, size_t n, float threshold, uint64_t* out_words);
 

@@ -474,6 +474,46 @@ impl BinaryCorpus {
         })?;
         Ok(idx.into_iter().zip(sc).take(count).map(|(i, s)| (i as usize, s)).collect())
     }
+
+    /// `hamming_top_k` for a batch of queries (`query_words`: `n_queries` codes back to back) in one call, one list per
+    /// query; batches run on the tensor cores when they qualify, with the same results.
+    pub fn hamming_top_k_many(&self, query_words: &[u64], n_queries: usize, query_dim_bits: usize, k: usize) -> Result<Vec<Vec<(usize, u32)>>> {
+        assert_eq!(query_dim_bits, self.dim_bits, "innr::binary_hamming: dimension mismatch ({query_dim_bits} vs {})", self.dim_bits);
+        let words = (self.dim_bits + 63) / 64;
+        assert_eq!(query_words.len(), n_queries * words);
+        if n_queries == 0 {
+            return Ok(Vec::new());
+        }
+        let kk = k.max(1);
+        let (mut idx, mut dist) = (vec![0u64; n_queries * kk], vec![0u32; n_queries * kk]);
+        let mut count = 0usize;
+        check(unsafe {
+            innr_cuda_hamming_topk(self.h.0, query_words.as_ptr(), n_queries, query_dim_bits, k, idx.as_mut_ptr(), dist.as_mut_ptr(), &mut count)
+        })?;
+        Ok((0..n_queries)
+            .map(|q| (0..count).map(|j| (idx[q * kk + j] as usize, dist[q * kk + j])).collect())
+            .collect())
+    }
+
+    /// `similarity_top_k` for a batch of queries (`query_words`: `n_queries` codes back to back) in one call, one list
+    /// per query, the same results as one call per query.
+    pub fn binary_top_k_many(&self, jaccard: bool, query_words: &[u64], n_queries: usize, query_dim_bits: usize, k: usize) -> Result<Vec<Vec<(usize, f32)>>> {
+        assert_eq!(query_dim_bits, self.dim_bits, "dimension mismatch ({query_dim_bits} vs {})", self.dim_bits);
+        let words = (self.dim_bits + 63) / 64;
+        assert_eq!(query_words.len(), n_queries * words);
+        if n_queries == 0 {
+            return Ok(Vec::new());
+        }
+        let kk = k.max(1);
+        let (mut idx, mut sc) = (vec![0u64; n_queries * kk], vec![0f32; n_queries * kk]);
+        let mut count = 0usize;
+        check(unsafe {
+            innr_cuda_binary_topk_batch(self.h.0, jaccard as c_int, query_words.as_ptr(), n_queries, query_dim_bits, k, idx.as_mut_ptr(), sc.as_mut_ptr(), &mut count)
+        })?;
+        Ok((0..n_queries)
+            .map(|q| (0..count).map(|j| (idx[q * kk + j] as usize, sc[q * kk + j])).collect())
+            .collect())
+    }
 }
 
 /// `encode_binary` (src/binary.rs:133-141): the words of the resulting `PackedBinary`.

@@ -15,7 +15,7 @@ from .batch import (BatchKnnResult, DeviceBatch, VerticalBatch, batch_cosine, ba
                     batch_l2_squared_into, batch_l2_squared_pruning, batch_norms, batch_norms_into, knn_tc_debug_bounds,
                     knn_screen_debug_bounds)
 from .binary import (BinaryCorpus, PackedBinary, binary_dot, binary_dot_all, binary_hamming, binary_jaccard,  # noqa: F401
-                     binary_jaccard_all, binary_topk, encode_binary, hamming_all,
+                     binary_jaccard_all, binary_topk, binary_topk_many, encode_binary, hamming_all,
                      hamming_topk, hamming_topk_many)
 from .maxsim import (TokenCorpus, maxsim, maxsim_corpus, maxsim_corpus_batch, maxsim_cosine, maxsim_topk,  # noqa: F401
                      maxsim_topk_batch)

@@ -41,6 +41,7 @@ SIGNATURES = {
     "innr_cuda_knn_tc_debug_bounds": [vp, ci, f32p, sz, sz, f32p, szp, f32p, u32p],
     "innr_cuda_knn_screen_debug_bounds": [vp, ci, f32p, sz, f32p, f32p],
     "innr_cuda_u8_tc_last_stats": [f32p, f32p, C.POINTER(C.c_double), u64p, C.POINTER(C.c_uint32), C.POINTER(ci)],
+    "innr_cuda_bin_tc_last_stats": [f32p, f32p, C.POINTER(C.c_double), u64p, C.POINTER(C.c_uint32), C.POINTER(ci)],
     "innr_cuda_u8_tc_debug_bounds": [vp, f32p, sz, sz, f32p, f32p, szp, u32p],
     "innr_cuda_launch_count": [u64p],
     "innr_cuda_last_kernel_ms": [f32p],
@@ -64,6 +65,8 @@ SIGNATURES = {
     "innr_cuda_batch_l2_squared_pruning": [vp, f32p, sz, f32, u64p, f32p, sz, szp],
     "innr_cuda_batch_knn_adaptive": [vp, f32p, sz, sz, sz, u64p, f32p, szp],
     "innr_cuda_binary_topk": [vp, ci, u64p, sz, sz, u64p, f32p, szp],
+    "innr_cuda_binary_topk_batch": [vp, ci, u64p, sz, sz, sz, u64p, f32p, szp],
+    "innr_cuda_binary_topk_keys_dev": [vp, ci, vp, sz, sz, vp, vp],
     "innr_cuda_batch_dimension_variance": [vp, f32p, sz],
     "innr_cuda_batch_knn_reordered": [vp, f32p, sz, sz, u64p, f32p, szp],
     "innr_cuda_batch_knn_keys_dev": [vp, ci, vp, sz, sz, vp, vp],
@@ -199,6 +202,15 @@ def u8_tc_last_stats() -> dict:
     """Statistics of the most recent batch_knn_u8 call that used the tensor-core filter (include/innr_cuda.h)."""
     f, t, ops, cand, ex, p = C.c_float(), C.c_float(), C.c_double(), C.c_uint64(), C.c_uint32(), C.c_int()
     call("innr_cuda_u8_tc_last_stats", C.byref(f), C.byref(t), C.byref(ops), C.byref(cand), C.byref(ex), C.byref(p))
+    return {"filter_ms": f.value, "total_ms": t.value, "filter_ops": ops.value, "candidates": cand.value,
+            "exact_scan_queries": ex.value, "passes": p.value}
+
+
+def bin_tc_last_stats() -> dict:
+    """Statistics of the most recent binary top-k call that used the tensor-core filter (include/innr_cuda.h). Waits for
+    that call to finish on the device."""
+    f, t, ops, cand, ex, p = C.c_float(), C.c_float(), C.c_double(), C.c_uint64(), C.c_uint32(), C.c_int()
+    call("innr_cuda_bin_tc_last_stats", C.byref(f), C.byref(t), C.byref(ops), C.byref(cand), C.byref(ex), C.byref(p))
     return {"filter_ms": f.value, "total_ms": t.value, "filter_ops": ops.value, "candidates": cand.value,
             "exact_scan_queries": ex.value, "passes": p.value}
 

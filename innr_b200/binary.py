@@ -136,6 +136,34 @@ def binary_topk(op: str, query: PackedBinary, corpus: BinaryCorpus, k: int):
     return idx[:cnt.value], sc[:cnt.value]
 
 
+def binary_topk_many(op: str, queries, corpus: BinaryCorpus, k: int):
+    """`binary_topk` for a batch of query codes in one call ((nq, words) uint64, or PackedBinary codes): the same
+    results as one `binary_topk` per query. Returns (indices uint64[nq, m], scores float32[nq, m]), m = min(k, n)."""
+    if len(queries) and isinstance(queries[0], PackedBinary):
+        queries = np.stack([np.asarray(q.data, dtype=np.uint64) for q in queries])
+    qs = np.ascontiguousarray(queries, dtype=np.uint64)
+    if qs.ndim == 1:
+        qs = qs.reshape(1, -1)
+    nq = qs.shape[0]
+    kk = max(k, 1)
+    idx = np.zeros((nq, kk), np.uint64)
+    sc = np.zeros((nq, kk), np.float32)
+    cnt = C.c_size_t(0)
+    L.call("innr_cuda_binary_topk_batch", corpus.h, {"dot": 0, "jaccard": 1}[op], qs.ctypes.data_as(L.u64p), nq,
+           corpus.dimension, k, idx.ctypes.data_as(L.u64p), sc.ctypes.data_as(L.f32p), C.byref(cnt))
+    return idx[:, :cnt.value], sc[:, :cnt.value]
+
+
+def binary_topk_keys_dev(op: str, dev_query_words, corpus: BinaryCorpus, k: int, dev_keys, stream=None):
+    """Device-resident batch: dev_query_words a CUDA uint64 tensor (nq, 2 * ceil(dim / 128)), zero padded; dev_keys a
+    CUDA int64 tensor (nq, k) receiving the keys (include/innr_cuda.h). Enqueued on `stream` (torch stream or None for
+    the current one); returns at once."""
+    import torch
+    s = stream if stream is not None else torch.cuda.current_stream(dev_query_words.device)
+    L.call("innr_cuda_binary_topk_keys_dev", corpus.h, {"dot": 0, "jaccard": 1}[op], C.c_void_p(dev_query_words.data_ptr()),
+           dev_query_words.shape[0], k, C.c_void_p(dev_keys.data_ptr()), C.c_void_p(s.cuda_stream))
+
+
 def binary_dot(a: PackedBinary, b: PackedBinary) -> int:  # src/binary.rs:178 (pairwise; 1-code corpus)
     assert a.dimension == b.dimension
     if a.dimension == 0:

@@ -46,9 +46,11 @@ struct innr_cuda_corpus {
   uint8_t* dev_sketch = nullptr;
   bool screen = false;
   // f32 PDX: lazily built operands of the tensor-core filter path (knn_tc.cu): exact norms, f16 unit vectors + TMA map;
-  // u8: the row radii of its filter path (u8_tc.cu, dev_radius)
+  // u8: the row radii of its filter path (u8_tc.cu, dev_radius); binary: the row popcounts of its filter path (bin_tc.cu,
+  // dev_popc)
   int tc_state = 0;  // 0 not built, 1 ready, -1 unusable (non-finite norms / no memory): exact scan only
   float* dev_radius = nullptr;
+  uint32_t* dev_popc = nullptr;
   float* dev_norms = nullptr;
   void* dev_xh = nullptr;
   CUtensorMap tm_xh;
@@ -154,6 +156,9 @@ struct DeviceCtx {
   unsigned async_next = 0;
   Buf d_query, d_keys, d_scores, d_aux, d_tcws, h_pin, h_counts;
   float last_ms = 0.0f;
+  // the binary filter's statistics stay on the device until innr_cuda_bin_tc_last_stats asks (bin_tc.cu: launch_bin_tc)
+  BinTcDevStats* bt_stats = nullptr;
+  std::vector<cudaEvent_t> bt_ev;
 };
 
 struct Options {
@@ -169,6 +174,13 @@ struct Options {
   size_t u8_tc_min_n = 100000;
   size_t u8_tc_min_queries = 8;
   size_t u8_tc_max_k = 32;
+  bool bin_tc = true;
+  // measured at C4 (100M x 1024 bit, DESIGN.md section 3.11): a filter call costs ~15 ms up to 64 queries; the CUDA-core
+  // route takes 12.6 ms for 16 queries and 25.2 ms for 32 at k = 10 (k = 100: 10.4 ms for 8, 20.8 ms for 16), so batches
+  // start at 32 queries. Every k <= 128 measured faster from 32 queries on.
+  size_t bin_tc_min_n = 100000;
+  size_t bin_tc_min_queries = 32;
+  size_t bin_tc_max_k = 128;
   bool kernel_timing = false;
 } g_opt;
 
@@ -180,6 +192,11 @@ DeviceCtx g_ctx[MAX_DEVICES];
 LaunchCounter g_launches{0};
 KnnTcStats g_tc_stats;
 KnnTcStats g_u8tc_stats;  // the last u8 filter call (kept apart: knn_tc_last_stats reports f32 calls only)
+// the last binary filter call: its device, what the host knew at launch and how many query chunks it had (the rest of its
+// statistics is read from the device's bt_stats / bt_ev when asked)
+int g_bintc_device = -1;
+BinTcCall g_bintc_call;
+size_t g_bintc_chunks = 0;
 thread_local int t_device = -1;
 thread_local std::string t_err;
 std::mutex& dev_mu(int d) { return g_dev_mu[(d >= 0 && d < MAX_DEVICES) ? d : 0]; }
@@ -374,6 +391,7 @@ void destroy_corpus(innr_cuda_corpus* c) {
   if (c->dev_sketch) cudaFree(c->dev_sketch);
   if (c->dev_xh) cudaFree(c->dev_xh);
   if (c->dev_radius) cudaFree(c->dev_radius);
+  if (c->dev_popc) cudaFree(c->dev_popc);
   if (c->dev_order) cudaFree(c->dev_order);
   delete c;
 }
@@ -468,6 +486,8 @@ int innr_cuda_shutdown(void) {
     cudaEventDestroy(c.ev0);
     cudaEventDestroy(c.ev1);
     for (int l = 0; l < 2; ++l) cudaEventDestroy(c.ws_event[l]);
+    for (cudaEvent_t e : c.bt_ev) cudaEventDestroy(e);
+    if (c.bt_stats) cudaFree(c.bt_stats);
     for (innr_cuda_ticket& t : c.async_slot) {
       if (t.stream) cudaStreamSynchronize(t.stream);
       if (t.d_query) cudaFree(t.d_query);
@@ -506,6 +526,10 @@ int innr_cuda_set_option(const char* name, double value) {
   else if (n == "u8_tc_min_n") g_opt.u8_tc_min_n = (size_t)value;
   else if (n == "u8_tc_min_queries") g_opt.u8_tc_min_queries = (size_t)value;
   else if (n == "u8_tc_max_k") g_opt.u8_tc_max_k = (size_t)value;
+  else if (n == "bin_tc") g_opt.bin_tc = value != 0;
+  else if (n == "bin_tc_min_n") g_opt.bin_tc_min_n = (size_t)value;
+  else if (n == "bin_tc_min_queries") g_opt.bin_tc_min_queries = (size_t)value;
+  else if (n == "bin_tc_max_k") g_opt.bin_tc_max_k = (size_t)value;
   else if (n == "kernel_timing") g_opt.kernel_timing = value != 0;
   else if (n == "u8_scaled_chains") u8_set_scaled_chains(value != 0);
   else return fail(INNR_EINVAL, "unknown option: " + n);
@@ -531,6 +555,40 @@ int innr_cuda_u8_tc_last_stats(float* out_filter_ms, float* out_total_ms, double
   if (out_candidates) *out_candidates = g_u8tc_stats.candidates;
   if (out_exact_scan_queries) *out_exact_scan_queries = g_u8tc_stats.overflowed;
   if (out_passes) *out_passes = g_u8tc_stats.passes;
+  return INNR_OK;
+}
+int innr_cuda_bin_tc_last_stats(float* out_filter_ms, float* out_total_ms, double* out_filter_ops,
+                                uint64_t* out_candidates, uint32_t* out_exact_scan_queries, int* out_passes) {
+  int device;
+  BinTcCall call;
+  size_t chunks;
+  {
+    std::lock_guard<std::mutex> lk(g_mu);
+    device = g_bintc_device;
+    call = g_bintc_call;
+    chunks = g_bintc_chunks;
+  }
+  float filter_ms = 0.0f, total_ms = 0.0f;
+  BinTcDevStats ds{};
+  if (device >= 0) {  // waits for that call (and only for it) to finish on the device
+    EntryGuard lk(device);
+    DeviceCtx& c = g_ctx[device];
+    CU(cudaSetDevice(device));
+    CU(cudaEventSynchronize(c.bt_ev[1]));
+    CU(cudaEventElapsedTime(&total_ms, c.bt_ev[0], c.bt_ev[1]));
+    for (size_t i = 0; i < chunks; ++i) {
+      float ms = 0.0f;
+      CU(cudaEventElapsedTime(&ms, c.bt_ev[2 + 2 * i], c.bt_ev[3 + 2 * i]));
+      filter_ms += ms;
+    }
+    CU(cudaMemcpy(&ds, c.bt_stats, sizeof(ds), cudaMemcpyDeviceToHost));
+  }
+  if (out_filter_ms) *out_filter_ms = filter_ms;
+  if (out_total_ms) *out_total_ms = total_ms;
+  if (out_filter_ops) *out_filter_ops = call.filter_ops;
+  if (out_candidates) *out_candidates = ds.candidates;
+  if (out_exact_scan_queries) *out_exact_scan_queries = ds.overflowed;
+  if (out_passes) *out_passes = call.passes;
   return INNR_OK;
 }
 int innr_cuda_launch_count(uint64_t* out_count) {
@@ -1654,6 +1712,94 @@ int innr_cuda_binary_jaccard_all(const innr_cuda_corpus* c, const uint64_t* quer
   return binary_setop_all(c, query_words, query_dim_bits, true, out_host);
 }
 
+// Query batches go through the tensor-core filter (bin_tc.cu: the exact keys, see there) when the corpus qualifies;
+// innr_cuda_set_option("bin_tc", 0) disables it. Single queries always take the scan.
+static bool bin_takes_tc_filter(const innr_cuda_corpus* c, size_t nq, size_t k) {
+  return g_opt.bin_tc && c->n >= g_opt.bin_tc_min_n && nq >= g_opt.bin_tc_min_queries && nq >= 2 && k <= g_opt.bin_tc_max_k &&
+         bin_tc_supported(bin_view(c), nq, k);
+}
+// the Hamming scans need a Workspace and nothing else: either lane will do
+static bool hamming_is_scan_only(const innr_cuda_corpus* c, size_t nq, size_t k) {
+  return k <= MAX_FUSED_K && !bin_takes_tc_filter(c, nq, k);
+}
+static bool setops_fused(const innr_cuda_corpus* c, size_t k) {
+  return k <= MAX_FUSED_K && c->chunks * sizeof(uint4) + 8 * k * sizeof(uint64_t) <= 48 * 1024;
+}
+static bool setops_is_scan_only(const innr_cuda_corpus* c, size_t nq, size_t k) {
+  return setops_fused(c, k) && !bin_takes_tc_filter(c, nq, k);
+}
+// The row popcounts of the filter path, built on first use (the handle stays immutable: a cache of the same data). On
+// failure (no memory) the corpus stays on the CUDA-core scans.
+static int bin_tc_prepare(innr_cuda_corpus* c, cudaStream_t s) {
+  if (c->tc_state != 0) return INNR_OK;
+  c->tc_state = -1;
+  if (cudaMalloc(&c->dev_popc, c->n * sizeof(uint32_t)) != cudaSuccess) {
+    cudaGetLastError();  // out of memory is not an error of the call: the scans answer
+    c->dev_popc = nullptr;
+    return INNR_OK;
+  }
+  CU(launch_bin_tc_popc(bin_view(c), c->dev_popc, s, &g_launches));
+  c->tc_state = 1;
+  return INNR_OK;
+}
+// op 0 Hamming, 1 binary_dot, 2 binary_jaccard; *taken = false when the corpus cannot take the filter (no memory). Lane 0:
+// the filter's scratch. Enqueues only: the statistics stay on the device.
+static int bin_tc_keys(const innr_cuda_corpus* c, DeviceCtx* ctx, int op, const uint64_t* dev_query_words, size_t nq, size_t k,
+                       uint64_t* dev_keys, cudaStream_t s, bool* taken) {
+  *taken = false;
+  int rc = bin_tc_prepare(const_cast<innr_cuda_corpus*>(c), s);
+  if (rc) return rc;
+  if (c->tc_state != 1) return INNR_OK;
+  CU(ctx->d_tcws.reserve(bin_tc_workspace_bytes(c->chunks, nq, k)));
+  if (!ctx->bt_stats) CU(cudaMalloc((void**)&ctx->bt_stats, sizeof(BinTcDevStats)));
+  const size_t chunks = (nq + BIN_TC_CHUNK_QUERIES - 1) / BIN_TC_CHUNK_QUERIES;
+  while (ctx->bt_ev.size() < 2 + 2 * chunks) {
+    cudaEvent_t e;
+    CU(cudaEventCreate(&e));
+    ctx->bt_ev.push_back(e);
+  }
+  BinTcCall call;
+  CU(launch_bin_tc(bin_view(c), op, c->dev_popc, dev_query_words, nq, k, dev_keys, ctx->d_tcws.p, ctx->bt_stats,
+                   ctx->bt_ev.data(), ctx->ws.num_sms, s, &g_launches, &call));
+  {
+    std::lock_guard<std::mutex> lg(g_mu);
+    g_bintc_device = ctx->device;
+    g_bintc_call = call;
+    g_bintc_chunks = chunks;
+  }
+  *taken = true;
+  return INNR_OK;
+}
+// binary_dot (op 0) / binary_jaccard (op 1) keys of nq queries, rows of k keys (sentinel padded past n): the filter for
+// batches that qualify, else the single-query route once per query
+static int setop_keys(const innr_cuda_corpus* c, DeviceCtx* ctx, int op, const uint64_t* dev_query_words, size_t nq, size_t k,
+                      uint64_t* dev_keys, cudaStream_t s, int lane = 0) {
+  if (bin_takes_tc_filter(c, nq, k)) {
+    bool taken;
+    int rc = bin_tc_keys(c, ctx, 1 + op, dev_query_words, nq, k, dev_keys, s, &taken);
+    if (rc || taken) return rc;
+  }
+  const size_t qw = 2 * c->chunks;
+  if (setops_fused(c, k)) {
+    for (size_t q = 0; q < nq; ++q)
+      CU(launch_binary_setops_topk(bin_view(c), op, dev_query_words + q * qw, k, dev_keys + q * k, ctx->lane_ws(lane), s,
+                                   &g_launches));
+    return INNR_OK;
+  }
+  const size_t kk = k < c->n ? k : c->n;
+  if (kk < k) CU(cudaMemsetAsync(dev_keys, 0xFF, nq * k * sizeof(uint64_t), s));
+  CU(ctx->d_scores.reserve(c->n * sizeof(uint32_t)));
+  for (size_t q = 0; q < nq; ++q) {
+    if (op)
+      CU(launch_binary_jaccard_all(bin_view(c), dev_query_words + q * qw, (float*)ctx->d_scores.p, s, &g_launches));
+    else
+      CU(launch_binary_dot_all(bin_view(c), dev_query_words + q * qw, (uint32_t*)ctx->d_scores.p, s, &g_launches));
+    CU(launch_topk_from_scores(ctx->d_scores.p, op ? 1 : 4, c->n, (uint32_t)c->index_base, kk, dev_keys + q * k, ctx->ws, s,
+                               &g_launches));
+  }
+  return INNR_OK;
+}
+
 // Top-k by binary_dot (op 0) or binary_jaccard (op 1) over a code set: the caller composition the reference shows for
 // Hamming (examples/binary_demo.rs:174-180) with the similarity ranked descending, ties -> lower index. Scores as f32
 // (dot counts are exact: dimension < 2^24).
@@ -1712,6 +1858,11 @@ int innr_cuda_binary_topk(const innr_cuda_corpus* c, int op, const uint64_t* que
 
 static int hamming_keys(const innr_cuda_corpus* c, DeviceCtx* ctx, const uint64_t* dev_query_words, size_t nq, size_t k,
                         uint64_t* dev_keys, cudaStream_t s, int lane = 0) {
+  if (bin_takes_tc_filter(c, nq, k)) {
+    bool taken;
+    int rc = bin_tc_keys(c, ctx, 0, dev_query_words, nq, k, dev_keys, s, &taken);
+    if (rc || taken) return rc;
+  }
   if (k <= MAX_FUSED_K) {
     CU(launch_hamming_topk(bin_view(c), dev_query_words, nq, k, dev_keys, ctx->lane_ws(lane), s, &g_launches));
     return INNR_OK;
@@ -1776,7 +1927,7 @@ int innr_cuda_hamming_topk_keys_dev(const innr_cuda_corpus* c, const uint64_t* d
   cudaStream_t s = (cudaStream_t)stream;
   DeviceCtx* ctx;
   int lane = 0;
-  int rc = ctx_for_dev(c, &ctx, s, k <= MAX_FUSED_K, &lane);
+  int rc = ctx_for_dev(c, &ctx, s, hamming_is_scan_only(c, n_queries, k), &lane);
   if (rc) return rc;
   DevRelease rel(*ctx, s, lane);
   if (c->n == 0 || c->words == 0) {
@@ -1784,6 +1935,76 @@ int innr_cuda_hamming_topk_keys_dev(const innr_cuda_corpus* c, const uint64_t* d
     return INNR_OK;
   }
   return hamming_keys(c, ctx, dev_query_words, n_queries, k, dev_keys, s, lane);
+}
+
+// n_queries calls of innr_cuda_binary_topk in one: query batches take the tensor-core filter (bin_tc.cu) when they qualify
+int innr_cuda_binary_topk_batch(const innr_cuda_corpus* c, int op, const uint64_t* query_words, size_t n_queries,
+                                size_t query_dim_bits, size_t k, uint64_t* out_idx, float* out_score, size_t* out_count) {
+  if (!c || c->kind != 1) return fail(INNR_EINVAL, "need a binary corpus");
+  if (op != 0 && op != 1) return fail(INNR_EINVAL, "binary_topk: op must be 0 (dot) or 1 (jaccard)");
+  if (query_dim_bits != c->dim_bits) return fail(INNR_EINVAL, "dimension mismatch");  // assert_eq!(a.dimension, b.dimension)
+  if (out_count) *out_count = 0;
+  if (c->n == 0 || k == 0 || n_queries == 0) return INNR_OK;
+  if (!out_idx || !out_score || (!query_words && c->words)) return fail(INNR_EINVAL, "null argument");
+  if (c->dim_bits >= (1u << 24)) return fail(INNR_EUNSUPPORTED, "binary_topk: dimension >= 2^24");
+  const size_t kk = k < c->n ? k : c->n;
+  if (c->words == 0) {  // no words: dot 0 / jaccard 1.0 for every code, index order
+    for (size_t q = 0; q < n_queries; ++q)
+      for (size_t j = 0; j < kk; ++j) {
+        out_idx[q * k + j] = c->index_base + j;
+        out_score[q * k + j] = op ? 1.0f : 0.0f;
+      }
+    if (out_count) *out_count = kk;
+    return INNR_OK;
+  }
+  EntryGuard lk(c->device);
+  DeviceCtx* ctx;
+  int rc = ctx_for(c, &ctx);
+  if (rc) return rc;
+  rc = stage_binary_queries(*ctx, c, query_words, n_queries);
+  if (rc) return rc;
+  CU(ctx->d_keys.reserve(n_queries * kk * sizeof(uint64_t)));
+  Timed tm(*ctx);
+  rc = setop_keys(c, ctx, op, (const uint64_t*)ctx->d_query.p, n_queries, kk, (uint64_t*)ctx->d_keys.p, ctx->stream);
+  if (rc) return rc;
+  tm.stop();
+  rc = fetch_keys(*ctx, n_queries, kk, tm, [&](const uint64_t* keys) {
+    for (size_t q = 0; q < n_queries; ++q) {
+      const uint64_t* kq = keys + q * kk;
+      if (op) {
+        decode_keys_f32(kq, kk, true, out_idx + q * k, out_score + q * k);
+      } else {
+        for (size_t j = 0; j < kk; ++j) {
+          out_idx[q * k + j] = kq[j] & 0xFFFFFFFFull;
+          out_score[q * k + j] = (float)(~(uint32_t)(kq[j] >> 32));
+        }
+      }
+    }
+  });
+  if (rc) return rc;
+  if (out_count) *out_count = kk;
+  return INNR_OK;
+}
+
+int innr_cuda_binary_topk_keys_dev(const innr_cuda_corpus* c, int op, const uint64_t* dev_query_words, size_t n_queries,
+                                   size_t k, uint64_t* dev_keys, void* stream) {
+  if (!c || c->kind != 1) return fail(INNR_EINVAL, "need a binary corpus");
+  if (op != 0 && op != 1) return fail(INNR_EINVAL, "binary_topk: op must be 0 (dot) or 1 (jaccard)");
+  if (k == 0 || n_queries == 0) return INNR_OK;
+  if (c->n > 0 && c->words == 0) return fail(INNR_EUNSUPPORTED, "zero-dimensional codes: use innr_cuda_binary_topk_batch");
+  if (c->dim_bits >= (1u << 24)) return fail(INNR_EUNSUPPORTED, "binary_topk: dimension >= 2^24");
+  EntryGuard lk(c->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  DeviceCtx* ctx;
+  int lane = 0;
+  int rc = ctx_for_dev(c, &ctx, s, setops_is_scan_only(c, n_queries, k), &lane);
+  if (rc) return rc;
+  DevRelease rel(*ctx, s, lane);
+  if (c->n == 0) {
+    CU(cudaMemsetAsync(dev_keys, 0xFF, n_queries * k * sizeof(uint64_t), s));
+    return INNR_OK;
+  }
+  return setop_keys(c, ctx, op, dev_query_words, n_queries, k, dev_keys, s, lane);
 }
 
 int innr_cuda_encode_binary(const float* values, size_t n, float threshold, uint64_t* out_words) {
@@ -2654,7 +2875,7 @@ int innr_cuda_hamming_topk_async(const innr_cuda_corpus* c, const uint64_t* quer
       }
     CU(cudaMemcpyAsync(t->d_query, t->h_in, qbytes, cudaMemcpyHostToDevice, t->stream));
     int lane = 0;
-    rc = ensure_ctx(c->device, &ctx, kk <= MAX_FUSED_K ? WS_DEV_SCAN : WS_DEV, t->stream, &lane);
+    rc = ensure_ctx(c->device, &ctx, hamming_is_scan_only(c, n_queries, kk) ? WS_DEV_SCAN : WS_DEV, t->stream, &lane);
     if (rc) return rc;
     DevRelease rel(*ctx, t->stream, lane);
     rc = hamming_keys(c, ctx, (const uint64_t*)t->d_query, n_queries, kk, (uint64_t*)t->d_keys, t->stream, lane);
@@ -3623,7 +3844,7 @@ int innr_cuda_hamming_topk_sharded_async(const innr_cuda_corpus* const* shards, 
     }
   return sharded_async_via_exchange(
       g, shards, n_shards, padded.data(), padded.size() * sizeof(uint64_t), n_queries, k, k < n_total ? k : n_total,
-      INNR_METRIC_L2, [&](size_t) { return true; },
+      INNR_METRIC_L2, [&](size_t i) { return shards[i]->n == 0 || hamming_is_scan_only(shards[i], n_queries, k); },
       [&](size_t i, DeviceCtx* ctx, void* dq, uint64_t* dk, cudaStream_t s, int lane) -> int {
         const innr_cuda_corpus* c = shards[i];
         if (c->n == 0) {

@@ -579,4 +579,93 @@ cudaError_t launch_hamming_topk(const BinView& v, const uint64_t* dev_query_word
   return cudaSuccess;
 }
 
+namespace {
+// Queries the tensor-core filter (bin_tc.cu) flagged on the device: grid (FLAGGED_CTAS, nq), CTA (x, q) returns at once
+// unless counts[q] > cap. Otherwise the FLAGGED_CTAS CTAs of query q split the rows, each merges its warps' lists into
+// partials[q][x], and the last of them to finish (ticket tickets[q], zero on entry, reset on exit) merges the
+// FLAGGED_CTAS lists into out_keys[q]. The keys are those of the single-query kernels above.
+template <int OP, int R>
+__global__ void __launch_bounds__(HAM_THREADS) binary_flagged_topk_kernel(const HamArgs a, const unsigned* __restrict__ counts,
+                                                                          unsigned cap) {
+  const unsigned q = blockIdx.y;
+  if (counts[q] <= cap) return;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  uint4* sq = reinterpret_cast<uint4*>(smem_raw);
+  uint64_t* smem_keys = reinterpret_cast<uint64_t*>(sq + a.chunks);
+  __shared__ unsigned s_last;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+  const uint64_t* qw = a.query_words + (size_t)q * 2 * a.chunks;
+  for (unsigned c = threadIdx.x; c < a.chunks; c += blockDim.x) {
+    const uint64_t w0 = qw[2 * c], w1 = qw[2 * c + 1];
+    sq[c] = make_uint4((unsigned)w0, (unsigned)(w0 >> 32), (unsigned)w1, (unsigned)(w1 >> 32));
+  }
+  __syncthreads();
+  WarpList<R> list;
+  list.init();
+  uint64_t thr = KEY_SENTINEL;
+  for (unsigned tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
+    const unsigned i = tile * HAM_THREADS + threadIdx.x;
+    const bool valid = i < a.n;
+    uint64_t key = KEY_SENTINEL;
+    if (valid) {
+      if (OP == 0) {
+        key = make_key_u32(code_distance<0>(a.data + i, a.ld, a.chunks, sq), a.index_base + i);
+      } else {
+        unsigned inter, uni;
+        setop_counts<OP == 2>(a, a.data + i, sq, inter, uni);
+        if (OP == 2) key = make_key_desc(uni == 0 ? 1.0f : __fdiv_rn(__uint2float_rn(inter), __uint2float_rn(uni)), a.index_base + i);
+        else key = make_key_u32(~inter, a.index_base + i);
+      }
+    }
+    list.offer(key, valid, thr, a.k, lane);
+  }
+  block_tree_merge<R>(list, a.k, smem_keys);
+  uint64_t* mine = a.partials + ((size_t)q * gridDim.x + blockIdx.x) * a.k;
+  if (warp == 0) list.store(mine, a.k, lane);
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = (atomicAdd(&a.tickets[q], 1u) == gridDim.x - 1) ? 1u : 0u;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  WarpList<R> acc;
+  acc.init();
+  warp_merge_lists<R, true>(acc, a.partials + (size_t)q * gridDim.x * a.k, warp, n_warps, (int)gridDim.x, (size_t)a.k, a.k,
+                            lane);
+  block_tree_merge<R>(acc, a.k, smem_keys);
+  if (warp == 0) acc.store(a.out_keys + (size_t)q * a.k, a.k, lane);
+  if (threadIdx.x == 0) a.tickets[q] = 0u;
+}
+
+template <int OP, int R>
+cudaError_t launch_flagged(const HamArgs& a, size_t nq, const unsigned* counts, unsigned cap, size_t smem, cudaStream_t s) {
+  binary_flagged_topk_kernel<OP, R><<<dim3(BIN_FLAGGED_CTAS, (unsigned)nq), HAM_THREADS, smem, s>>>(a, counts, cap);
+  return cudaGetLastError();
+}
+template <int R>
+cudaError_t launch_flagged_op(int op, const HamArgs& a, size_t nq, const unsigned* counts, unsigned cap, size_t smem,
+                              cudaStream_t s) {
+  if (op == 0) return launch_flagged<0, R>(a, nq, counts, cap, smem, s);
+  if (op == 1) return launch_flagged<1, R>(a, nq, counts, cap, smem, s);
+  return launch_flagged<2, R>(a, nq, counts, cap, smem, s);
+}
+}  // namespace
+
+cudaError_t launch_binary_flagged_topk(const BinView& v, int op, const uint64_t* dev_query_words, size_t nq, size_t k,
+                                       const unsigned* dev_counts, unsigned cap, uint64_t* partials, unsigned* tickets,
+                                       uint64_t* dev_keys, cudaStream_t s, LaunchCounter* launches) {
+  if (v.n == 0 || nq == 0 || k == 0 || k > 128 || op < 0 || op > 2) return cudaErrorInvalidValue;
+  HamArgs a = make_args(v, dev_query_words);
+  a.k = (int)k;
+  a.partials = partials;
+  a.tickets = tickets;
+  a.out_keys = dev_keys;
+  const size_t smem = v.chunks * sizeof(uint4) + (size_t)(HAM_THREADS / 32) * k * sizeof(uint64_t);
+  if (smem > 48 * 1024) return cudaErrorInvalidValue;
+  const cudaError_t e = k <= 32 ? launch_flagged_op<1>(op, a, nq, dev_counts, cap, smem, s)
+                                : launch_flagged_op<4>(op, a, nq, dev_counts, cap, smem, s);
+  if (e == cudaSuccess) ++*launches;
+  return e;
+}
+
 }  // namespace innr

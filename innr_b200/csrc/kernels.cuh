@@ -235,6 +235,38 @@ cudaError_t launch_binary_setops_topk(const BinView& v, int jaccard, const uint6
                                       Workspace& ws, cudaStream_t s, LaunchCounter* launches);
 cudaError_t launch_hamming_topk(const BinView& v, const uint64_t* dev_query_words, size_t nq, size_t k,
                                 uint64_t* dev_keys, Workspace& ws, cudaStream_t s, LaunchCounter* launches);
+// Exact top-k of the queries a device-side count flags (counts[q] > cap), on the CUDA cores: op 0 Hamming, 1 binary_dot,
+// 2 binary_jaccard, the keys of the kernels above, rows of k keys at dev_keys + q * k (other rows untouched). The grid
+// (BIN_FLAGGED_CTAS x nq CTAs) does not depend on the counts; a CTA whose query is not flagged returns at once.
+// partials: nq * BIN_FLAGGED_CTAS * k keys; tickets: nq counters, zero on entry and left zero.
+constexpr unsigned BIN_FLAGGED_CTAS = 16;
+cudaError_t launch_binary_flagged_topk(const BinView& v, int op, const uint64_t* dev_query_words, size_t nq, size_t k,
+                                       const unsigned* dev_counts, unsigned cap, uint64_t* partials, unsigned* tickets,
+                                       uint64_t* dev_keys, cudaStream_t s, LaunchCounter* launches);
+// tensor-core filter for binary query batches (bin_tc.cu): exact keys from integer MMAs over unpacked bits, k <= 128.
+// op 0 Hamming, 1 binary_dot, 2 binary_jaccard. Never synchronises the host: overflowed queries are flagged on the device
+// and answered by launch_binary_flagged_topk in the same stream.
+constexpr size_t BIN_TC_MAX_DIM_BITS = 8192;
+bool bin_tc_supported(const BinView& v, size_t nq, size_t k);
+size_t bin_tc_workspace_bytes(size_t chunks, size_t nq, size_t k);
+// once per corpus: dev_popc[i] = popcount of code i (n u32)
+cudaError_t launch_bin_tc_popc(const BinView& v, uint32_t* dev_popc, cudaStream_t s, LaunchCounter* launches);
+// statistics kept on the device (bin_tc_last_stats copies them when asked): final-pass candidates, overflowed queries
+struct BinTcDevStats {
+  unsigned long long candidates;
+  unsigned overflowed;
+  unsigned pad;
+};
+struct BinTcCall {  // what the host knows of the last call once it is enqueued
+  double filter_ops = 0;
+  int passes = 0;
+};
+// ev (null: not timed): [0] call begin, [1] call end, then one (final-pass begin, end) pair per chunk of
+// BIN_TC_CHUNK_QUERIES queries. dev_stats is zeroed by the call.
+constexpr size_t BIN_TC_CHUNK_QUERIES = 1024;
+cudaError_t launch_bin_tc(const BinView& v, int op, const uint32_t* dev_popc, const uint64_t* dev_query_words, size_t nq,
+                          size_t k, uint64_t* dev_keys, void* workspace, BinTcDevStats* dev_stats, cudaEvent_t* ev, int num_sms,
+                          cudaStream_t s, LaunchCounter* launches, BinTcCall* call);
 cudaError_t launch_encode_binary(const float* dev_values, size_t n, float threshold, uint64_t* dev_words,
                                  cudaStream_t s, LaunchCounter* launches);
 cudaError_t launch_binary_from_pdx(const PdxView& v, float threshold,

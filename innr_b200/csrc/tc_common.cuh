@@ -164,6 +164,37 @@ __device__ __forceinline__ bool elect_one_sync() {
 __device__ __forceinline__ uint64_t desc_advance(uint64_t desc, uint32_t bytes) { return desc + (uint64_t)(bytes >> 4); }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
+// ---- integer MMAs on K-major byte operands (u8_tc.cu, bin_tc.cu) ----------------------------------------------------
+// one contiguous global -> shared bulk copy (no tensor map), completion on an mbarrier (complete_tx::bytes)
+__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gsrc, unsigned bytes, uint64_t* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(smem_u32(bar))
+               : "memory");
+}
+template <bool ACC>
+__device__ __forceinline__ void umma_i8_c(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "n"(ACC ? 1 : 0)
+      : "memory");
+}
+// kind::i8: D = S32 (c_format 2), A = UINT8 (a_format 0), B = INT8 (b_format 1), both K-major
+__device__ __forceinline__ uint32_t make_idesc_u8s8(int M, int N) {
+  return (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+// K-major operand without swizzle: 8-row x 16-byte core matrices (128 contiguous bytes); SBO = byte stride between
+// core matrices along M / N (8 rows), LBO = byte stride between them along K (one chunk to the next)
+__device__ __forceinline__ uint64_t make_smem_desc_kmajor_noswizzle(uint32_t smem_addr, uint32_t lbo, uint32_t sbo) {
+  uint64_t d = 0;
+  d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
+  d |= (uint64_t)((lbo >> 4) & 0x3FFF) << 16;
+  d |= (uint64_t)((sbo >> 4) & 0x3FFF) << 32;
+  d |= (uint64_t)1 << 46;  // version; layout type 0 = SWIZZLE_NONE
+  return d;
+}
+
 // ---- descriptors ----------------------------------------------------------------------------------------------------
 // K-major operand panel stored as [rows][128 bytes] with the 128-byte swizzle (what TMA SWIZZLE_128B writes):
 // canonical layout ((8,n),2):((8,SBO),1) in 16-byte units -> SBO = 8 rows * 128 B = 1024 B, LBO unused (1).

@@ -1,6 +1,6 @@
 // tc_filter.cuh -- the parts of the exact-result tensor-core filters that do not depend on the corpus encoding, shared by
-// the f32 path (knn_tc.cu) and the u8 path (u8_tc.cu): the candidate list capacity, the prefix schedule of the filter
-// passes and the selection of the next pass's threshold.
+// the f32 path (knn_tc.cu), the u8 path (u8_tc.cu) and the binary path (bin_tc.cu): the candidate list capacity, the
+// prefix schedule of the filter passes and the selection of the next pass's threshold.
 //
 // A pass over rows [0, n_i) appends (row, lower bound) of every pair whose UPPER bound reaches the query's threshold; the
 // k-th largest LOWER bound of the appended pairs is a valid lower bound of the reference's k-th best score and becomes the
@@ -105,6 +105,38 @@ inline void launch_select(size_t nq, size_t k, const unsigned* qflag, unsigned* 
                           cudaStream_t s) {
   if (k <= 32) select_kernel<1><<<(unsigned)((nq + 3) / 4), 128, 0, s>>>((unsigned)nq, (unsigned)k, qflag, cnt, cand_lb, thr);
   else select_kernel<4><<<(unsigned)((nq + 3) / 4), 128, 0, s>>>((unsigned)nq, (unsigned)k, qflag, cnt, cand_lb, thr);
+}
+
+// ---- the same step for filters that append exact keys (bin_tc.cu): the next threshold is the k-th smallest stored KEY ---
+// An overflowed list still gives a valid threshold: any k stored keys belong to real rows. KEY_SENTINEL when fewer than k
+// keys are stored (the next pass then keeps every pair).
+template <int R>
+__global__ void select_keys_kernel(unsigned nq, unsigned k, unsigned* __restrict__ cand_count,
+                                   const uint64_t* __restrict__ cand_key, uint64_t* __restrict__ thr_key) {
+  const unsigned q = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (q >= nq) return;
+  unsigned cnt = cand_count[q];
+  if (cnt > CAND_CAP) cnt = CAND_CAP;
+  WarpList<R> list;
+  list.init();
+  uint64_t t = KEY_SENTINEL;
+  for (unsigned c0 = 0; c0 < cnt; c0 += 32) {
+    const unsigned c = c0 + lane;
+    const bool valid = c < cnt;
+    list.offer(valid ? cand_key[(size_t)q * CAND_CAP + c] : KEY_SENTINEL, valid, t, (int)k, lane);
+  }
+  const uint64_t kth = list.at((int)k - 1);
+  if (lane == 0) {
+    thr_key[q] = kth;
+    cand_count[q] = 0;
+  }
+}
+
+inline void launch_select_keys(size_t nq, size_t k, unsigned* cnt, const uint64_t* cand_key, uint64_t* thr_key,
+                               cudaStream_t s) {
+  if (k <= 32) select_keys_kernel<1><<<(unsigned)((nq + 3) / 4), 128, 0, s>>>((unsigned)nq, (unsigned)k, cnt, cand_key, thr_key);
+  else select_keys_kernel<4><<<(unsigned)((nq + 3) / 4), 128, 0, s>>>((unsigned)nq, (unsigned)k, cnt, cand_key, thr_key);
 }
 
 }  // namespace
