@@ -16,9 +16,19 @@ threads and 228 KB of shared memory per SM, 148 SMs):
   u8_scan_pair_kernel    288 threads, 164-167 registers, 192 KB ring  -> 1 CTA / SM                    -> <=  148 CTAs
   pdx_screen_kernel      256 threads                                  -> <= 8 CTAs / SM (thread limit) -> <= 1184 CTAs
   pdx_scan_kernel        256 threads                                  -> <= 8 CTAs / SM (thread limit) -> <= 1184 CTAs
+    (the masked form of batch_knn_filtered: 38 / 64 registers for R = 1 / 4; the reordered form PDX_L2_PERM)
+  ternary_topk_kernel    256 threads, 32-40 registers (all OP, R)     -> <= 8 CTAs / SM (thread limit) -> <= 1184 CTAs
+  binary_setops_topk_kernel  256 threads, 32-40 registers             -> <= 8 CTAs / SM (thread limit) -> <= 1184 CTAs
+  topk_scores_kernel     256 threads, grid capped at 4 x 148 = 592 CTAs (launch_topk_from_scores); every selection
+                         of k > 128, of topk_from_distances and of the filtered / adaptive rounds: <= 592 x 256
+                         elements per grid-stride step
   maxsim_tc_kernel       grid = 148 CTAs (one per SM)
+Every case asserts its own premise from its sizes (_n_tiles): tiles (or grid-stride steps) >= 8 x the largest grid.
+The tests after the MaxSim ones share module-scoped corpora (each built once) and end with launches of different
+grids back to back on one workspace.
 
-Each test prints its wall time and the device memory in use at its peak (run with -rP to see it)."""
+Each test and each shared corpus prints its wall time, the device memory in use at its peak and the process's
+resident host memory at its peak (run with -rP to see it)."""
 import ctypes as C
 import os
 import time
@@ -43,24 +53,46 @@ def ib():
 
 
 class _Usage:
+    """Wall time, device memory in use at its peak (sampled by note()), and the process's resident host memory at its
+    peak (sampled every 20 ms by a thread)."""
+
     def __init__(self):
+        import threading
         import torch
         self.total = torch.cuda.mem_get_info()[1]
         self.peak = self.total - torch.cuda.mem_get_info()[0]
         self.t0 = time.time()
+        self.host_peak = 0
+        self._stop = threading.Event()
+        self._thread = threading.Thread(target=self._sample_host, daemon=True)
+        self._thread.start()
+
+    def _sample_host(self):
+        page = os.sysconf("SC_PAGE_SIZE")
+        while True:
+            with open("/proc/self/statm") as f:
+                self.host_peak = max(self.host_peak, int(f.read().split()[1]) * page)
+            if self._stop.wait(0.02):
+                return
 
     def note(self):
         import torch
         torch.cuda.synchronize()
         self.peak = max(self.peak, self.total - torch.cuda.mem_get_info()[0])
 
+    def report(self, name):
+        self.note()
+        self._stop.set()
+        self._thread.join()
+        print(f"[many-tiles] {name}: wall {time.time() - self.t0:.1f} s, peak device memory in use {self.peak / 1e9:.1f} GB,"
+              f" peak host memory resident {self.host_peak / 1e9:.1f} GB")
+
 
 @pytest.fixture
 def usage(request):
     u = _Usage()
     yield u
-    u.note()
-    print(f"[many-tiles] {request.node.name}: wall {time.time() - u.t0:.1f} s, peak device memory in use {u.peak / 1e9:.1f} GB")
+    u.report(request.node.name)
 
 
 def bits(a):
@@ -141,12 +173,14 @@ def test_hamming_1024bit_many_tiles(ib, oracle, usage):
                 codes[pl.pick(region)] = flipped(q, m)
     corpus = ib.BinaryCorpus.from_words(codes.reshape(-1), n, 1024)
     usage.note()
-    widx, wd = oracle.hamming_topk_many(qs, codes, 128, n_threads=min(NT, 5))   # stable sort: k < 128 is a prefix
+    widx, wd = oracle.hamming_topk_many(qs, codes, 300, n_threads=min(NT, 5))   # stable sort: k < 300 is a prefix
     assert wd[:, 127].max() <= 10
-    for k in KS:
+    for k in KS + (129, 300):   # 129 and 300: the scores pass, then selection rounds of kind 2
         for j in range(5):
             gi, gd = ib.hamming_topk(qs[j], corpus, k)
             assert gi.tolist() == widx[j, :k].tolist() and gd.tolist() == wd[j, :k].tolist(), ("single", j, k)
+        if k > 128:
+            continue
         for lo, hi in ((0, 2), (1, 4), (0, 4), (0, 5)):
             gi, gd = ib.hamming_topk_many(qs[lo:hi], corpus, k)
             assert np.array_equal(gi, widx[lo:hi, :k]) and np.array_equal(gd, wd[lo:hi, :k]), ("batch", lo, hi, k)
@@ -205,11 +239,13 @@ def test_u8_many_tiles(ib, oracle, usage, n, d):
             mat[pl.group(count)] = row
     corpus = ib.U8Corpus.from_rows(mat, gp)
     usage.note()
-    widx, wsc = oracle.batch_knn_u8_many(qs, mat, op, 128, n_threads=min(NT, 4))   # stable sort: k < 128 is a prefix
-    for k in KS:
+    widx, wsc = oracle.batch_knn_u8_many(qs, mat, op, 300, n_threads=min(NT, 4))   # stable sort: k < 300 is a prefix
+    for k in KS + (129, 300):   # 129 and 300: the scores pass, then selection rounds of kind 1
         for j in (0, 1):
             gi, gs = ib.batch_knn_u8_many(qs[j], corpus, k)
             assert np.array_equal(gi[0], widx[j, :k]) and np.array_equal(bits(gs[0]), bits(wsc[j, :k])), ("single", j, k)
+        if k > 128:
+            continue
         gi, gs = ib.batch_knn_u8_many(qs, corpus, k)   # two pairs
         assert np.array_equal(gi, widx[:, :k]) and np.array_equal(bits(gs), bits(wsc[:, :k])), ("pairs", k)
 
@@ -454,3 +490,439 @@ def test_maxsim_tc_mixed_lengths(ib, oracle, usage):
     assert int(off[-1]) // 128 >= 8 * SMS
     for cosine in (True, False):
         _maxsim_checks(ib, oracle, corpus, toks, off, qs, cosine, rel=False)
+
+
+# ------------------------------------------------------------------------------------------------ 5. ternary top-k
+KS_ROUNDS = KS + (129, 300)   # k > 128: the scores pass, then selection rounds of topk_scores_kernel
+BIG_BASE = 3_000_000_000      # > 2^31: a signed or truncated index shows
+TER_N = 2_500_037             # 9,766 tiles of 256 codes, the last holding 197
+
+
+def _n_tiles(n, tile, max_grid):
+    """Tiles (or, for topk_scores_kernel, grid-stride steps of 256 elements) of a launch of n rows, asserted to give each
+    CTA of the largest grid the kernel can have at least 8 of them."""
+    nt = -(-n // tile)
+    assert nt >= 8 * max_grid, (n, tile, nt, max_grid)
+    return nt
+
+
+def _pool_map(fn, items):
+    from concurrent.futures import ThreadPoolExecutor
+    with ThreadPoolExecutor(NT) as ex:
+        return list(ex.map(fn, items))
+
+
+T_ODD, T_EVEN, ONE = np.uint64(0x5555555555555555), np.uint64(0xAAAAAAAAAAAAAAAA), np.uint64(1)
+
+
+def _ter_masks(w):
+    """innr_ref.cpp ternary_dot / ternary_hamming: +1 and -1 positions (one bit per value) and nonzero positions."""
+    hi = (w & T_EVEN) >> ONE
+    return w & ~hi & T_ODD, ~w & hi & T_ODD, (w & T_ODD) | hi
+
+
+def _ter_ref_int(words, qw, block=1 << 16):
+    """ternary_dot and ternary_hamming of every row of row-major words against query words qw."""
+    n = len(words)
+    dot, ham = np.empty(n, np.int32), np.empty(n, np.int32)
+    qp, qn, qz = _ter_masks(qw)
+
+    def work(b0):
+        w = words[b0:b0 + block]
+        p, m, z = _ter_masks(w)
+        same = np.bitwise_count((p & qp) | (m & qn)).sum(axis=1, dtype=np.int32)
+        diff = np.bitwise_count((p & qn) | (m & qp)).sum(axis=1, dtype=np.int32)
+        dot[b0:b0 + block] = same - diff
+        x = w ^ qw
+        ham[b0:b0 + block] = np.bitwise_count(((x & T_ODD) | ((x & T_EVEN) >> ONE)) & z & qz).sum(axis=1, dtype=np.int32)
+
+    _pool_map(work, range(0, n, block))
+    return dot, ham
+
+
+def _ter_ref_asym(words, q, block=1 << 14):
+    """ternary::asymmetric_dot of every row: the sequential f32 sum s = s + q[j] * t[j] (products and sums rounded
+    separately, 0b11 reads 0), over dimension-major values unpacked from the words."""
+    n, nw = words.shape
+    d = len(q)
+    out = np.empty(n, np.float32)
+    qc = np.asarray(q, np.float32)[:, None]
+
+    def work(b0):
+        w = np.ascontiguousarray(words[b0:b0 + block].T)                     # (words, rows)
+        by = np.ascontiguousarray(w.view(np.uint8).reshape(nw, -1, 8).transpose(0, 2, 1))   # byte b of word i
+        c = np.empty((nw, 8, 4, by.shape[2]), np.uint8)
+        for t in range(4):
+            c[:, :, t] = (by >> (2 * t)) & 3
+        c = c.reshape(nw * 32, -1)[:d]                                          # (d, rows) 2-bit codes
+        p = np.multiply((c & 1).astype(np.int8) - (c >> 1).astype(np.int8), qc, dtype=np.float32)
+        s = np.zeros(p.shape[1], np.float32)
+        for j in range(d):
+            np.add(s, p[j], out=s)
+        out[b0:b0 + block] = s
+
+    _pool_map(work, range(0, n, block))
+    return out
+
+
+def _stable_order(scores, descending, k):
+    """The first k of a stable sort (ties -> lower index) under the order of the keys: f32 by total order."""
+    if scores.dtype == np.float32:
+        b = scores.view(np.uint32)
+        key = np.where(b >> np.uint32(31), ~b, b | np.uint32(0x80000000))
+        key = ~key if descending else key
+    else:
+        key = -scores.astype(np.int64) if descending else scores
+    part = np.argpartition(key, k)[:k + 1] if len(key) > k + 1 else np.arange(len(key))
+    cut = key[part].max()   # every row with a key <= the (k+1)-th smallest, then sorted stably
+    cand = np.flatnonzero(key <= cut)
+    return cand[np.argsort(key[cand], kind="stable")][:k]
+
+
+def _valid_ternary(w, d):
+    """pairs 0b11 -> 0b01, padding pairs cleared: what PackedTernary::set can produce"""
+    w = w & ~((w & T_ODD) << ONE)
+    if d % 32:
+        w[..., -1] &= np.uint64((1 << (2 * (d % 32))) - 1)
+    return w
+
+
+@pytest.fixture(scope="module")
+def ternary(ib, oracle):
+    """For d = 200 (a partial 64-value chunk and a partial word) and d = 1024: 2,500,037 raw random ternary codes (0b11
+    pairs and dirty padding bits included, as from_words accepts them) at index_base 3,000,000,000, two ternary queries
+    and one f32 query, and the reference top-300 of every (op, query). Planted per ternary query: LEVELS copies of the
+    query with m = 1..5 nonzero values negated (dot |q|nz - 2m, Hamming m); per f32 query: LEVELS copies each of five
+    rows sign(q) with its 3, 6, ... largest |q| values zeroed (identical rows: identical sums)."""
+    u = _Usage()
+    out = {}
+    for d in (200, 1024):
+        words = oracle.ghash_u64_mt(0x4A11_0100 + d, 0, TER_N * ((d + 31) // 32), NT).reshape(TER_N, -1)
+        qws = _valid_ternary(oracle.ghash_u64(0x4A11_0101 + d, 0, 2 * words.shape[1]).reshape(2, -1), d)
+        qf = oracle.ghash_f32(0x4A11_0102 + d, 0, d)
+        qf[d // 3] = -0.0
+        pl = Planter(TER_N, 256, d)
+        rng = np.random.default_rng(d)
+        for qw in qws:
+            nzp = np.flatnonzero(np.array([(int(qw[j // 32]) >> (2 * (j % 32))) & 3 for j in range(d)]) != 0)
+            for m, count in zip(range(1, 6), LEVELS):
+                for i in pl.group(count):
+                    row = qw.copy()
+                    for j in rng.choice(nzp, size=m, replace=False):
+                        row[j // 32] ^= np.uint64(3 << (2 * (j % 32)))
+                    words[i] = row
+        best = np.where(qf > 0, 1, np.where(qf < 0, 2, 0))
+        order = np.argsort(-np.abs(qf), kind="stable")
+        for lvl, count in enumerate(LEVELS):
+            vals = best.copy()
+            vals[order[:3 * (lvl + 1)]] = 0
+            row = np.zeros(words.shape[1], np.uint64)
+            for j in np.flatnonzero(vals):
+                row[j // 32] |= np.uint64(int(vals[j]) << (2 * (j % 32)))
+            words[pl.group(count)] = row
+        if d % 32:   # dirty padding pairs: the upload masks them, as PackedTernary::new does
+            words[::7, -1] |= ~np.uint64((1 << (2 * (d % 32))) - 1)
+        corpus = ib.TernaryCorpus.from_words(words.reshape(-1), TER_N, d, index_base=BIG_BASE)
+        if d % 32:
+            words[:, -1] &= np.uint64((1 << (2 * (d % 32))) - 1)
+        want = {}
+        for j, qw in enumerate(qws):
+            dot, ham = _ter_ref_int(words, qw)
+            want["dot", j] = (_stable_order(dot, True, 300), dot)
+            want["hamming", j] = (_stable_order(ham, False, 300), ham)
+        asym = _ter_ref_asym(words, qf)
+        want["asymmetric_dot", 0] = (_stable_order(asym, True, 300), asym)
+        # the numpy restatement against the oracle's: planted rows, the last tile, and random rows
+        rows = sorted(pl.taken)[::3] + list(range(TER_N - 60, TER_N)) + list(range(0, 40))
+        oq = [oracle.PackedTernary(qw, d) for qw in qws]
+        for i in rows:
+            oc = oracle.PackedTernary(words[i], d)
+            for j in range(2):
+                assert oracle.ternary_dot(oq[j], oc) == want["dot", j][1][i], (d, i)
+                assert oracle.ternary_hamming(oq[j], oc) == want["hamming", j][1][i], (d, i)
+            assert bits(np.float32(oracle.ternary_asymmetric_dot(qf, oc))) == bits(asym[i]), (d, i)
+        out[d] = {"corpus": corpus,
+                  "queries": {"dot": [ib.PackedTernary(qw, d) for qw in qws],
+                              "hamming": [ib.PackedTernary(qw, d) for qw in qws], "asymmetric_dot": [qf]},
+                  "want": {key: (idx, sc[idx].astype(np.float32)) for key, (idx, sc) in want.items()}}
+        del words, dot, ham, asym
+    u.report("fixture ternary")
+    return out
+
+
+def test_ternary_topk_many_tiles(ib, ternary, usage):
+    """ternary_topk_kernel<OP, R>, all three ops: 9,766 tiles of 256 codes, <= 1184 CTAs (256 threads, 32-40 registers:
+    thread limit) -> >= 8.2 tiles per CTA; k = 129 and 300 take the scores kernel and selection rounds of kinds 0 and 1
+    over 2,500,037 scores (>= 16 grid-stride steps per thread of topk_scores_kernel's 592 CTAs). Indices carry
+    index_base = 3,000,000,000; scores compared bit for bit."""
+    _n_tiles(TER_N, 256, 8 * SMS)
+    _n_tiles(TER_N, 256, 4 * SMS)
+    usage.note()
+    for d, t in ternary.items():
+        for (op, j), (widx, wsc) in t["want"].items():
+            q = t["queries"][op][j]
+            for k in KS_ROUNDS:
+                gi, gs = ib.ternary_topk(op, q, t["corpus"], k)
+                assert gi.tolist() == (widx[:k] + BIG_BASE).tolist(), (d, op, j, k, gi[:6], widx[:6] + BIG_BASE)
+                assert np.array_equal(bits(gs), bits(wsc[:k])), (d, op, j, k)
+
+
+def test_ternary_from_split_corpus(ib, oracle, usage):
+    """ternary_from_pdx_kernel over split planes at scale: encode_ternary of a split DeviceBatch of 2,500,037 x 100
+    ghash rows (100 values: a partial chunk and a partial word) on the device must give the codes numpy gives: every
+    dot and Hamming score of two queries, and the top-k of all three ops, equal those of the uploaded numpy words."""
+    n, d, thr = TER_N, 100, 0.25
+    rows = oracle.ghash_f32_mt(0x4A11_0103, 0, n * d, NT).reshape(n, d)
+    split = ib.DeviceBatch.from_rows_flat(rows.reshape(-1), n, d)   # n >= f32_split_min_rows: split planes
+    derived = ib.TernaryCorpus.from_f32(split, thr)
+    del split
+    nw = (d + 31) // 32
+    words = np.zeros((n, nw), np.uint64)
+
+    def enc(b0, block=1 << 16):
+        v = rows[b0:b0 + block]
+        c = np.zeros((len(v), nw * 32), np.uint64)
+        c[:, :d] = np.where(v > thr, 1, np.where(v < -thr, 2, 0))
+        words[b0:b0 + block] = (c.reshape(len(v), nw, 32) << (2 * np.arange(32, dtype=np.uint64))).sum(axis=2, dtype=np.uint64)
+
+    _pool_map(enc, range(0, n, 1 << 16))
+    assert np.count_nonzero(words) > n
+    uploaded = ib.TernaryCorpus.from_words(words.reshape(-1), n, d)
+    usage.note()
+    qws = _valid_ternary(oracle.ghash_u64(0x4A11_0104, 0, 2 * nw).reshape(2, nw), d)
+    qf = oracle.ghash_f32(0x4A11_0105, 0, d)
+    for qw in qws:
+        q = ib.PackedTernary(qw, d)
+        for op in ("dot", "hamming"):
+            assert np.array_equal(ib.ternary_scores_all(op, q, derived), ib.ternary_scores_all(op, q, uploaded)), op
+    dot, ham = _ter_ref_int(words, qws[0])
+    assert np.array_equal(ib.ternary_scores_all("dot", ib.PackedTernary(qws[0], d), derived), dot)
+    for op, q in (("dot", ib.PackedTernary(qws[0], d)), ("hamming", ib.PackedTernary(qws[1], d)), ("asymmetric_dot", qf)):
+        for k in (10, 128, 300):
+            gi, gs = ib.ternary_topk(op, q, derived, k)
+            wi, ws = ib.ternary_topk(op, q, uploaded, k)
+            assert np.array_equal(gi, wi) and np.array_equal(bits(gs), bits(ws)), (op, k)
+
+
+# ------------------------------------------------------------------------------------------------ 6. binary dot / Jaccard
+@pytest.fixture(scope="module")
+def setops(ib, oracle):
+    """8,000,200 x 1024-bit codes at index_base 0 and 2,500,037 x 200-bit codes at index_base 3,000,000,000, ghash rows
+    with planted tie groups for each of two random queries: LEVELS copies of the query with m = 2, 4, .. 10 of its bits
+    cleared (dot |q| - m, Jaccard (|q| - m) / |q|), LEVELS copies with m bits set outside it (dot |q|, Jaccard |q| / (|q|
+    + m)); and 60 empty rows. Queries: the two, and the empty code. Reference top-300 of both ops (ref_setop_topk)."""
+    from test_gpu_bin_tc import ref_setop_topk
+    u = _Usage()
+    out = {}
+    for n, dim, base in ((8_000_200, 1024, 0), (TER_N, 200, BIG_BASE)):
+        nw = (dim + 63) // 64
+        codes = oracle.ghash_u64_mt(0x4A11_0110 + dim, 0, n * nw, NT).reshape(n, nw)
+        if dim % 64:
+            codes[:, -1] &= np.uint64((1 << (dim % 64)) - 1)
+        qs = oracle.ghash_u64(0x4A11_0111 + dim, 0, 3 * nw).reshape(3, nw)
+        if dim % 64:
+            qs[:, -1] &= np.uint64((1 << (dim % 64)) - 1)
+        qs[2] = 0
+        pl = Planter(n, 256, dim)
+        rng = np.random.default_rng(dim)
+        for q in qs[:2]:
+            qb = np.unpackbits(q.view(np.uint8), bitorder="little")
+            on, off = np.flatnonzero(qb[:dim]), np.flatnonzero(qb[:dim] == 0)
+            for src, sign in ((on, 0), (off, 1)):
+                for m, count in zip((2, 4, 6, 8, 10), LEVELS):
+                    for i in pl.group(count):
+                        b = qb.copy()
+                        b[rng.choice(src, size=m, replace=False)] = sign
+                        codes[i] = np.packbits(b, bitorder="little").view(np.uint64)
+        codes[pl.group(60)] = 0
+        corpus = ib.BinaryCorpus.from_words(codes.reshape(-1), n, dim, index_base=base)
+        want = {op: ref_setop_topk(op, qs, codes, 300) for op in ("dot", "jaccard")}
+        out[dim] = {"corpus": corpus, "qs": qs, "n": n, "base": base, "want": want}
+        del codes
+    u.report("fixture setops")
+    return out
+
+
+def test_binary_setops_topk_many_tiles(ib, setops, usage):
+    """binary_setops_topk_kernel<JACCARD, R> (one query): 31,251 tiles of 256 codes (1024 bits) and 9,766 (200 bits),
+    <= 1184 CTAs (256 threads, 32-40 registers: thread limit) -> >= 26 / >= 8.2 tiles per CTA. k = 129 and 300: the
+    scores kernels, then selection rounds of kind 4 (dot, u32 descending) and kind 1 (Jaccard) over >= 16 grid-stride
+    steps per thread of 592 CTAs. Indices and score bits against ref_setop_topk."""
+    usage.note()
+    for dim, s in setops.items():
+        _n_tiles(s["n"], 256, 8 * SMS)
+        for op in ("dot", "jaccard"):
+            widx, wsc = s["want"][op]
+            for j, q in enumerate(s["qs"]):
+                pq = ib.PackedBinary(q, dim)
+                for k in KS_ROUNDS:
+                    gi, gs = ib.binary_topk(op, pq, s["corpus"], k)
+                    assert gi.tolist() == (widx[j, :k] + np.uint64(s["base"])).tolist(), (dim, op, j, k, gi[:6], widx[j, :6])
+                    assert np.array_equal(bits(gs), bits(wsc[j, :k])), (dim, op, j, k)
+
+    import torch
+    from innr_b200 import _lib as L
+    s = setops[1024]
+    dq = torch.from_numpy(s["qs"].view(np.int64)).cuda()
+    for opi, op in enumerate(("dot", "jaccard")):
+        def run(j, k, st):
+            out = torch.empty(k, dtype=torch.int64, device="cuda")
+            L.call("innr_cuda_binary_topk_keys_dev", s["corpus"].h, opi, C.c_void_p(dq[j].data_ptr()), 1, k,
+                   C.c_void_p(out.data_ptr()), _stream_ptr(st))
+            return out
+
+        for k in (10, 100):
+            _check_abab(run, k, lambda o, j: (o.view(np.uint64) & np.uint64(0xFFFFFFFF)).tolist()
+                        == s["want"][op][0][j, :k].tolist())
+
+
+# ------------------------------------------------------------------------------------------------ 7. selection rounds
+def _planted_distances(oracle, n, seed):
+    """Integer distances in [0, 2000) (about n / 2000 copies of each), with 100 copies of -3, 60 of -2 and 130 of -1
+    planted over the Planter regions: sorted positions 100-159 (127 / 128 inside) and 160-289 (255 / 256 inside) are
+    tie groups whose members sit in different regions."""
+    d = np.floor(oracle.ghash_f32_mt(seed, 0, n, NT).astype(np.float64) * 1000.0 + 1000.0).astype(np.float32)
+    d = np.clip(d, 0, 1999)
+    pl = Planter(n, 256, seed)
+    for v, count in ((-3.0, 100), (-2.0, 60), (-1.0, 130)):
+        d[pl.group(count)] = v
+    return d
+
+
+def test_topk_from_distances_rounds(ib, oracle, usage):
+    """topk_scores_kernel<R, 0> in rounds of <= 128, each bounded by the last key of the round before: 5,000,011
+    distances, <= 592 CTAs x 256 threads -> >= 33 grid-stride steps per thread; k = 1 .. 5000."""
+    n = 5_000_011
+    _n_tiles(n, 256, 4 * SMS)
+    d = _planted_distances(oracle, n, 0x4A11_0120)
+    assert len(np.unique(d)) == 2003
+    want = np.lexsort((np.arange(n), d))[:5000]
+    ws = d[want]
+    assert ws[127] == ws[128] == -2 and ws[255] == ws[256] == -1
+    usage.note()
+    for k in (1, 127, 128, 129, 255, 256, 257, 1000, 5000):
+        got = ib.topk_from_distances(d, k)
+        assert [i for i, _ in got] == want[:k].tolist(), k
+        assert np.array_equal(bits([v for _, v in got]), bits(ws[:k])), k
+
+
+# ------------------------------------------------------------------------------------------------ 8. filtered / reordered
+FLT_N = 9_700_037   # 9,473 tiles of 1024 rows
+
+
+@pytest.fixture(scope="module")
+def filtered(ib, oracle):
+    """9,700,037 x 16 ghash rows with _plant_f32's tie groups for two queries, stored split (default options) and plain;
+    every row's squared L2 distance to each query (oracle) and its stable ascending order; four masks."""
+    u = _Usage()
+    n, d = FLT_N, 16
+    rows = oracle.ghash_f32_mt(0x4A11_0130, 0, n * d, NT).reshape(n, d)
+    ob = oracle.ghash_vertical_batch(0x4A11_0130, 0, n, d, NT)
+    qs = oracle.ghash_f32(0x4A11_0131, 0, 2 * d).reshape(2, d)
+    pl = Planter(n, 1024, 5)
+    _plant_f32(rows, ob.data.reshape(d, n), qs, pl)
+    split = ib.DeviceBatch.from_rows_flat(rows.reshape(-1), n, d)
+    ib.set_option("f32_split_min_rows", 2**62)
+    try:
+        plain = ib.DeviceBatch.from_rows_flat(rows.reshape(-1), n, d)
+    finally:
+        ib.set_option("f32_split_min_rows", SPLIT_DEFAULT)
+    del rows
+    dist = [oracle.batch_l2_squared(q, ob) for q in qs]
+    order = [np.argsort(x, kind="stable") for x in dist]
+    rng = np.random.default_rng(6)
+    nt = -(-n // 1024)
+    local = np.zeros(n, bool)
+    for t in (0, 32, nt - 1):   # tile 0, the first tile of finish group 1, the last partial tile
+        local[t * 1024:(t + 1) * 1024] = True
+    masks = {"half": rng.random(n) < 0.5, "sparse": rng.random(n) < 0.01, "all": np.ones(n, bool), "tiles": local}
+    planted = np.array(sorted(pl.taken))
+    assert 0 < np.count_nonzero(masks["half"][planted]) < len(planted)
+    u.report("fixture filtered")
+    return {"split": split, "plain": plain, "qs": qs, "ob": ob, "dist": dist, "order": order, "masks": masks, "n": n}
+
+
+def test_filtered_knn_many_tiles(ib, oracle, filtered, usage):
+    """pdx_scan_kernel<L2, 1, R, true, MASKED> (k <= 128): 9,473 tiles of 1024 rows, <= 1184 CTAs (256 threads, 38 / 64
+    registers for R = 1 / 4) -> >= 8.0 tiles per CTA; k = 129 and 700 take the distance pass and the masked selection
+    rounds (>= 64 grid-stride steps per thread of 592 CTAs). Reference: the oracle's distance of every row, the passing
+    rows in stable ascending order (ties -> lower index, DESIGN section 4)."""
+    f = filtered
+    _n_tiles(f["n"], 1024, 8 * SMS)
+    _n_tiles(f["n"], 256, 4 * SMS)
+    usage.note()
+    for mname, mask in f["masks"].items():
+        for j, q in enumerate(f["qs"]):
+            want = f["order"][j][mask[f["order"][j]]][:700]
+            wsc = f["dist"][j][want]
+            for store in ("split", "plain"):
+                for k in (1, 10, 32, 33, 128, 129, 700):
+                    g = ib.batch_knn_filtered(q, f[store], k, mask)
+                    assert g.indices == want[:k].tolist(), (mname, j, store, k, g.indices[:6], want[:6])
+                    assert np.array_equal(bits(g.scores), bits(wsc[:k])), (mname, j, store, k)
+    mask = f["masks"]["sparse"]
+    w = oracle.batch_knn_filtered(f["qs"][0], f["ob"], 33, mask.item)
+    g = ib.batch_knn_filtered(f["qs"][0], f["split"], 33, mask)
+    assert g.indices == w.indices and np.array_equal(bits(g.scores), bits(w.scores))
+
+
+def test_reordered_knn_many_tiles(ib, oracle, filtered, usage):
+    """pdx_scan_kernel<PDX_L2_PERM, ...> (batch_knn_reordered): the corpus of the filtered case, split and plain, 9,473
+    tiles of 1024 rows -> >= 8.0 tiles per CTA of <= 1184; against the oracle, indices and score bits."""
+    f = filtered
+    _n_tiles(f["n"], 1024, 8 * SMS)
+    usage.note()
+    for q in f["qs"]:
+        w = oracle.batch_knn_reordered(q, f["ob"], 128)
+        for store in ("split", "plain"):
+            for k in (1, 10, 128):
+                g = ib.batch_knn_reordered(q, f[store], k)
+                assert g.indices == w.indices[:k], (store, k, g.indices[:6], w.indices[:6])
+                assert np.array_equal(bits(g.scores), bits(w.scores[:k])), (store, k)
+
+
+def test_adaptive_knn_many_steps(ib, oracle, usage):
+    """batch_knn_adaptive on 1,300,007 x 96 rows (split under default options): its warm-up, masked and kind-3 selection
+    rounds stride >= 8 times over 592 CTAs x 256 threads (8 x 592 x 256 = 1,212,416 elements). The "planted" and "ties"
+    inputs of test_knn_adaptive_bit_exact, against the oracle."""
+    from test_gpu_parity import _adaptive_case
+    n, d = 1_300_007, 96
+    _n_tiles(n, 256, 4 * SMS)
+    for kind in ("planted", "ties"):
+        rng = np.random.default_rng(n * 17 + d)
+        rows = _adaptive_case(rng, kind, n, d)
+        q = _adaptive_case(rng, kind, 1, d)[0] if kind != "planted" else np.zeros(d, np.float32)
+        gb = ib.DeviceBatch.from_rows_flat(rows.reshape(-1), n, d)
+        ob = oracle.VerticalBatch.from_flat(rows.reshape(-1), n, d)
+        del rows
+        usage.note()
+        for k in (10, 150, 1000):
+            for w in (8, 33):
+                g, want = ib.batch_knn_adaptive(q, gb, k, w), oracle.batch_knn_adaptive(q, ob, k, w)
+                assert g.indices == want.indices, (kind, k, w, g.indices[:6], want.indices[:6])
+                assert np.array_equal(bits(g.scores), bits(want.scores)), (kind, k, w)
+        del gb, ob
+
+
+# ------------------------------------------------------------------------------------------------ 9. grids in sequence
+def test_grids_in_sequence(ib, oracle, ternary, setops, filtered, usage):
+    """Launches of different grids back to back on the device's own stream, sharing one workspace: ternary top-k (up to
+    1184 CTAs, R = 1 then 4), two topk_from_distances rounds (592), set-operation top-k, filtered kNN, ternary again.
+    Each entry returns its own result, so each must equal the same call made alone (here: the reference); a ticket of
+    block_finish left set by one grid would corrupt the next launch's merge."""
+    t, s, f = ternary[200], setops[1024], filtered
+    dist = _planted_distances(oracle, 1_000_003, 0x4A11_0140)
+    want_d = np.lexsort((np.arange(len(dist)), dist))[:129]
+    mask = f["masks"]["half"]
+    want_f = f["order"][0][mask[f["order"][0]]][:10]
+    usage.note()
+    for _ in range(3):
+        for k in (10, 100):
+            gi, _s = ib.ternary_topk("dot", t["queries"]["dot"][0], t["corpus"], k)
+            assert gi.tolist() == (t["want"]["dot", 0][0][:k] + BIG_BASE).tolist(), k
+        assert [i for i, _ in ib.topk_from_distances(dist, 129)] == want_d.tolist()
+        gi, _s = ib.binary_topk("jaccard", ib.PackedBinary(s["qs"][0], 1024), s["corpus"], 33)
+        assert gi.tolist() == s["want"]["jaccard"][0][0, :33].tolist()
+        assert ib.batch_knn_filtered(f["qs"][0], f["split"], 10, mask).indices == want_f.tolist()
+        gi, _s = ib.ternary_topk("asymmetric_dot", t["queries"]["asymmetric_dot"][0], t["corpus"], 128)
+        assert gi.tolist() == (t["want"]["asymmetric_dot", 0][0][:128] + BIG_BASE).tolist()
